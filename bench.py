@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — benchmark of the gorp batch extraction path (BASELINE.json metric) over all five BASELINE configs.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 A step = one pass of the hot path (newline index -> combined DFA -> capture -> result rows -> histogram) over one
 batch of synthetic log text resident in HBM. N > 1: one process per GPU (torchrun), lines sharded as independent
@@ -24,6 +24,11 @@ histogram must equal the per-line outcomes. `parity.corpus_hash` sums all shards
 
 --impl reference times the CPU restatement alone (the reference is pure Java; no JVM exists in this image), same
 `config` as this arm, on a bounded sample of it per step.
+
+--dump-outputs DIR writes what the last timed step of `value` returned (rank 0's shard) as DIR/<name>.npy, so that two
+builds can be compared output for output: the whole histogram, and ext_id / line_off / spans of a fixed, seeded sample of
+lines (line_index) sized to keep all files under 64 MB. Integers are stored exactly: float32 for ext_id, float64 for the rest.
+The corpus is a pure function of (workload, line index), so the same arguments give the same inputs on every run.
 """
 from __future__ import annotations
 
@@ -38,6 +43,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the bench writes nothing into the tree (it may be read-only)
 
 import numpy as np  # noqa: E402
 
@@ -54,6 +60,8 @@ PREFIX_LINES = 1_000_000          # per rank: lines whose GPU rows are compared 
 CONFIG5_TOTAL_LINES = 281_600_000  # config #5: 100 GB of UTF-16 (355 B per line on average), sharded over the ranks
 EXTRA_CONFIGS = ["syslog200", "utf16mix", "weblog", "simple"]  # configs[] order: the 40 %-target config first
 TRAFFIC_FILE = os.path.join(ROOT, "profiles", "ncu_traffic.json")  # written by tools_ncu_traffic.py from an ncu --set full capture
+DUMP_BYTES = 56 << 20  # --dump-outputs: all .npy files together stay below 64 MB
+DUMP_SEED = 0x5EED00D0  # --dump-outputs: the sampled lines depend on this seed and the line count only
 
 
 def hbm_peak():
@@ -200,6 +208,32 @@ def run_reference(args, rank, world):
     }))
 
 
+def dump_outputs(out_dir, dres, n_bins, dev):
+    """Writes the gorp_device_result of the last call as DIR/<name>.npy: n_lines and the histogram whole, the per-line
+    arrays at a seeded sample of lines (line_index; every line when they fit): ext_id[i], (line_off[i], line_off[i + 1])
+    and the span row of line i."""
+    import torch
+    from gorp_b200 import parityhash
+    n, stride = int(dres.n_lines), int(dres.span_stride)
+    ext_t, sp_t = parityhash.device_results(dres, dev)
+    off_t = torch.as_tensor(parityhash.DeviceArray(dres.d_line_off, (n + 1,), "<i8"), device=dev)
+    hist_t = torch.as_tensor(parityhash.DeviceArray(dres.d_histogram, (n_bins,), "<i8"), device=dev)
+    per_line = 8 + 4 + 16 + 8 * stride
+    n_sample = min(n, (DUMP_BYTES - 8 * (n_bins + 1)) // per_line)
+    idx = np.arange(n) if n_sample == n else np.sort(np.random.default_rng(DUMP_SEED).choice(n, n_sample, replace=False))
+    idx_t = torch.from_numpy(idx).to(dev)
+    arrays = {"n_lines": np.array([n], dtype=np.float64),
+              "histogram": hist_t.cpu().numpy().astype(np.float64),
+              "line_index": idx.astype(np.float64),
+              "ext_id": ext_t[idx_t].cpu().numpy().astype(np.float32),
+              "line_off": torch.stack((off_t[idx_t], off_t[idx_t + 1]), dim=1).cpu().numpy().astype(np.float64),
+              "spans": sp_t[idx_t].cpu().numpy().astype(np.float64)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    print("[bench] outputs of the last timed step: %d of %d lines -> %s" % (n_sample, n, out_dir), file=sys.stderr)
+
+
 class Env:
     pass
 
@@ -236,7 +270,8 @@ def bind_numa(cudart, index):
     return info
 
 
-def device_config_run(env, workload, lines_per_gpu, steps, warmup, sampler=None, keep=False, first_line=None, corpus_note=None):
+def device_config_run(env, workload, lines_per_gpu, steps, warmup, sampler=None, keep=False, first_line=None, corpus_note=None,
+                      dump_dir=None):
     """One config, device-resident: returns the result dict (and, with keep=True, the engine / text for the e2e leg)."""
     torch, dist, lib, _ffi, Blob, _check, cudart = env.torch, env.dist, env.lib, env.ffi, env.Blob, env.check, env.cudart
     from gorp_b200 import corpusgen, parityhash, sharding
@@ -333,6 +368,8 @@ def device_config_run(env, workload, lines_per_gpu, steps, warmup, sampler=None,
     if per_step:
         print("[bench] %s ms per step:" % workload, [round(a.elapsed_time(b), 2) for a, b in per_step], file=sys.stderr)
     clocks = sampler.stop() if sampler else None
+    if dump_dir and rank == 0:
+        dump_outputs(dump_dir, dres, n_bins, dev)
     ms = e0.elapsed_time(e1) / steps
     if world > 1:  # every rank holds the job-wide histogram: its sum is the job's line count
         assert int(d_hist.sum().item()) == n_lines * world, (int(d_hist.sum().item()), n_lines * world)
@@ -567,7 +604,10 @@ def main():
     ap.add_argument("--skip-cpu", action="store_true", help="profiling runs only")
     ap.add_argument("--no-clock-sampler", action="store_true", help="diagnostics: do not run nvidia-smi beside the timed region")
     ap.add_argument("--workload", default="readme", choices=sorted(WORKLOADS), help="BASELINE.json config of `value` (default: #2, the headline)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step of `value` as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -599,7 +639,8 @@ def main():
     sampler = ClockSampler(local_rank)
     if not args.no_clock_sampler:
         sampler.launch()
-    head, clocks, kept = device_config_run(env, args.workload, args.lines_per_gpu, args.steps, args.warmup, sampler=sampler, keep=True)
+    head, clocks, kept = device_config_run(env, args.workload, args.lines_per_gpu, args.steps, args.warmup, sampler=sampler, keep=True,
+                                           dump_dir=args.dump_outputs)
     e2e = e2e_run(env, kept, args.workload)
     env.lib.gorp_engine_destroy(kept[0])
     kept = None
