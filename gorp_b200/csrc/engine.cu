@@ -2,11 +2,11 @@
 //
 // Device pipeline per batch (one stream, no host round trip except reading the line count of the text form):
 //   text form            : K1 count -> scan -> K1 scatter -> K1 finish          => line_off[n+1], n_lines
+//                          (the List<String> form brings its own line index: the caller's offsets)
 //   small definitions    : fused walk (kernels/tailwalk.cu, "all" mode) over the line index => ext_id, spans, histogram
-//                          (tier: the chunk-owner one-pass kernel K0c, kernels/chunkwalk.cu, without K1)
 //   big definitions      : K2b line walk over the early-exit table => candidates -> K3 histogram -> bucket pass ->
 //                          K4c tail walk (+ K4b capture walk for extractions without a tail) => ext_id, spans
-//   forced tiers         : K0d, K1h, K2 dfa_scan, K4 tdfa_capture (one line per thread)
+//   fallbacks            : K2 dfa_scan, K4 tdfa_capture (one line per thread)
 #include <cuda_runtime.h>
 #include <sys/syscall.h>
 #include <unistd.h>
@@ -121,11 +121,6 @@ T* upload(const std::vector<T>& v, std::vector<void*>& owned) {
 }
 
 constexpr int kMaxTimed = 12;
-// The decoupled look-back words are the only hot read-write global data of the one-pass kernels. They get 2 MB pages of
-// their own: when this buffer came out of the pool of the engine's small table allocations, k0_chunkwalk_extract ran
-// 15-30 % slower (same SASS, same box; measured A/B, profiles/README.md round 1e).
-constexpr size_t kTileStateMinBytes = 4u << 20;
-
 struct DeviceCtx {
     int device = 0;
     int numa_node = -1;
@@ -136,8 +131,6 @@ struct DeviceCtx {
     DfaDirectDev dfa_direct{};
     TdfaFastDev cap_fast{};
     CapDev cap{};
-    OnePassDev onepass{};
-    OnePassDev chunkwalk{};      // same automaton, table variant of kernels/chunkwalk.cu
     DfaWalkDev dfawalk{};        // class-indexed combined DFA of kernels/dfawalk.cu (text form, any definition)
     PikeDev pike{};              // simulating Pike VM for extractions without a determinised capture automaton (kernels/pike.cu)
     DevBuf pike_scratch;
@@ -146,25 +139,20 @@ struct DeviceCtx {
     DfaWalkDev dfawalk_cut{};    // the same with the early-exit cut of host/tails.hpp (K2b when the tail walk follows)
     TailDev tails{};             // per-extraction tail automata of kernels/tailwalk.cu
     TailDev fused_tail{};        // the one-pass automaton of host/fused.hpp as ONE tail table for every line (K1 + tail walk, "fused walk")
-    bool fusedwalk_default = false;  // small definitions: K1 + fused walk instead of the chunk-owner kernel K0c (GORP_SMALL_PATH)
-    bool cut_effective = false;  // most states of the combined DFA are cut: the chunk-owner walk with early exit (K0d cut)
     uint32_t tail_flush_every = 8;  // walk iterations per round of the tail walk (GORP_TAIL_FLUSH)
     uint32_t item_lines = kCapItemLines;  // work items of the capture walks (GORP_ITEM_LINES)
     bool item_interleave = false;         // ... listed by relative position inside their bucket (GORP_ITEM_ORDER=1)
     DevBuf long_lines, recs;
     CapImgDev capimg{};          // per-extraction capture tables of kernels/capwalk.cu (text form, any definition)
     bool force_k4 = false;       // GORP_FORCE_K4=1: one-line-per-thread capture kernels (K4) instead of the bucketed K4b
-    DevBuf perm, items, buckets, nl_masks, cand_tmp;
-    int dfa_tier = 0;            // GORP_DFA_TIER: 0 = by line length, 1 = chunk-owner walk (K0d), 2 = line index + lane queue (K1 + K2b),
-                                 // 3 = line index with the head walk inside its count pass (K1h)
-    bool force_k1k2 = false;     // GORP_FORCE_K1K2=1: newline index + DFA scan as separate kernels (K1, K2) instead of K0d
+    DevBuf perm, items, buckets, nl_masks;
+    bool force_k1k2 = false;     // GORP_FORCE_K1K2=1: newline index without masks + one-line-per-thread DFA scan (K1, K2) instead of K2b
     uint32_t* d_slots = nullptr;
     uint32_t n_ext = 0;
     uint32_t max_slots = 0;
     bool force_general = false;  // GORP_FORCE_GENERAL=1: always use the general (masked) kernels
-    bool force_twopass = false;  // GORP_FORCE_TWOPASS=1: never use the one-pass automaton kernel (K1 -> K2 -> K4 instead)
-    double lines_per_unit = 1.0 / 24.0;  // running estimate that sizes the one-pass kernel's tiles and output arrays
-    DevBuf tile_state;
+    bool force_twopass = false;  // GORP_FORCE_TWOPASS=1: never use the fused walk (small definitions take the big-definition path)
+    double lines_per_unit = 1.0 / 24.0;  // running estimate that sizes the row arrays of a host-buffer call (run_pieces)
     // host-buffer calls are pipelined in pieces: H2D of piece k+1 (s_in) overlaps the kernels of piece k (stream) and
     // the D2H of the rows of piece k-1 (s_out); the rows of all pieces accumulate in acc_*
     cudaStream_t s_in = nullptr, s_out = nullptr;
@@ -173,7 +161,7 @@ struct DeviceCtx {
     DevBuf textbuf[2], offbuf[2], bytebuf[2], acc_ext, acc_off, acc_spans, acc_hist;
     // per-call scratch, serialised by `mu`
     std::mutex mu;
-    DevBuf text, off_in, line_off, tile_counts, tile_base, scan_scratch, ext_id, spans, hist, scalars, debug;
+    DevBuf text, off_in, line_off, tile_counts, tile_base, scan_scratch, ext_id, spans, hist, scalars;
     // per-kernel device time: CUDA events on the launching stream, accumulated over timed calls
     cudaEvent_t ev[kMaxTimed + 1]{};
     const char* ev_name[kMaxTimed]{};
@@ -320,7 +308,6 @@ void build_device(DeviceCtx& c, const DeviceModel& m, const FusedAutomaton& fuse
     if (const char* f = std::getenv("GORP_FORCE_TWOPASS")) c.force_twopass = f[0] == '1';
     if (const char* f = std::getenv("GORP_FORCE_K1K2")) c.force_k1k2 = f[0] == '1';
     if (const char* f = std::getenv("GORP_FORCE_K4")) c.force_k4 = f[0] == '1';
-    if (const char* f = std::getenv("GORP_DFA_TIER")) c.dfa_tier = std::atoi(f);
     if (const char* f = std::getenv("GORP_L2_FETCH")) cudaDeviceSetLimit(cudaLimitMaxL2FetchGranularity, static_cast<size_t>(std::atoi(f)));  // diagnostics
     for (auto& e : c.ev) CK(cudaEventCreate(&e));
     // the reference's tables as they are (matchAll)
@@ -396,7 +383,7 @@ void build_device(DeviceCtx& c, const DeviceModel& m, const FusedAutomaton& fuse
             c.dfa_direct.enabled = 1;
         }
     }
-    // chunk-walk / line-walk DFA tier: class-indexed u16 rows + DEADSCAN / SKIP / FIN rows (host/walktables.hpp)
+    // line-walk DFA tier (K2b): class-indexed u16 rows + DEADSCAN / SKIP / FIN rows (host/walktables.hpp)
     if (!std::getenv("GORP_SKIP_NEWTABLES")) {
         const DfaWalkTable t = build_dfawalk_table(m);
         if (t.available) {
@@ -544,142 +531,13 @@ void build_device(DeviceCtx& c, const DeviceModel& m, const FusedAutomaton& fuse
                     c.dfawalk_cut.xcls = upload(t.xcls, c.owned);
                     c.dfawalk_cut.enabled = 1;
                     d.enabled = 1;
-                    // the chunk-owner variant of the early-exit walk (one pass, newline masks) measured 4.87 ms against 4.53 ms for
-                    // K1 + K2b on config #4 (profiles/README.md, round 2): kept as a tier (GORP_CUT_WALK=1), off by default
-                    c.cut_effective = false;
-                    if (const char* f = std::getenv("GORP_CUT_WALK")) c.cut_effective = f[0] == '1';
                     if (const char* f = std::getenv("GORP_TAIL_FLUSH")) c.tail_flush_every = std::min(64, std::max(1, std::atoi(f)));
                 }
             }
         }
-        // one-pass automaton: DFA x capture automata folded into one automaton (host/fused.hpp) — table of the K0c tier
-        {
-            const FusedAutomaton& A = fused;
-            if (A.available) {
-                const uint32_t Sx = A.n_states, J = A.n_jcls, n_out = static_cast<uint32_t>(A.outcomes.size());
-                // columns: [0,128) = ASCII units, then one column per joint class that a unit >= 0x80 (or a pair) can take
-                std::vector<int32_t> col_of_j(J, -1);
-                std::vector<uint32_t> j_of_col;
-                auto col = [&](uint32_t j) {
-                    if (col_of_j[j] < 0) {
-                        col_of_j[j] = static_cast<int32_t>(128 + j_of_col.size());
-                        j_of_col.push_back(j);
-                    }
-                    return static_cast<uint16_t>(col_of_j[j]);
-                };
-                std::vector<uint16_t> xcol(65536);
-                for (uint32_t u = 0; u < 128; ++u) xcol[u] = static_cast<uint16_t>(u);
-                for (uint32_t u = 128; u < 65536; ++u) xcol[u] = col(A.jcls[u]);
-                for (uint32_t u = 0xD800; u < 0xDC00; ++u) col(A.pair_of[A.jcls[u]]);
-                const uint32_t width = static_cast<uint32_t>((128 + j_of_col.size() + 3) & ~size_t(3));
-                std::vector<uint16_t> pair_col(width, 0);
-                for (uint32_t k = 0; k < width; ++k) pair_col[k] = static_cast<uint16_t>(k);
-                for (size_t k = 0; k < j_of_col.size(); ++k) pair_col[128 + k] = col(A.pair_of[j_of_col[k]]);
-                const uint32_t skip_base = Sx, fin_base = Sx + 7, n_rows = fin_base + n_out;
-                const uint32_t len_slot = A.n_op_slots + 1, n_slots = A.n_op_slots + 2;
-                const bool fits = static_cast<uint64_t>(n_rows) * width / 4 < (1u << 14) && n_slots < 250;
-                if (fits) {
-                    std::vector<uint32_t> rows(static_cast<size_t>(n_rows) * width, 0);
-                    for (uint32_t r = 0; r < n_rows; ++r)
-                        for (uint32_t k = 0; k < width; ++k) {
-                            uint32_t next = r, slot = 0;
-                            if (r < Sx) {
-                                if (k == 0x0A) {
-                                    next = fin_base + A.outcome_of[r];
-                                    slot = len_slot;
-                                } else if (k < 128 || k - 128 < j_of_col.size()) {
-                                    const uint32_t j = k < 128 ? A.jcls[k] : j_of_col[k - 128];
-                                    const uint32_t ent = A.trans[static_cast<size_t>(r) * J + j];
-                                    if ((ent & 0xFFFFu) == 0xFFFFu) next = fin_base;  // dead: MISS
-                                    else next = ent & 0xFFFFu, slot = ent >> 16;
-                                } else {
-                                    next = fin_base;  // padding column, never addressed
-                                }
-                            } else if (r < fin_base) {
-                                next = r == skip_base ? 0u : r - 1;  // SKIP chain
-                            }
-                            rows[static_cast<size_t>(r) * width + k] = (next << 16) | slot;
-                        }
-                    uint32_t max_slots = 0;
-                    for (uint32_t g : m.n_groups) max_slots = std::max(max_slots, 2 * g);
-                    max_slots = std::max(max_slots, 1u);
-                    std::vector<int32_t> out_ext(n_out);
-                    std::vector<uint32_t> out_res(static_cast<size_t>(n_out) * max_slots, 0), init;
-                    for (uint32_t o = 0; o < n_out; ++o) {
-                        out_ext[o] = A.outcomes[o].ext_code;
-                        if (out_ext[o] < 0) continue;
-                        for (uint32_t k = 0; k < 2 * m.n_groups[out_ext[o]]; ++k) {
-                            uint32_t packed = A.res[A.outcomes[o].res_off + k], fixed = 0, n = 0;
-                            for (uint32_t sh = 0; sh < 32 && (packed >> sh) & 0xFFu; sh += 8, ++n) {
-                                const uint32_t id = (packed >> sh) & 0xFFu;
-                                fixed |= (id == FusedAutomaton::kLenSlot ? len_slot : id) << sh;
-                            }
-                            if (n > 1)
-                                for (uint32_t sh = 0; sh < 8 * n; sh += 8) {
-                                    const uint32_t id = (fixed >> sh) & 0xFFu;
-                                    if (std::find(init.begin(), init.end(), id) == init.end()) init.push_back(id);
-                                }
-                            out_res[static_cast<size_t>(o) * max_slots + k] = fixed;
-                        }
-                    }
-                    c.onepass.rows = upload(rows, c.owned);
-                    c.onepass.n_rows = n_rows;
-                    c.onepass.width = width;
-                    c.onepass.n_states = Sx;
-                    c.onepass.skip_base = skip_base;
-                    c.onepass.fin_base = fin_base;
-                    c.onepass.n_outcomes = n_out;
-                    c.onepass.n_slots = n_slots;
-                    c.onepass.out_ext = upload(out_ext, c.owned);
-                    c.onepass.out_res = upload(out_res, c.owned);
-                    c.onepass.max_slots = max_slots;
-                    c.onepass.xcol = upload(xcol, c.owned);
-                    c.onepass.pair_col = upload(pair_col, c.owned);
-                    c.onepass.init_slots = upload(init, c.owned);
-                    c.onepass.n_init = static_cast<uint32_t>(init.size());
-                    c.onepass.enabled = 1;
-                    // chunk-walk variant of the table (kernels/chunkwalk.cu): a dead automaton keeps scanning to the
-                    // line's '\n' (row DEADSCAN) because the thread goes on with the next line from there
-                    //   rows [0,Sx) states, Sx = DEADSCAN, [Sx+1, Sx+16) SKIP_1..15 (32-byte loads), [Sx+16, ..) outcome rows
-                    {
-                        const uint32_t dscan = Sx, skip2 = Sx + 1, fin2 = Sx + 16, n_rows2 = fin2 + n_out;
-                        if (static_cast<uint64_t>(n_rows2) * width / 4 < (1u << 14)) {
-                            std::vector<uint32_t> rows2(static_cast<size_t>(n_rows2) * width, 0);
-                            for (uint32_t r = 0; r < n_rows2; ++r)
-                                for (uint32_t k = 0; k < width; ++k) {
-                                    uint32_t next = r, slot = 0;
-                                    if (r < Sx) {
-                                        if (k == 0x0A) {
-                                            next = fin2 + A.outcome_of[r];
-                                            slot = len_slot;
-                                        } else if (k < 128 || k - 128 < j_of_col.size()) {
-                                            const uint32_t j = k < 128 ? A.jcls[k] : j_of_col[k - 128];
-                                            const uint32_t ent = A.trans[static_cast<size_t>(r) * J + j];
-                                            if ((ent & 0xFFFFu) == 0xFFFFu) next = dscan;
-                                            else next = ent & 0xFFFFu, slot = ent >> 16;
-                                        } else {
-                                            next = dscan;  // padding column, never addressed
-                                        }
-                                    } else if (r == dscan) {
-                                        if (k == 0x0A) next = fin2, slot = len_slot;  // outcome 0 = MISS
-                                    } else if (r < fin2) {
-                                        next = r == skip2 ? 0u : r - 1;  // SKIP chain
-                                    }
-                                    rows2[static_cast<size_t>(r) * width + k] = (next << 16) | slot;
-                                }
-                            c.chunkwalk = c.onepass;
-                            c.chunkwalk.rows = upload(rows2, c.owned);
-                            c.chunkwalk.n_rows = n_rows2;
-                            c.chunkwalk.skip_base = skip2;
-                            c.chunkwalk.fin_base = fin2;
-                        }
-                    }
-                }
-            }
-        }
-        // fused walk: the same one-pass automaton laid out as ONE tail table (host/tails.hpp format) that every line walks, behind
-        // the newline index K1 — lanes claim consecutive lines (kernels/tailwalk.cu, `all` mode): no chunk ownership, no
-        // look-back, no bucket pass
+        // fused walk: the one-pass automaton of host/fused.hpp (DFA x capture automata folded into one automaton) laid out as ONE
+        // tail table (host/tails.hpp format) that every line walks, behind the newline index K1 — lanes claim consecutive lines
+        // (kernels/tailwalk.cu, `all` mode): no bucket pass
         if (fused.available && !std::getenv("GORP_NO_FUSEDWALK")) {
             const TailSet FT = build_fused_tailset(fused, m, c.max_slots);
             const TailImage img = build_tail_image(FT, c.max_slots);
@@ -687,10 +545,6 @@ void build_device(DeviceCtx& c, const DeviceModel& m, const FusedAutomaton& fuse
                 upload_tail_image(img, FT, c.max_slots, c.fused_tail, c.owned);
                 c.fused_tail.enabled = tailwalk_smem_bytes(c.fused_tail, 256) <= 200 * 1024 ? 1u : 0u;
             }
-            // measured (profiles/README.md round 2): config #2 K0c 11.46 ms vs K1 + fused walk 9.98 ms per 100 M lines, config #1 3.35 vs
-            // 2.67 ms per 40 M lines -> the fused walk is the default, K0c stays as a tier (GORP_SMALL_PATH=chunkwalk)
-            c.fusedwalk_default = true;
-            if (const char* f = std::getenv("GORP_SMALL_PATH")) c.fusedwalk_default = std::string(f) != "chunkwalk";
         }
         c.cap.cls = upload(m.symbols.classmap, c.owned);
         c.cap.n_classes = m.symbols.n_classes;
@@ -772,13 +626,6 @@ struct Timer {
             cudaEventRecord(c.ev[0], s);
         }
     }
-    // a retry re-measures from here: the slots recorded since `n` are dropped
-    int position() const { return c.n_ev; }
-    void rewind(int n) {
-        if (!on || n > c.n_ev) return;
-        c.n_ev = n;
-        cudaEventRecord(c.ev[n], s);
-    }
     void mark(const char* name, int launches) {
         c.launches += launches;
         if (!on || c.n_ev >= kMaxTimed) return;
@@ -787,177 +634,6 @@ struct Timer {
         cudaEventRecord(c.ev[c.n_ev], s);
     }
 };
-
-// Text form through the chunk-walk one-pass kernel. Returns false when the batch has to take another path.
-bool run_chunkwalk(DeviceCtx& c, const uint16_t* d_text, int64_t n_units, cudaStream_t stream, Timer& tm, int64_t* d_scalars,
-                   int64_t& n_lines, gorp_device_result* out) {
-    if (n_units <= 0 || c.force_general || c.force_twopass || !c.chunkwalk.enabled) return false;
-    if (reinterpret_cast<uintptr_t>(d_text) & 31) return false;  // the walk uses 256-bit loads
-    uint32_t threads = 0;
-    if (!k0_chunkwalk_plan(c.chunkwalk, &threads)) return false;
-    Launch L{stream, c.sm_count};
-    c.hist.reserve((c.n_ext + 2) * 8);
-    bool exact = false;
-    const int tm_pos = tm.position();
-    for (int attempt = 0; attempt < 2; ++attempt) {
-        tm.rewind(tm_pos);
-        OnePassParams P{};
-        P.text = d_text;
-        P.n_units = n_units;
-        P.tile_units = threads * kChunkUnits;
-        P.per = 0;
-        if (const char* f = std::getenv("GORP_CW_PREFETCH")) P.per = static_cast<uint32_t>(std::atoi(f));
-        P.n_tiles = (n_units + P.tile_units - 1) / P.tile_units;
-        P.a = c.chunkwalk;
-        P.slots_per_ext = c.d_slots;
-        P.n_ext = c.n_ext;
-        P.span_stride = c.max_slots;
-        // look-back state: [status n_tiles][ticket (8 B)][totals 3 x int64]
-        const size_t state_bytes = static_cast<size_t>(P.n_tiles) * 8 + 8 + 24;
-        c.tile_state.reserve(std::max<size_t>(state_bytes, kTileStateMinBytes));
-        int64_t cap_lines = static_cast<int64_t>(static_cast<double>(n_units) * c.lines_per_unit * 1.25) + 4096;
-        if (exact) cap_lines = n_lines + 16;
-        if (const char* f = std::getenv("GORP_PAD_ROWS")) cap_lines += std::atoll(f);
-        c.ext_id.reserve(static_cast<size_t>(cap_lines + 1) * 4);
-        c.line_off.reserve(static_cast<size_t>(cap_lines + 2) * 8);
-        c.spans.reserve((static_cast<size_t>(cap_lines) * c.max_slots + 4) * 4);
-        P.ext_id = c.ext_id.as<int32_t>();
-        P.line_off = c.line_off.as<int64_t>();
-        P.spans = c.spans.as<int32_t>();
-        P.hist = c.hist.as<unsigned long long>();
-        P.cap_lines = cap_lines;
-        unsigned char* st = c.tile_state.as<unsigned char>();
-        P.tile_status = reinterpret_cast<unsigned long long*>(st);
-        P.ticket = reinterpret_cast<unsigned int*>(st + static_cast<size_t>(P.n_tiles) * 8);
-        P.totals = reinterpret_cast<int64_t*>(st + static_cast<size_t>(P.n_tiles) * 8 + 8);
-        CK(cudaMemsetAsync(st, 0, state_bytes, stream));
-        CK(cudaMemsetAsync(c.hist.p, 0, (c.n_ext + 2) * 8, stream));
-        if (std::getenv("GORP_ONEPASS_DEBUG"))
-            std::fprintf(stderr, "[chunkwalk debug] threads=%u grid=%d smem=%zu tiles=%lld n_slots=%u rows=%u width=%u cap_lines=%lld text=%p ext=%p off=%p spans=%p state=%p\n",
-                         threads, k0_chunkwalk_grid(L, P, threads), chunkwalk_smem_bytes(P.a, threads), static_cast<long long>(P.n_tiles),
-                         P.a.n_slots, P.a.n_rows, P.a.width, static_cast<long long>(cap_lines), static_cast<const void*>(d_text), static_cast<void*>(P.ext_id),
-                         static_cast<void*>(P.line_off), static_cast<void*>(P.spans), static_cast<void*>(st));
-        const bool debug = std::getenv("GORP_ONEPASS_DEBUG") != nullptr;
-        const int grid = k0_chunkwalk_grid(L, P, threads);
-        if (debug) {
-            c.debug.reserve(static_cast<size_t>(grid) * 16 * 8);
-            CK(cudaMemsetAsync(c.debug.p, 0, static_cast<size_t>(grid) * 16 * 8, stream));
-            P.debug = c.debug.as<long long>();
-        }
-        k0_chunkwalk_extract(L, P, threads);
-        tm.mark("k0_chunkwalk_extract", 1);
-        CK(cudaGetLastError());
-        int64_t totals[3] = {0, 0, 0};
-        CK(cudaMemcpyAsync(totals, P.totals, 24, cudaMemcpyDeviceToHost, stream));
-        CK(cudaStreamSynchronize(stream));
-        if (debug) {  // CTAs per SM, tiles per CTA, spread of the CTA run times
-            std::vector<long long> h(static_cast<size_t>(grid) * 16);
-            CK(cudaMemcpy(h.data(), c.debug.p, h.size() * 8, cudaMemcpyDeviceToHost));
-            std::vector<int> per_sm(1024, 0);
-            long long t_min = h[2], t_max = h[3], tiles_min = h[1], tiles_max = h[1], late = 0;
-            double phase[7] = {0, 0, 0, 0, 0, 0, 0};
-            for (int b = 0; b < grid; ++b) {
-                ++per_sm[h[b * 16] & 1023];
-                t_min = std::min(t_min, h[b * 16 + 2]);
-                t_max = std::max(t_max, h[b * 16 + 3]);
-                tiles_min = std::min(tiles_min, h[b * 16 + 1]);
-                tiles_max = std::max(tiles_max, h[b * 16 + 1]);
-                for (int i = 0; i < 7; ++i) phase[i] += static_cast<double>(h[b * 16 + 4 + i]);
-            }
-            {
-                double tot = 0;
-                for (int i = 0; i < 6; ++i) tot += phase[i];
-                std::fprintf(stderr, "[chunkwalk debug] thread-cycles by phase: pre-scan %.1f%%, scan+barrier %.1f%%, walk %.1f%%, wait for first row %.1f%%, "
-                                     "result rows %.1f%%, end-of-tile wait %.1f%% (look-back of warp 0: %.1f%% of one warp's time)\n",
-                             100 * phase[0] / tot, 100 * phase[1] / tot, 100 * phase[2] / tot, 100 * phase[3] / tot, 100 * phase[4] / tot,
-                             100 * phase[5] / tot, 100 * phase[6] * (threads / 32.0) / tot);
-            }
-            for (int b = 0; b < grid; ++b) late += (h[b * 16 + 2] - t_min) > 100000 ? 1 : 0;  // started > 100 us after the first
-            int sm1 = 0, sm2 = 0, sm3 = 0;
-            for (int v : per_sm) sm1 += v == 1, sm2 += v == 2, sm3 += v > 2;
-            std::fprintf(stderr, "[chunkwalk debug] kernel span %.3f ms; SMs with 1/2/>2 CTAs: %d/%d/%d; tiles per CTA %lld..%lld; CTAs started late: %lld\n",
-                         (t_max - t_min) / 1e6, sm1, sm2, sm3, tiles_min, tiles_max, late);
-        }
-        n_lines = totals[0];
-        c.lines_per_unit = std::max(static_cast<double>(n_lines) / static_cast<double>(n_units), 1e-6);
-        if (totals[2] & 1) {  // capacity overflow: rerun once with the exact size
-            exact = true;
-            continue;
-        }
-        CK(cudaMemcpyAsync(d_scalars, P.totals, 8, cudaMemcpyDeviceToDevice, stream));
-        if (out) {
-            out->n_lines = n_lines;
-            out->span_stride = static_cast<int32_t>(c.max_slots);
-            out->d_ext_id = P.ext_id;
-            out->d_line_off = P.line_off;
-            out->d_spans = P.spans;
-            out->d_histogram = c.hist.as<int64_t>();
-            out->d_n_lines = d_scalars;
-        }
-        return true;
-    }
-    return false;
-}
-
-// Text form, newline index + combined DFA through the chunk-walk DFA kernel (K0d): fills c.line_off / c.ext_id.
-// Returns false when the batch has to take K1 + K2 instead.
-bool run_dfawalk(DeviceCtx& c, const uint16_t* d_text, int64_t n_units, cudaStream_t stream, Timer& tm, int64_t* d_scalars,
-                 int64_t& n_lines, bool& ends_with_nl, bool cut) {
-    const DfaWalkDev& table = cut ? c.dfawalk_cut : c.dfawalk;
-    if (n_units <= 0 || c.force_general || c.force_k1k2 || !table.enabled) return false;
-    if (reinterpret_cast<uintptr_t>(d_text) & 31) return false;  // the walk uses 256-bit loads
-    uint32_t threads = 0;
-    bool in_smem = false;
-    if (!k0_dfawalk_plan(table, &threads, &in_smem, cut)) return false;
-    Launch L{stream, c.sm_count};
-    bool exact = false;
-    const int tm_pos = tm.position();
-    for (int attempt = 0; attempt < 2; ++attempt) {
-        tm.rewind(tm_pos);
-        DfaWalkParams P{};
-        P.text = d_text;
-        P.n_units = n_units;
-        const int64_t tile_units = static_cast<int64_t>(threads) * kChunkUnits;
-        P.n_tiles = (n_units + tile_units - 1) / tile_units;
-        P.a = table;
-        P.cut = cut ? 1u : 0u;
-        P.stage_rows = kDfaWalkStagePerThread * threads;
-        const size_t state_bytes = static_cast<size_t>(P.n_tiles) * 8 + 8 + 24;
-        c.tile_state.reserve(std::max<size_t>(state_bytes, kTileStateMinBytes));
-        int64_t cap_lines = static_cast<int64_t>(static_cast<double>(n_units) * c.lines_per_unit * 1.25) + 4096;
-        if (exact) cap_lines = n_lines + 16;
-        c.ext_id.reserve(static_cast<size_t>(cap_lines + 1) * 4);
-        c.line_off.reserve(static_cast<size_t>(cap_lines + 2) * 8);
-        P.ext_id = c.ext_id.as<int32_t>();
-        P.line_off = c.line_off.as<int64_t>();
-        P.cap_lines = cap_lines;
-        unsigned char* st = c.tile_state.as<unsigned char>();
-        P.tile_status = reinterpret_cast<unsigned long long*>(st);
-        P.ticket = reinterpret_cast<unsigned int*>(st + static_cast<size_t>(P.n_tiles) * 8);
-        P.totals = reinterpret_cast<int64_t*>(st + static_cast<size_t>(P.n_tiles) * 8 + 8);
-        CK(cudaMemsetAsync(st, 0, state_bytes, stream));
-        if (std::getenv("GORP_ONEPASS_DEBUG"))
-            std::fprintf(stderr, "[dfawalk debug] threads=%u grid=%d smem=%zu (table %s) tiles=%lld rows=%u K=%u cap_lines=%lld\n", threads,
-                         k0_dfawalk_grid(L, P, threads, in_smem), dfawalk_smem_bytes(P.a, threads, in_smem, cut), in_smem ? "in smem" : "global",
-                         static_cast<long long>(P.n_tiles), P.a.n_rows, P.a.K, static_cast<long long>(cap_lines));
-        k0_dfawalk_scan(L, P, threads, in_smem);
-        tm.mark(cut ? "k0_dfawalk_cut" : "k0_dfawalk_scan", 1);
-        CK(cudaGetLastError());
-        int64_t totals[3] = {0, 0, 0};
-        CK(cudaMemcpyAsync(totals, P.totals, 24, cudaMemcpyDeviceToHost, stream));
-        CK(cudaStreamSynchronize(stream));
-        n_lines = totals[0];
-        ends_with_nl = totals[1] != 0;
-        c.lines_per_unit = std::max(static_cast<double>(n_lines) / static_cast<double>(n_units), 1e-6);
-        if (totals[2] & 1) {  // capacity overflow: rerun once with the exact size
-            exact = true;
-            continue;
-        }
-        CK(cudaMemcpyAsync(d_scalars, P.totals, 8, cudaMemcpyDeviceToDevice, stream));
-        return true;
-    }
-    return false;
-}
 
 // Runs the device pipeline. Text form when d_off == nullptr. Caller holds c.mu and has set the device.
 // Returns n_lines (synchronises once for the text form to size the per-line arrays).
@@ -997,93 +673,36 @@ int64_t run_pipeline_tables(DeviceCtx& c, const uint16_t* d_text, int64_t n_unit
     const int64_t* d_line_off;
     int sep;
     bool ends_with_nl = true;
-    // small definitions, text form: the chunk-owner one-pass kernel K0c, or (GORP_SMALL_PATH=fusedwalk) the newline index K1
-    // followed by the fused walk — every line through the one-pass automaton laid out as a tail table
-    const bool fusedwalk = c.fused_tail.enabled && c.fusedwalk_default && (!d_off || n_units > 0) && !c.force_twopass && !c.force_general &&
-                           !c.force_k1k2 && !c.force_k4 && !c.cap.match_only && c.max_slots > 0 && (reinterpret_cast<uintptr_t>(d_text) & 31) == 0;
-    if (!d_off && !fusedwalk && run_chunkwalk(c, d_text, n_units, stream, tm, d_n_lines, n_lines, out)) return n_lines;
-    bool scanned = false;  // ext_id already holds the combined-DFA result
-    // long or ragged lines: a line index (K1) + lanes that pull lines dynamically (K2b) beats the chunk-owner walk (K0d),
-    // whose threads are stuck with whatever lines start in their chunk
-    // ... unless nearly every walk leaves the combined DFA early (host/tails.hpp): then a chunk owner only walks the heads of
-    // its lines and skips from line to line through the newline masks of the pre-scan — one pass over the text
-    const bool tails_ok = c.tails.enabled && !c.cap.match_only && c.max_slots > 0 && !c.force_general && !c.force_k4 && !c.force_k1k2;
-    const bool cut_walk = !d_off && tails_ok && c.cut_effective && c.dfa_tier != 2 && c.dfa_tier != 1;
-    const bool by_lines = !cut_walk && (c.dfa_tier == 2 || c.dfa_tier == 3 || (c.dfa_tier == 0 && c.lines_per_unit < 1.0 / 100.0));
-    bool cut_scanned = false;
-    if (!d_off && !by_lines && !fusedwalk && run_dfawalk(c, d_text, n_units, stream, tm, d_n_lines, n_lines, ends_with_nl, cut_walk)) {
-        sep = 1;
-        scanned = true;
-        cut_scanned = cut_walk;
-        d_line_off = c.line_off.as<int64_t>();
-    } else if (!d_off) {
+    if (!d_off) {  // text form: the newline index K1
         sep = 1;
         const int64_t n_tiles = (n_units + kNlTile - 1) / kNlTile;
         c.tile_counts.reserve(static_cast<size_t>(n_tiles + 1) * 4);
         c.tile_base.reserve(static_cast<size_t>(n_tiles + 2) * 8);
         c.scan_scratch.reserve(static_cast<size_t>(n_tiles / 4096 + 8) * 8);
         const bool with_masks = !c.force_k1k2 && !c.force_general;  // the count pass leaves the '\n' masks for the scatter pass
-        // K1h (tier GORP_DFA_TIER=3, off by default): the count pass also walks the line heads over the (early-exit) combined-DFA
-        // table — the text of a tile is walked while it is in L2, and K2b's pass over the text is gone. The candidates are
-        // parked per tile and reach ext_id in the scatter pass; K2b takes over when a tile is too dense. Measured (profiles/
-        // README.md round 2): config #4 5.39 ms against 1.92 + 1.86 ms for K1 + K2b, config #3 17.8 against 2.4 + 4.0 ms — a
-        // CTA alternates between a streaming phase and a walk phase with one line per thread, and neither overlaps the other
-        // well enough; K2b's lanes that claim lines from a queue keep 48 warps per SM walking.
-        const DfaWalkDev& head_table = tails_ok ? c.dfawalk_cut : c.dfawalk;
-        bool headwalk = with_masks && !fusedwalk && !c.cap.match_only && !c.force_k4 && c.dfa_tier == 3 && (reinterpret_cast<uintptr_t>(d_text) & 31) == 0 &&
-                        n_units < (1ll << 40) && k1h_plan(head_table);
-        uint32_t* hw_scalars = nullptr;
         if (with_masks) {
             c.nl_masks.reserve(static_cast<size_t>(n_tiles + 4) * 256 * 4);
-            if (headwalk) {
-                c.cand_tmp.reserve(static_cast<size_t>(n_tiles + 4) * kHwCap * 2);
-                hw_scalars = reinterpret_cast<uint32_t*>(d_n_lines + 8);  // 3 words of the scalar block
-                CK(cudaMemsetAsync(hw_scalars, 0, 12, stream));
-                HeadWalkParams H{};
-                H.text = d_text;
-                H.n_units = n_units;
-                H.a = head_table;
-                H.tile_counts = c.tile_counts.as<uint32_t>();
-                H.masks = c.nl_masks.as<uint32_t>();
-                H.cand = c.cand_tmp.as<uint16_t>();
-                H.scalars = hw_scalars;
-                k1h_count_headwalk(L, H);
-            } else {
-                k1_count_newlines_masks(L, d_text, n_units, c.tile_counts.as<uint32_t>(), c.nl_masks.as<uint32_t>());
-            }
+            k1_count_newlines_masks(L, d_text, n_units, c.tile_counts.as<uint32_t>(), c.nl_masks.as<uint32_t>());
         } else {
             k1_count_newlines(L, d_text, n_units, c.tile_counts.as<uint32_t>());
         }
-        tm.mark(headwalk ? "k1h_count_headwalk" : "k1_count_newlines", 1);
+        tm.mark("k1_count_newlines", 1);
         scan_u32_to_i64(L, c.tile_counts.as<uint32_t>(), n_tiles, c.tile_base.as<int64_t>(), c.scan_scratch.as<int64_t>());
         tm.mark("scan_tiles", 3);
         // the one host round trip of the text form: the newline total (and the last unit) size the per-line arrays
         int64_t total_nl = 0;
         uint16_t last_unit = 0x0A;
-        uint32_t hw_dense = 0;
         CK(cudaMemcpyAsync(&total_nl, c.tile_base.as<int64_t>() + n_tiles, 8, cudaMemcpyDeviceToHost, stream));
         if (n_units > 0) CK(cudaMemcpyAsync(&last_unit, d_text + n_units - 1, 2, cudaMemcpyDeviceToHost, stream));
-        if (headwalk) CK(cudaMemcpyAsync(&hw_dense, hw_scalars + 1, 4, cudaMemcpyDeviceToHost, stream));
         CK(cudaStreamSynchronize(stream));
         n_lines = total_nl + (last_unit != 0x0A ? 1 : 0);
         ends_with_nl = last_unit == 0x0A;
         if (n_units > 0) c.lines_per_unit = std::max(static_cast<double>(n_lines) / static_cast<double>(n_units), 1e-6);
         c.line_off.reserve(static_cast<size_t>(total_nl + 3) * 8);
-        // the candidates are those of `head_table`: usable when the stages below make the same choice (with_tails) and no tile
-        // overflowed its candidate slots
-        headwalk = headwalk && !hw_dense && n_lines > 0 && n_lines < (1ll << 32);
-        if (headwalk) c.ext_id.reserve((static_cast<size_t>(n_lines) + 1) * 4);
-        if (with_masks)
-            k1_scatter_masks(L, c.nl_masks.as<uint32_t>(), n_units, c.tile_base.as<int64_t>(), c.line_off.as<int64_t>(),
-                             headwalk ? c.cand_tmp.as<uint16_t>() : nullptr, headwalk ? hw_scalars + 2 : nullptr,
-                             headwalk ? c.ext_id.as<int32_t>() : nullptr);
+        if (with_masks) k1_scatter_masks(L, c.nl_masks.as<uint32_t>(), n_units, c.tile_base.as<int64_t>(), c.line_off.as<int64_t>());
         else k1_scatter_newlines(L, d_text, n_units, c.tile_base.as<int64_t>(), c.line_off.as<int64_t>());
         k1_finish(L, d_text, n_units, c.tile_base.as<int64_t>() + n_tiles, c.line_off.as<int64_t>(), d_n_lines);
         tm.mark("k1_scatter_newlines", 2);
-        if (headwalk) {
-            scanned = true;
-            cut_scanned = tails_ok;
-        }
         d_line_off = c.line_off.as<int64_t>();
     } else {
         sep = 0;
@@ -1093,9 +712,15 @@ int64_t run_pipeline_tables(DeviceCtx& c, const uint16_t* d_text, int64_t n_unit
     const size_t nl = static_cast<size_t>(n_lines);
     c.ext_id.reserve((nl + 1) * 4);
     c.hist.reserve((c.n_ext + 2) * 8);
+    // small definitions: the fused walk — every line through the one-pass automaton laid out as a tail table
+    const bool fusedwalk = c.fused_tail.enabled && (!d_off || n_units > 0) && !c.force_twopass && !c.force_general && !c.force_k1k2 &&
+                           !c.force_k4 && !c.cap.match_only && c.max_slots > 0 && (reinterpret_cast<uintptr_t>(d_text) & 31) == 0;
     if (fusedwalk && n_lines > 0 && n_lines < (1ll << 32)) {
         const uint32_t stride = c.max_slots;
-        c.spans.reserve((nl * stride + 4) * 4);
+        size_t rows = nl;  // GORP_PAD_ROWS (diagnostics): spare rows, which shift every allocation that follows
+        if (const char* f = std::getenv("GORP_PAD_ROWS")) rows += static_cast<size_t>(std::atoll(f));
+        c.ext_id.reserve((rows + 1) * 4);
+        c.spans.reserve((rows * stride + 4) * 4);
         c.buckets.reserve(64);
         uint32_t* ticket = c.buckets.as<uint32_t>();  // [item ticket, n_long]
         CK(cudaMemsetAsync(ticket, 0, 8, stream));
@@ -1150,9 +775,8 @@ int64_t run_pipeline_tables(DeviceCtx& c, const uint16_t* d_text, int64_t n_unit
                             !c.force_k1k2 && n_lines > 0 && n_lines < (1ll << 32) && (reinterpret_cast<uintptr_t>(d_text) & 31) == 0 &&
                             (sep == 1 || n_units > 0);
     const DfaWalkDev& walk_table = with_tails ? c.dfawalk_cut : c.dfawalk;
-    bool candidates = cut_scanned;  // ext_id holds candidates of the cut table: only the tail walk may follow (its conditions are those of with_tails)
-    if (scanned) {
-    } else if ((sep == 1 || with_tails) && !c.force_general && !c.force_k1k2 && (reinterpret_cast<uintptr_t>(d_text) & 31) == 0 &&
+    bool candidates = false;  // ext_id holds candidates of the cut table (K2b walked it): only the tail walk may follow
+    if ((sep == 1 || with_tails) && !c.force_general && !c.force_k1k2 && (reinterpret_cast<uintptr_t>(d_text) & 31) == 0 &&
                k2b_linewalk_plan(walk_table, &lw_threads, &lw_smem)) {
         candidates = with_tails;
         LineWalkParams W{};

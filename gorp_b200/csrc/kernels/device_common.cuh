@@ -1,4 +1,4 @@
-// Device helpers shared by the fast tiers (fast.cu) and the fused kernel (fused.cu). Header-only (no -rdc).
+// Device helpers shared by the kernel files (fast.cu, dfawalk.cu, capwalk.cu, tailwalk.cu, ...). Header-only (no -rdc).
 #pragma once
 #include "kernels.cuh"
 
@@ -24,18 +24,7 @@ __device__ __forceinline__ uint32_t unit_at(const uint4& v, int k) {
     return (k & 1) ? (w >> 16) : (w & 0xFFFFu);
 }
 
-// ---- shared by the chunk-walk kernels (chunkwalk.cu, dfawalk.cu): decoupled look-back status words, text loads, newline masks
-constexpr unsigned long long kStAgg = 1ull << 62, kStPre = 2ull << 62;
-
-__device__ __forceinline__ unsigned long long ld_acquire(const unsigned long long* p) {
-    unsigned long long v;
-    asm volatile("ld.acquire.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ void st_release(unsigned long long* p, unsigned long long v) {
-    asm volatile("st.release.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
-}
-
+// ---- text loads, newline masks
 // 8 units at text position `pos` (a multiple of 8); units at or beyond n_units read as '\n'
 __device__ __forceinline__ uint4 load_chunk(const uint16_t* __restrict__ text, int64_t pos, int64_t n_units) {
     if (pos + 8 <= n_units) return __ldg(reinterpret_cast<const uint4*>(text + pos));

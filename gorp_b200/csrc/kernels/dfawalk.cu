@@ -1,20 +1,16 @@
-// K0d — chunk-walk DFA kernel (sm_100a): newline index + combined-DFA scan of the text form in ONE pass over the text,
-// for definitions whose one-pass product automaton (host/fused.hpp) is not available. Stands in for
-// PolyMatcher.match + Automata.step/accept (reference autom/PolyMatcher.java:123-133, autom/Automata.java:133-139)
-// and the first-index dispatch of Gorp.java:166-167; the capture half runs afterwards, bucketed by extraction
-// (kernels/capwalk.cu).
+// K2b — line-walk DFA kernel (sm_100a): the combined-DFA scan over an existing line index (K1's, or the caller's offsets
+// in the List<String> form). Stands in for PolyMatcher.match + Automata.step/accept (reference autom/PolyMatcher.java:123-133,
+// autom/Automata.java:133-139) and the first-index dispatch of Gorp.java:166-167; the capture half runs afterwards, bucketed
+// by extraction (kernels/capwalk.cu, kernels/tailwalk.cu).
 //
-// Work decomposition = kernels/chunkwalk.cu: the text is cut into chunks of kChunkUnits units, one per thread; a CTA
-// takes a tile of blockDim.x consecutive chunks by in-order ticket; a thread owns the lines whose preceding '\n' lies
-// in its chunk and walks them one after the other with 256-bit loads, so every lane walks about kChunkUnits units
-// whatever the line lengths are. Differences:
-//   * the automaton is the class-indexed combined DFA (u16 next-row entries, K = classes + 1 columns, the last column
-//     is '\n'); it lives in shared memory when it fits, otherwise it is read through L1/L2 (template kSmem);
-//       rows [0,S) states | S = DEADSCAN (dead, keeps scanning to the line's '\n') | S+1..S+15 = SKIP_1..15 (units that
-//       precede the line in its first 32-byte block) | fin_base = S+16: FIN(-1), FIN(0..E-1) absorbing outcome rows
-//   * a finished line is only (extraction id, start): rows are staged in shared memory by tile-local row index and go
-//     out after the walk with fully coalesced stores, once the tile's first row is known (decoupled look-back by warp 0
-//     during the walk).
+// The automaton is the class-indexed combined DFA (u16 next-row entries, K = classes + 1 columns, the last column is '\n'),
+// or its early-exit variant when the tail walk follows (host/walktables.hpp); it lives in shared memory when it fits,
+// otherwise it is read through L1/L2 (template kSmem):
+//     rows [0,S) states | S = DEADSCAN (dead, keeps scanning to the line's '\n') | S+1..S+15 = SKIP_1..15 (units that
+//     precede the line in its first 32-byte block) | fin_base = S+16: FIN(-1), FIN(0..E-1) absorbing outcome rows
+// A WARP takes work items of kLineItemLines consecutive lines, every lane walks one line at a time in 32-byte blocks and
+// claims its next line one line ahead (ballot-ranked, no atomics), so lanes stay busy whatever the line lengths are (long or
+// ragged lines, 10 KB outliers). A finished line writes its extraction id (or -1; with the early-exit table: the candidate).
 #include "device_common.cuh"
 
 namespace gorp {
@@ -32,47 +28,6 @@ __device__ __forceinline__ uint32_t lds16(uint32_t addr) {
 // newline mask of 16 units (bit k = unit k is '\n')
 __device__ __forceinline__ uint32_t nl_mask16(const Units16& u) {
     return nl_bits4(u.a.x, u.a.y) | (nl_bits4(u.a.z, u.a.w) << 4) | (nl_bits4(u.b.x, u.b.y) << 8) | (nl_bits4(u.b.z, u.b.w) << 12);
-}
-
-// exclusive prefix of the tile's line count over all earlier tiles (decoupled look-back, called by every lane of warp 0;
-// publishes the tile's aggregate first). 128 predecessors per probe: see kernels/chunkwalk.cu.
-__device__ __forceinline__ unsigned long long lookback_exclusive(unsigned long long* tile_status, int64_t tile, uint32_t total,
-                                                                 uint32_t lane) {
-    unsigned long long pre = 0;
-    if (tile == 0) return 0;
-    if (lane == 0) st_release(tile_status + tile, kStAgg | static_cast<unsigned long long>(total));
-    for (int64_t j = tile - 1;; j -= 128) {
-        unsigned long long v[4];
-#pragma unroll
-        for (int m = 0; m < 4; ++m) {
-            const int64_t idx = j - (lane * 4 + m);
-            v[m] = idx >= 0 ? ld_acquire(tile_status + idx) : kStPre;  // before tile 0: an empty inclusive prefix
-        }
-#pragma unroll
-        for (int m = 0; m < 4; ++m) {
-            const int64_t idx = j - (lane * 4 + m);
-            while ((v[m] >> 62) == 0) {
-                __nanosleep(32);
-                v[m] = ld_acquire(tile_status + idx);
-            }
-        }
-        unsigned long long part = 0;  // aggregates up to and including the lane's nearest inclusive prefix
-        bool has = false;
-#pragma unroll
-        for (int m = 0; m < 4; ++m)
-            if (!has) {
-                part += v[m] & ~(3ull << 62);
-                has = (v[m] >> 62) == 2;
-            }
-        const uint32_t pmask = __ballot_sync(0xffffffffu, has);
-        const uint32_t firstp = pmask ? static_cast<uint32_t>(__ffs(pmask)) - 1u : 32u;
-        unsigned long long l = lane <= firstp ? part : 0ull;
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) l += __shfl_xor_sync(0xffffffffu, l, o);
-        pre += l;
-        if (pmask) break;
-    }
-    return pre;
 }
 
 template <bool kSmem>
@@ -141,252 +96,6 @@ __device__ __noinline__ uint32_t dw_bounded16(const DfaWalkDev& A, uint32_t st, 
     return st;
 }
 
-// kCut: the table is the early-exit variant (host/walktables.hpp: build_dfawalk_table_cut) — a walk may reach a FIN row long
-// before the line's '\n', so the thread finds its next line through the newline bit mask of its chunk (kept from the
-// pre-scan) instead of scanning on; nothing beyond the head of a line is read a second time.
-template <bool kSmem, bool kCut>
-__global__ void __launch_bounds__(1024, 1) dfawalk_kernel(DfaWalkParams P) {
-    extern __shared__ __align__(128) unsigned char smem[];
-    const uint32_t kT = blockDim.x;
-    const DfaWalkDev& A = P.a;
-    constexpr uint32_t C = kChunkUnits;
-    const uint32_t row_bytes = A.K * 2;
-    const uint32_t table_bytes = kSmem ? ((A.n_rows * row_bytes + 15u) & ~15u) : 0u;
-    // ---- carve shared memory: [table][cx 128 x u32][staged ext][staged start][kCut: newline masks, 32 bytes per thread]
-    uint32_t* s_cx = reinterpret_cast<uint32_t*>(smem + table_bytes);
-    int32_t* s_sext = reinterpret_cast<int32_t*>(s_cx + 128);
-    uint32_t* s_sstart = reinterpret_cast<uint32_t*>(s_sext + P.stage_rows);
-    unsigned char* s_masks = reinterpret_cast<unsigned char*>(s_sstart + P.stage_rows);  // [thread][32]: bit k of byte j = unit 8j + k
-    __shared__ uint32_t s_warp[32];
-    __shared__ long long s_tile, s_base;
-    __shared__ int s_skip_writes;
-    __shared__ unsigned int s_flag;  // (tile + 1) once s_base / s_skip_writes of the tile are valid
-
-    const uint32_t tab_abs = static_cast<uint32_t>(__cvta_generic_to_shared(smem));
-    const uint32_t cx_abs = static_cast<uint32_t>(__cvta_generic_to_shared(s_cx));
-    const unsigned char* __restrict__ tab_g = reinterpret_cast<const unsigned char*>(A.table);
-    if (kSmem) {
-        const uint32_t n16 = (A.n_rows * row_bytes + 15u) / 16u;  // the global copy is padded to 16 bytes
-        const uint4* src = reinterpret_cast<const uint4*>(A.table);
-        uint4* dst = reinterpret_cast<uint4*>(smem);
-        for (uint32_t i = threadIdx.x; i < n16; i += kT) dst[i] = __ldg(src + i);
-    }
-    for (uint32_t i = threadIdx.x; i < 128; i += kT) s_cx[i] = (kSmem ? tab_abs : 0u) + __ldg(A.cls128 + i);
-    if (threadIdx.x == 0) s_flag = 0;
-
-    const uint32_t fin_base = A.fin_base, skip0 = A.n_states;  // SKIP_k = skip0 + k
-    const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5, n_warps = kT >> 5;
-
-    long long ticket_ahead = threadIdx.x == 0 ? static_cast<long long>(atomicAdd(P.ticket, 1u)) : 0;
-    for (;;) {
-        __syncthreads();  // the previous tile no longer uses s_tile / s_warp / the staging area; table setup done
-        if (threadIdx.x == 0) s_tile = ticket_ahead;
-        __syncthreads();
-        const int64_t tile = s_tile;
-        if (tile >= P.n_tiles) break;
-        if (threadIdx.x == 0) ticket_ahead = static_cast<long long>(atomicAdd(P.ticket, 1u));
-        const int64_t tile0 = tile * kT * static_cast<int64_t>(C);
-        {  // start fetching this tile's chunks now; the pre-scan consumes them in order
-            const int64_t n0 = tile0 + static_cast<int64_t>(threadIdx.x) * C;
-            if (n0 + C <= P.n_units) asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(P.text + n0), "n"(C * 2) : "memory");
-        }
-        // ---- newline pre-scan, per warp with coalesced loads: iteration i reads the 32 x 16 bytes of lane i's chunk;
-        // a '\n' at position p counts when it starts a line (p + 1 < n_units). Lane i keeps the count and the first.
-        uint32_t cnt = 0, first = 0;
-        {
-            const int64_t wbase = tile0 + static_cast<int64_t>(warp) * 32 * C;
-            const bool inside = wbase + 32 * static_cast<int64_t>(C) + 1 <= P.n_units;
-            if (wbase < P.n_units) {
-#pragma unroll 4
-                for (uint32_t i = 0; i < 32; ++i) {
-                    const int64_t p = wbase + i * C + lane * 8;
-                    uint32_t m;
-                    if (inside) {
-                        const uint4 v = __ldg(reinterpret_cast<const uint4*>(P.text + p));
-                        m = nl_bits4(v.x, v.y) | (nl_bits4(v.z, v.w) << 4);
-                    } else {
-                        const uint4 v = load_chunk(P.text, p, P.n_units);
-                        m = nl_bits4(v.x, v.y) | (nl_bits4(v.z, v.w) << 4);
-                        const int64_t room = P.n_units - 1 - p;  // positions (relative to p) that count: [0, room)
-                        m = room <= 0 ? 0u : (room < 8 ? m & ((1u << static_cast<uint32_t>(room)) - 1u) : m);
-                    }
-                    if (kCut) {  // the chunk's mask goes through shared memory: lane j holds byte j of the chunk of thread (warp, i)
-                        s_masks[(warp * 32 + i) * 32 + lane] = static_cast<unsigned char>(m);
-                    } else {
-                        const uint32_t tot = __reduce_add_sync(0xffffffffu, static_cast<uint32_t>(__popc(m)));
-                        const uint32_t has = __ballot_sync(0xffffffffu, m != 0);
-                        const uint32_t fl = has ? static_cast<uint32_t>(__ffs(has)) - 1u : 0u;
-                        const uint32_t mf = __shfl_sync(0xffffffffu, m, fl);
-                        if (lane == i) {
-                            cnt = tot;
-                            first = fl * 8 + static_cast<uint32_t>(__ffs(mf)) - 1u;
-                        }
-                    }
-                }
-            } else if (kCut) {
-                for (uint32_t i = 0; i < 32; ++i) s_masks[(warp * 32 + i) * 32 + lane] = 0;
-            }
-        }
-        uint32_t nlm[8] = {0, 0, 0, 0, 0, 0, 0, 0};  // kCut: bit p of the 256-bit mask = unit p of this thread's chunk starts... is a '\n' that starts a line
-        if (kCut) {
-            __syncwarp();
-            const uint4 lo4 = *reinterpret_cast<const uint4*>(s_masks + threadIdx.x * 32), hi4 = *reinterpret_cast<const uint4*>(s_masks + threadIdx.x * 32 + 16);
-            nlm[0] = lo4.x, nlm[1] = lo4.y, nlm[2] = lo4.z, nlm[3] = lo4.w, nlm[4] = hi4.x, nlm[5] = hi4.y, nlm[6] = hi4.z, nlm[7] = hi4.w;
-            bool found = false;
-#pragma unroll
-            for (int w = 0; w < 8; ++w) {
-                cnt += static_cast<uint32_t>(__popc(nlm[w]));
-                if (!found && nlm[w]) {
-                    first = w * 32 + static_cast<uint32_t>(__ffs(nlm[w])) - 1u;
-                    found = true;
-                }
-            }
-        }
-        const bool line0 = tile == 0 && threadIdx.x == 0 && P.n_units > 0;  // the line at offset 0
-        const uint32_t mine = cnt + (line0 ? 1u : 0u);
-
-        // ---- block scan of the line counts; warp 0 then resolves the tile's first row by decoupled look-back
-        uint32_t incl = mine;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o);
-            if (lane >= o) incl += t;
-        }
-        if (lane == 31) s_warp[warp] = incl;
-        __syncthreads();
-        uint32_t wsum = 0, total = 0;
-        for (uint32_t w = 0; w < n_warps; ++w) {
-            const uint32_t x = s_warp[w];
-            if (w < warp) wsum += x;
-            total += x;
-        }
-        const uint32_t row0 = wsum + incl - mine;  // tile-local index of this thread's first row
-        if (warp == 0) {
-            const unsigned long long pre = lookback_exclusive(P.tile_status, tile, total, lane);
-            if (lane == 0) {
-                const long long line_end = static_cast<long long>(pre) + total;
-                st_release(P.tile_status + tile, kStPre | static_cast<unsigned long long>(line_end));
-                const bool over = line_end > P.cap_lines;
-                if (over) atomicOr(reinterpret_cast<unsigned long long*>(P.totals + 2), 1ull);
-                if (tile == P.n_tiles - 1) {
-                    P.totals[0] = line_end;
-                    P.totals[1] = P.text[P.n_units - 1] == 0x0A ? 1 : 0;
-                    // line i spans [line_off[i], line_off[i+1] - 1): a text that does not end in '\n' gets n_units + 1
-                    if (!over) P.line_off[line_end] = P.n_units + (P.text[P.n_units - 1] == 0x0A ? 0 : 1);
-                }
-                s_base = static_cast<long long>(pre);
-                s_skip_writes = over ? 1 : 0;
-                __threadfence_block();
-                *reinterpret_cast<volatile unsigned int*>(&s_flag) = static_cast<unsigned int>(tile + 1);
-            }
-            __syncwarp();
-        }
-
-        // ---- walk the owned lines one after the other; positions are tile-relative
-        if (mine) {
-            const uint32_t c_end = (threadIdx.x + 1) * C;  // tile-relative end of the chunk
-            const int64_t n_rel = P.n_units - tile0;       // tile-relative end of the text
-            uint32_t start = line0 ? 0u : threadIdx.x * C + first + 1;
-            uint32_t q = start & ~15u;
-            uint32_t lo = start & 15u;
-            uint32_t st = lo ? skip0 + lo : 0u;
-            uint32_t row = row0;
-            for (;;) {
-                const Units16 u = load_units16(P.text, tile0 + q, P.n_units);
-                if (((u.a.x | u.a.y | u.a.z | u.a.w | u.b.x | u.b.y | u.b.z | u.b.w) & 0xFF80FF80u) == 0u) {
-                    st = dw_step<kSmem, 0>(st, u.a.x, cx_abs, row_bytes, tab_g);
-                    st = dw_step<kSmem, 2>(st, u.a.x, cx_abs, row_bytes, tab_g);
-                    st = dw_step<kSmem, 0>(st, u.a.y, cx_abs, row_bytes, tab_g);
-                    st = dw_step<kSmem, 2>(st, u.a.y, cx_abs, row_bytes, tab_g);
-                    st = dw_step<kSmem, 0>(st, u.a.z, cx_abs, row_bytes, tab_g);
-                    st = dw_step<kSmem, 2>(st, u.a.z, cx_abs, row_bytes, tab_g);
-                    st = dw_step<kSmem, 0>(st, u.a.w, cx_abs, row_bytes, tab_g);
-                    st = dw_step<kSmem, 2>(st, u.a.w, cx_abs, row_bytes, tab_g);
-                    st = dw_step<kSmem, 0>(st, u.b.x, cx_abs, row_bytes, tab_g);
-                    st = dw_step<kSmem, 2>(st, u.b.x, cx_abs, row_bytes, tab_g);
-                    st = dw_step<kSmem, 0>(st, u.b.y, cx_abs, row_bytes, tab_g);
-                    st = dw_step<kSmem, 2>(st, u.b.y, cx_abs, row_bytes, tab_g);
-                    st = dw_step<kSmem, 0>(st, u.b.z, cx_abs, row_bytes, tab_g);
-                    st = dw_step<kSmem, 2>(st, u.b.z, cx_abs, row_bytes, tab_g);
-                    st = dw_step<kSmem, 0>(st, u.b.w, cx_abs, row_bytes, tab_g);
-                    st = dw_step<kSmem, 2>(st, u.b.w, cx_abs, row_bytes, tab_g);
-                } else {
-                    st = dw_slow8<kSmem>(A, st, u.a, cx_abs, tab_abs, row_bytes, tab_g);
-                    st = dw_slow8<kSmem>(A, st, u.b, cx_abs, tab_abs, row_bytes, tab_g);
-                }
-                if (st >= fin_base) {  // the line ended inside these 16 units: at its first '\n' at or after `start`
-                    uint32_t nl;  // tile-relative position of the line's '\n' (kCut: 0xFFFFFFFF when it lies beyond the chunk)
-                    if (kCut) {
-                        // the walk may have stopped anywhere in the line: the next '\n' of this thread's chunk at or after `start`
-                        const uint32_t c0 = threadIdx.x * C;
-                        nl = 0xFFFFFFFFu;
-                        if (start < c0 + C) {
-                            const uint32_t rel = start > c0 ? start - c0 : 0u;  // (the line at offset 0 of the text starts before the first '\n')
-#pragma unroll
-                            for (int w = 0; w < 8; ++w) {
-                                uint32_t mw = nlm[w];
-                                if (static_cast<uint32_t>(w) == (rel >> 5)) mw &= ~0u << (rel & 31u);
-                                else if (static_cast<uint32_t>(w) < (rel >> 5)) mw = 0;
-                                if (nl == 0xFFFFFFFFu && mw) nl = c0 + w * 32 + static_cast<uint32_t>(__ffs(mw)) - 1u;
-                            }
-                        }
-                    } else {
-                        uint32_t m = nl_mask16(u);
-                        if (q < start) m &= ~0u << (start - q);
-                        nl = q + static_cast<uint32_t>(__ffs(m)) - 1u;
-                    }
-                    const int32_t ext = static_cast<int32_t>(st - fin_base) - 1;
-                    if (row < P.stage_rows) {
-                        s_sext[row] = ext;
-                        s_sstart[row] = start;
-                    } else {  // denser tile than the staging area: this row goes out directly
-                        while (*reinterpret_cast<volatile unsigned int*>(&s_flag) != static_cast<unsigned int>(tile + 1)) {
-                            __nanosleep(64);
-                        }
-                        __threadfence_block();
-                        if (!*reinterpret_cast<volatile int*>(&s_skip_writes)) {
-                            const int64_t g = *reinterpret_cast<volatile long long*>(&s_base) + row;
-                            P.ext_id[g] = ext;
-                            P.line_off[g] = tile0 + start;
-                        }
-                    }
-                    ++row;
-                    if (nl < c_end && static_cast<int64_t>(nl) + 1 < n_rel) {
-                        start = nl + 1;
-                        q = start & ~15u;
-                        lo = start & 15u;
-                        st = lo ? skip0 + lo : 0u;
-                        continue;
-                    }
-                    break;
-                }
-                q += 16;
-            }
-        }
-        // ---- coalesced copy-out of the staged rows
-        __syncthreads();
-        {
-            while (*reinterpret_cast<volatile unsigned int*>(&s_flag) != static_cast<unsigned int>(tile + 1)) {
-                __nanosleep(64);
-            }
-            __threadfence_block();
-            if (!*reinterpret_cast<volatile int*>(&s_skip_writes)) {
-                const int64_t base = *reinterpret_cast<volatile long long*>(&s_base);
-                const uint32_t n = total < P.stage_rows ? total : P.stage_rows;
-                for (uint32_t i = threadIdx.x; i < n; i += kT) {
-                    P.ext_id[base + i] = s_sext[i];
-                    P.line_off[base + i] = tile0 + s_sstart[i];
-                }
-            }
-        }
-    }
-}
-
-// ------------------------------------------------------------------ K2b: the same automaton over an existing line index
-// Lines come from line_off (K1); a WARP takes work items of kLineItemLines consecutive lines, every lane walks one line
-// at a time in 32-byte blocks and claims its next line one line ahead (ballot-ranked, no atomics), so lanes stay busy
-// whatever the line lengths are (long or ragged lines, 10 KB outliers) — the case the chunk-owner walk above handles
-// badly, because there a thread's work is fixed by where the lines happen to start.
 template <bool kSmem, bool kLines>
 __global__ void __launch_bounds__(768, 2) linewalk_kernel(LineWalkParams P) {
     extern __shared__ __align__(128) unsigned char smem[];
@@ -508,246 +217,10 @@ __global__ void __launch_bounds__(768, 2) linewalk_kernel(LineWalkParams P) {
     }
 }
 
-// ------------------------------------------------------------------ K1h: newline count + head walk in one pass
-// A CTA of 256 threads takes super-tiles of 4 x kNlTile = 32768 units by ticket. Phase 1 is K1's count pass (thread t reads
-// units [128 t, 128 t + 128) with streaming 128-bit loads, leaves the 4 newline mask words and the per-tile counts); the line
-// starts of the super-tile (~230 of them) are listed in shared memory by (tile, ordinal of their '\n' inside the tile).
-// Phase 2: thread i walks the head of line i over the early-exit table in shared memory (the text is in L2 from phase 1)
-// and parks the FIN row it reaches in cand[tile * kHwCap + ordinal]. Other CTAs of the SM stream while this one walks.
-constexpr int kHwThreads = 256;
-constexpr int kHwTiles = 4;
-static_assert(kHwThreads * 128 == kHwTiles * kNlTile, "a thread of K1h covers 128 units");
-
-__device__ __forceinline__ uint4 hw_ld_stream(const uint4* p) {
-    uint4 r;
-    asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p));
-    return r;
-}
-
-__device__ __forceinline__ uint32_t hw_walk_head(const HeadWalkParams& P, int64_t start, uint32_t cx_abs, uint32_t tab_abs, uint32_t row_bytes) {
-    const DfaWalkDev& A = P.a;
-    int64_t q = start & ~int64_t(15);
-    const uint32_t lo = static_cast<uint32_t>(start - q);
-    uint32_t st = lo ? A.n_states + lo : 0u;
-    while (st < A.fin_base) {
-        const Units16 u = load_units16_l2keep(P.text, q, P.n_units);
-        if (((u.a.x | u.a.y | u.a.z | u.a.w | u.b.x | u.b.y | u.b.z | u.b.w) & 0xFF80FF80u) == 0u) {
-            st = dw_step<true, 0>(st, u.a.x, cx_abs, row_bytes, nullptr);
-            st = dw_step<true, 2>(st, u.a.x, cx_abs, row_bytes, nullptr);
-            st = dw_step<true, 0>(st, u.a.y, cx_abs, row_bytes, nullptr);
-            st = dw_step<true, 2>(st, u.a.y, cx_abs, row_bytes, nullptr);
-            st = dw_step<true, 0>(st, u.a.z, cx_abs, row_bytes, nullptr);
-            st = dw_step<true, 2>(st, u.a.z, cx_abs, row_bytes, nullptr);
-            st = dw_step<true, 0>(st, u.a.w, cx_abs, row_bytes, nullptr);
-            st = dw_step<true, 2>(st, u.a.w, cx_abs, row_bytes, nullptr);
-            st = dw_step<true, 0>(st, u.b.x, cx_abs, row_bytes, nullptr);
-            st = dw_step<true, 2>(st, u.b.x, cx_abs, row_bytes, nullptr);
-            st = dw_step<true, 0>(st, u.b.y, cx_abs, row_bytes, nullptr);
-            st = dw_step<true, 2>(st, u.b.y, cx_abs, row_bytes, nullptr);
-            st = dw_step<true, 0>(st, u.b.z, cx_abs, row_bytes, nullptr);
-            st = dw_step<true, 2>(st, u.b.z, cx_abs, row_bytes, nullptr);
-            st = dw_step<true, 0>(st, u.b.w, cx_abs, row_bytes, nullptr);
-            st = dw_step<true, 2>(st, u.b.w, cx_abs, row_bytes, nullptr);
-        } else {
-            st = dw_slow8<true>(A, st, u.a, cx_abs, tab_abs, row_bytes, nullptr);
-            st = dw_slow8<true>(A, st, u.b, cx_abs, tab_abs, row_bytes, nullptr);
-        }
-        q += 16;
-    }
-    return st - A.fin_base;
-}
-
-__global__ void __launch_bounds__(kHwThreads) headwalk_count_kernel(HeadWalkParams P) {
-    extern __shared__ __align__(128) unsigned char smem[];
-    const DfaWalkDev& A = P.a;
-    const uint32_t row_bytes = A.K * 2;
-    const uint32_t table_bytes = (A.n_rows * row_bytes + 15u) & ~15u;
-    uint32_t* s_cx = reinterpret_cast<uint32_t*>(smem + table_bytes);
-    uint16_t* s_start = reinterpret_cast<uint16_t*>(s_cx + 128);  // [kHwTiles][kHwCap] super-tile-relative start - 1 of a line
-    __shared__ uint32_t s_wsum[kHwThreads / 32];
-    __shared__ long long s_super;
-    const uint32_t tab_abs = static_cast<uint32_t>(__cvta_generic_to_shared(smem));
-    const uint32_t cx_abs = static_cast<uint32_t>(__cvta_generic_to_shared(s_cx));
-    {
-        const uint32_t n16 = (A.n_rows * row_bytes + 15u) / 16u;
-        const uint4* src = reinterpret_cast<const uint4*>(A.table);
-        uint4* dst = reinterpret_cast<uint4*>(smem);
-        for (uint32_t i = threadIdx.x; i < n16; i += kHwThreads) dst[i] = __ldg(src + i);
-    }
-    for (uint32_t i = threadIdx.x; i < 128; i += kHwThreads) s_cx[i] = tab_abs + __ldg(A.cls128 + i);
-    const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
-    const int64_t n_tiles = (P.n_units + kNlTile - 1) / kNlTile;
-    const int64_t n_super = (n_tiles + kHwTiles - 1) / kHwTiles;
-    for (;;) {
-        __syncthreads();  // table ready (first iteration); the previous super-tile no longer uses s_start / s_wsum
-        if (threadIdx.x == 0) s_super = static_cast<long long>(atomicAdd(P.scalars, 1u));
-        __syncthreads();
-        const int64_t sup = s_super;
-        if (sup >= n_super) break;
-        const int64_t base_u = sup * (kHwTiles * static_cast<int64_t>(kNlTile));
-        // ---- phase 1: the count pass of K1
-        uint32_t m[4];
-        const int64_t mine = base_u + static_cast<int64_t>(threadIdx.x) * 128;
-        if (mine + 128 <= P.n_units) {
-            const uint4* src = reinterpret_cast<const uint4*>(P.text + mine);
-            uint4 v[16];
-#pragma unroll
-            for (int j = 0; j < 16; ++j) v[j] = hw_ld_stream(src + j);
-#pragma unroll
-            for (int w = 0; w < 4; ++w) {
-                uint32_t mask = 0;
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    const uint4 x = v[w * 4 + j];
-                    mask |= (nl_bits4(x.x, x.y) | (nl_bits4(x.z, x.w) << 4)) << (j * 8);
-                }
-                m[w] = mask;
-            }
-        } else {
-#pragma unroll
-            for (int w = 0; w < 4; ++w) {
-                uint32_t mask = 0;
-                for (int k = 0; k < 32; ++k) {
-                    const int64_t p = mine + w * 32 + k;
-                    if (p < P.n_units && P.text[p] == 0x0A) mask |= 1u << k;
-                }
-                m[w] = mask;
-            }
-        }
-        const int64_t tile = sup * kHwTiles + (warp >> 1);  // the kNlTile tile of this warp pair (64 threads x 128 units)
-        if (tile < n_tiles) *reinterpret_cast<uint4*>(P.masks + tile * 256 + (threadIdx.x & 63u) * 4) = make_uint4(m[0], m[1], m[2], m[3]);
-        const uint32_t cnt = __popc(m[0]) + __popc(m[1]) + __popc(m[2]) + __popc(m[3]);
-        uint32_t incl = cnt;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o);
-            if (lane >= static_cast<uint32_t>(o)) incl += t;
-        }
-        if (lane == 31) s_wsum[warp] = incl;
-        __syncthreads();
-        const uint32_t g = warp >> 1;
-        const uint32_t c_g = s_wsum[2 * g] + s_wsum[2 * g + 1];
-        uint32_t ord = ((warp & 1u) ? s_wsum[warp - 1] : 0u) + incl - cnt;
-        if ((threadIdx.x & 63u) == 0 && tile < n_tiles) {
-            P.tile_counts[tile] = c_g;
-            if (c_g > kHwCap) atomicOr(P.scalars + 1, 1u);
-        }
-#pragma unroll
-        for (int w = 0; w < 4; ++w) {
-            uint32_t mm = m[w];
-            while (mm) {
-                const uint32_t k = static_cast<uint32_t>(__ffs(mm)) - 1u;
-                mm &= mm - 1;
-                if (ord < kHwCap) s_start[g * kHwCap + ord] = static_cast<uint16_t>(threadIdx.x * 128u + w * 32u + k);  // position of the '\n'
-                ++ord;
-            }
-        }
-        __syncthreads();
-        // ---- phase 2: the heads of the lines that follow those newlines
-        uint32_t n_g[kHwTiles], total = 0;
-#pragma unroll
-        for (int t = 0; t < kHwTiles; ++t) {
-            n_g[t] = min(s_wsum[2 * t] + s_wsum[2 * t + 1], kHwCap);
-            total += n_g[t];
-        }
-        for (uint32_t i = threadIdx.x; i < total; i += kHwThreads) {
-            uint32_t t = 0, o = i;
-#pragma unroll
-            for (int k = 0; k < kHwTiles - 1; ++k)
-                if (t == static_cast<uint32_t>(k) && o >= n_g[k]) o -= n_g[k], ++t;
-            const int64_t start = base_u + s_start[t * kHwCap + o] + 1;
-            uint32_t c = 0;
-            if (start < P.n_units) c = hw_walk_head(P, start, cx_abs, tab_abs, row_bytes);
-            P.cand[(sup * kHwTiles + t) * static_cast<int64_t>(kHwCap) + o] = static_cast<uint16_t>(c);
-        }
-        if (sup == 0 && threadIdx.x == kHwThreads - 1 && P.n_units > 0) P.scalars[2] = hw_walk_head(P, 0, cx_abs, tab_abs, row_bytes);
-    }
-}
-
 }  // namespace
-
-size_t dfawalk_smem_bytes(const DfaWalkDev& a, uint32_t threads, bool in_smem, bool cut) {
-    size_t b = in_smem ? ((static_cast<size_t>(a.n_rows) * a.K * 2 + 15) & ~size_t(15)) : 0;
-    b += 128 * 4;
-    b += static_cast<size_t>(kDfaWalkStagePerThread) * threads * 8;
-    if (cut) b += static_cast<size_t>(threads) * 32;
-    return b + 128;
-}
-
-namespace {
-template <class Kernel>
-int dfawalk_blocks_per_sm(Kernel kernel, uint32_t threads, size_t smem) {
-    allow_max_dynamic_smem(kernel);
-    int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, static_cast<int>(threads), smem) != cudaSuccess) {
-        cudaGetLastError();
-        return 0;
-    }
-    return per_sm;
-}
-int dfawalk_blocks(uint32_t threads, size_t smem, bool in_smem, bool cut) {
-    if (cut) return dfawalk_blocks_per_sm(dfawalk_kernel<true, true>, threads, smem);
-    return in_smem ? dfawalk_blocks_per_sm(dfawalk_kernel<true, false>, threads, smem) : dfawalk_blocks_per_sm(dfawalk_kernel<false, false>, threads, smem);
-}
-}  // namespace
-
-// picks table placement and CTA size: the table goes to shared memory when that still leaves >= 16 resident warps per SM
-// (the early-exit variant always has its small table in shared memory)
-bool k0_dfawalk_plan(const DfaWalkDev& a, uint32_t* threads, bool* in_smem, bool cut) {
-    if (!a.enabled) return false;
-    for (int pass = 0; pass < 2; ++pass) {
-        const bool sm = pass == 0;
-        if (cut && !sm) break;
-        uint32_t best = 0, best_warps = 0;
-        for (uint32_t kT : {1024u, 512u, 256u}) {
-            const size_t smem = dfawalk_smem_bytes(a, kT, sm, cut);
-            if (smem > 226 * 1024) continue;
-            const uint32_t warps = static_cast<uint32_t>(dfawalk_blocks(kT, smem, sm, cut)) * kT / 32;
-            if (warps > best_warps) best = kT, best_warps = warps;
-        }
-        if (best && (best_warps >= 16 || !sm)) {
-            *threads = best;
-            *in_smem = sm;
-            return true;
-        }
-    }
-    return false;
-}
-
-int k0_dfawalk_grid(const Launch& L, const DfaWalkParams& P, uint32_t threads, bool in_smem) {
-    const size_t smem = dfawalk_smem_bytes(P.a, threads, in_smem, P.cut != 0);
-    int per_sm = dfawalk_blocks(threads, smem, in_smem, P.cut != 0);
-    if (per_sm < 1) per_sm = 1;
-    const int64_t cap = static_cast<int64_t>(L.sm_count) * per_sm;
-    const int g = static_cast<int>(P.n_tiles < cap ? P.n_tiles : cap);
-    return g < 1 ? 1 : g;
-}
-
-void k0_dfawalk_scan(const Launch& L, const DfaWalkParams& P, uint32_t threads, bool in_smem) {
-    const size_t smem = dfawalk_smem_bytes(P.a, threads, in_smem, P.cut != 0);
-    const int g = k0_dfawalk_grid(L, P, threads, in_smem);
-    if (P.cut) dfawalk_kernel<true, true><<<g, static_cast<int>(threads), smem, L.stream>>>(P);
-    else if (in_smem) dfawalk_kernel<true, false><<<g, static_cast<int>(threads), smem, L.stream>>>(P);
-    else dfawalk_kernel<false, false><<<g, static_cast<int>(threads), smem, L.stream>>>(P);
-}
 
 size_t linewalk_smem_bytes(const DfaWalkDev& a, bool in_smem) {
     return (in_smem ? ((static_cast<size_t>(a.n_rows) * a.K * 2 + 15) & ~size_t(15)) : 0) + 128 * 4 + 128 * 2 + 128;
-}
-
-static size_t headwalk_smem_bytes(const DfaWalkDev& a) {
-    return ((static_cast<size_t>(a.n_rows) * a.K * 2 + 15) & ~size_t(15)) + 128 * 4 + static_cast<size_t>(kHwTiles) * kHwCap * 2 + 128;
-}
-
-bool k1h_plan(const DfaWalkDev& a) { return a.enabled && a.fin_base + 65535u > a.n_rows && headwalk_smem_bytes(a) <= 110 * 1024; }
-
-void k1h_count_headwalk(const Launch& L, const HeadWalkParams& P) {
-    if (P.n_units <= 0) return;
-    const size_t smem = headwalk_smem_bytes(P.a);
-    allow_max_dynamic_smem(headwalk_count_kernel);
-    int per_sm = 1;
-    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, headwalk_count_kernel, kHwThreads, smem);
-    headwalk_count_kernel<<<L.sm_count * (per_sm < 1 ? 1 : per_sm), kHwThreads, smem, L.stream>>>(P);
 }
 
 bool k2b_linewalk_plan(const DfaWalkDev& a, uint32_t* threads, bool* in_smem) {

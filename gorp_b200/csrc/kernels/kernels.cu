@@ -140,9 +140,7 @@ __global__ void __launch_bounds__(kThreads) nl_count_mask_kernel(const uint16_t*
 // lane l takes the 8 mask words of units [256 l, 256 l + 256) of the tile, the warp scans the counts, every lane writes
 // the starts of its lines.
 __global__ void __launch_bounds__(kThreads) nl_scatter_mask_kernel(const uint32_t* __restrict__ masks, const int64_t* __restrict__ tile_base,
-                                                                   int64_t* __restrict__ line_off, int64_t n_tiles,
-                                                                   const uint16_t* __restrict__ cand, const uint32_t* __restrict__ cand0,
-                                                                   int32_t* __restrict__ ext_id) {
+                                                                   int64_t* __restrict__ line_off, int64_t n_tiles) {
     static_assert(kNlTile == 32 * 256, "one lane = 8 mask words");
     const uint32_t lane = threadIdx.x & 31u;
     const int64_t tile = static_cast<int64_t>(blockIdx.x) * (kThreads / 32) + (threadIdx.x >> 5);
@@ -161,17 +159,12 @@ __global__ void __launch_bounds__(kThreads) nl_scatter_mask_kernel(const uint32_
     }
     int64_t slot = 1 + tile_base[tile] + (incl - cnt);  // line_off[j] = start of line j (j >= 1)
     const int64_t unit1 = tile * kNlTile + static_cast<int64_t>(lane) * 256 + 1;
-    uint32_t ord = incl - cnt;  // the lane's first '\n' is the ord-th of the tile: where K1h parked the candidate of the line after it
-    const uint16_t* tcand = cand ? cand + tile * kHwCap : nullptr;
-    if (cand && tile == 0 && lane == 0) ext_id[0] = static_cast<int32_t>(*cand0) - 1;
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
         uint32_t m = w[j];
         while (m) {
             const int k = __ffs(m) - 1;
             m &= m - 1;
-            if (cand) ext_id[slot] = ord < kHwCap ? static_cast<int32_t>(tcand[ord]) - 1 : -1;
-            ++ord;
             line_off[slot++] = unit1 + j * 32 + k;
         }
     }
@@ -482,11 +475,10 @@ void k1_count_newlines_masks(const Launch& L, const uint16_t* text, int64_t n_un
     nl_count_mask_kernel<<<blocks_for(n_units, kNlTile), kThreads, 0, L.stream>>>(text, n_units, tile_counts, masks);
 }
 
-void k1_scatter_masks(const Launch& L, const uint32_t* masks, int64_t n_units, const int64_t* tile_base, int64_t* line_off,
-                      const uint16_t* cand, const uint32_t* cand0, int32_t* ext_id) {
+void k1_scatter_masks(const Launch& L, const uint32_t* masks, int64_t n_units, const int64_t* tile_base, int64_t* line_off) {
     if (n_units <= 0) return;
     const int64_t n_tiles = (n_units + kNlTile - 1) / kNlTile;
-    nl_scatter_mask_kernel<<<blocks_for(n_tiles, kThreads / 32), kThreads, 0, L.stream>>>(masks, tile_base, line_off, n_tiles, cand, cand0, ext_id);
+    nl_scatter_mask_kernel<<<blocks_for(n_tiles, kThreads / 32), kThreads, 0, L.stream>>>(masks, tile_base, line_off, n_tiles);
 }
 
 void k1_finish(const Launch& L, const uint16_t* text, int64_t n_units, const int64_t* total_newlines, int64_t* line_off,

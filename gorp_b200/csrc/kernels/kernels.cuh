@@ -119,9 +119,7 @@ void k1_scatter_newlines(const Launch&, const uint16_t* text, int64_t n_units, c
 // same pair with the '\n' masks (one u32 per 32 units, ceil(n_units / kNlTile) * 256 words) as a side product of the
 // count pass: the scatter pass then reads the masks instead of the text (one HBM pass over the text instead of two)
 void k1_count_newlines_masks(const Launch&, const uint16_t* text, int64_t n_units, uint32_t* tile_counts, uint32_t* masks);
-// cand / cand0 / ext_id (K1h): the candidates parked per tile go to ext_id[line] on the way (cand0: the line at offset 0)
-void k1_scatter_masks(const Launch&, const uint32_t* masks, int64_t n_units, const int64_t* tile_base, int64_t* line_off,
-                      const uint16_t* cand = nullptr, const uint32_t* cand0 = nullptr, int32_t* ext_id = nullptr);
+void k1_scatter_masks(const Launch&, const uint32_t* masks, int64_t n_units, const int64_t* tile_base, int64_t* line_off);
 void k1_finish(const Launch&, const uint16_t* text, int64_t n_units, const int64_t* total_newlines, int64_t* line_off,
                int64_t* n_lines_out);
 
@@ -150,56 +148,9 @@ void k4_tdfa_capture(const Launch&, const CapDev&, const uint16_t* text, const i
 void k4_tdfa_fast(const Launch&, const TdfaFastDev&, const CapDev&, const uint16_t* text, int64_t n_units,
                   const int64_t* line_off, int64_t n_lines, uint32_t span_stride, int32_t* ext_id, int32_t* spans);
 
-// Table of the folded automaton of host/fused.hpp as the chunk-owner one-pass kernel K0c reads it (kernels/chunkwalk.cu; the
-// TMA-staged tile kernel that first used it lost to K0c in round 1 and was removed in round 2).
-constexpr int kOnePassHistBins = 256;
-struct OnePassDev {
-    const uint32_t* rows;        // [n_rows * width] raw entries: (next row << 16) | slot id
-                                 //   rows [0, n_states) automaton states, [skip_base, +7) SKIP_1..7 (units that precede
-                                 //   the line in its first 16-byte chunk), [fin_base, +n_outcomes) absorbing outcome rows
-                                 //   columns [0,128) ASCII units directly, [128, width) classes of the other units
-    uint32_t n_rows, width;      // width is a multiple of 4
-    uint32_t n_states, skip_base, fin_base, n_outcomes;
-    uint32_t n_slots;            // slot 0 = dummy (transitions without commands), 1..n_op op slots, n_op+1 = LEN
-    const int32_t* out_ext;      // [n_outcomes] -1 MISS | e | -2-e
-    const uint32_t* out_res;     // [n_outcomes * max_slots] per group boundary: up to 4 slot ids, one per byte, 0 ends
-    uint32_t max_slots;          // 2 * groups of the widest extraction
-    const uint16_t* xcol;        // [65536] unit -> column
-    const uint16_t* pair_col;    // [width] column of a high surrogate that is followed by a low surrogate
-    const uint32_t* init_slots;  // [n_init] slots reset to -1 per line (those read through a multi-writer maximum)
-    uint32_t n_init;
-    uint32_t enabled;
-};
-struct OnePassParams {
-    const uint16_t* text;
-    int64_t n_units, n_tiles;
-    uint32_t tile_units, per;            // tile_units = blockDim * per
-    OnePassDev a;
-    const uint32_t* slots_per_ext;
-    uint32_t n_ext;
-    uint32_t span_stride;                // int32 entries per result row of `spans` (2 * groups of the widest extraction)
-    int32_t* ext_id;
-    int64_t* line_off;
-    int32_t* spans;                      // [cap_lines * span_stride]
-    unsigned long long* hist;
-    int64_t cap_lines;
-    unsigned long long* tile_status;     // [n_tiles] zeroed by the caller: flag(2) | lines(62); flag 1 = the tile's own
-                                         // line count, flag 2 = inclusive prefix over tiles 0..t
-    unsigned int* ticket;                // zeroed by the caller
-    int64_t* totals;                     // [0] n_lines, [2] flags: 1 = capacity overflow, 2 = tile too dense
-    long long* debug;                    // optional [grid * 2 * 10] per-phase cycle counters (GORP_ONEPASS_DEBUG=1)
-};
-
-// K0c: chunk-walk one-pass kernel (text form) — see kernels/chunkwalk.cu. Uses OnePassParams (tile_units = threads *
-// kChunkUnits, per = kChunkUnits) with the DEADSCAN variant of the table.
-constexpr uint32_t kChunkUnits = 256;  // units per thread chunk
-size_t chunkwalk_smem_bytes(const OnePassDev&, uint32_t threads);
-bool k0_chunkwalk_plan(const OnePassDev&, uint32_t* threads);
-int k0_chunkwalk_grid(const Launch&, const OnePassParams&, uint32_t threads);
-void k0_chunkwalk_extract(const Launch&, const OnePassParams&, uint32_t threads);
-
-// K0d: chunk-walk DFA kernel (text form, any definition) — see kernels/dfawalk.cu. Newline index + combined DFA in one
-// pass: writes line_off[0..n] and ext_id (>= 0 | -1); the capture half follows (kernels/capwalk.cu).
+// K2b: combined-DFA walk over an existing line index (K1, or the caller's offsets), lanes pull lines dynamically — see
+// kernels/dfawalk.cu. Writes ext_id (>= 0 | -1; the candidate when `a` is the early-exit table and the tail walk follows).
+// Text form: every line must be terminated by '\n' in the text or end at n_units.
 struct DfaWalkDev {
     const uint16_t* table;       // [n_rows * K] next row (global copy, padded to 16 bytes; copied to shared memory
                                  // when it fits). Rows: [0,S) states, S = DEADSCAN, S+1..S+15 = SKIP_1..15,
@@ -210,27 +161,6 @@ struct DfaWalkDev {
     const uint16_t* xcls;        // [65536] unit -> column (units >= 0x80)
     uint32_t enabled;
 };
-struct DfaWalkParams {
-    const uint16_t* text;
-    int64_t n_units, n_tiles;    // tiles of blockDim * kChunkUnits units
-    DfaWalkDev a;
-    int32_t* ext_id;
-    int64_t* line_off;
-    int64_t cap_lines;
-    uint32_t stage_rows;         // rows staged in shared memory per tile (kDfaWalkStagePerThread * blockDim)
-    unsigned long long* tile_status;  // [n_tiles] zeroed by the caller (decoupled look-back, as OnePassParams)
-    unsigned int* ticket;        // zeroed by the caller
-    int64_t* totals;             // [0] n_lines, [1] 1 = the text ends with '\n', [2] flags: 1 = capacity overflow
-    uint32_t cut;                // 1: `a` is the early-exit table (ext_id = candidates, the tail walk must follow)
-};
-constexpr uint32_t kDfaWalkStagePerThread = 6;
-size_t dfawalk_smem_bytes(const DfaWalkDev&, uint32_t threads, bool in_smem, bool cut = false);
-bool k0_dfawalk_plan(const DfaWalkDev&, uint32_t* threads, bool* in_smem, bool cut = false);
-int k0_dfawalk_grid(const Launch&, const DfaWalkParams&, uint32_t threads, bool in_smem);
-void k0_dfawalk_scan(const Launch&, const DfaWalkParams&, uint32_t threads, bool in_smem);
-
-// K2b: the K0d automaton over an existing line index (K1), lanes pull lines dynamically — see kernels/dfawalk.cu.
-// Every line must be terminated by '\n' in the text or end at n_units.
 constexpr uint32_t kLineItemLines = 1024;
 struct LineWalkParams {
     const uint16_t* text;
@@ -243,23 +173,6 @@ struct LineWalkParams {
     uint32_t flags;              // GORP_WALK_FLAGS (diagnostics): 1 = text loads L2 evict-first
     uint32_t lines_form;         // 1: List<String> form — line i = [line_off[i], line_off[i+1]), a '\n' is content
 };
-// K1h: the count pass of the newline index (K1) and the combined-DFA walk of the line HEADS (K2b over the early-exit table) in
-// one pass over the text — see kernels/dfawalk.cu. The line index of a line is not known yet (the prefix sums come later),
-// so the candidate of the line that follows the j-th '\n' of an 8192-unit tile is parked in cand[tile * kHwCap + j] (value
-// = FIN row - fin_base: 0 = MISS, e + 1) and the scatter pass of K1 copies it to ext_id. `dense` is set when a tile has
-// more line starts than kHwCap (the caller then runs K2b over the line index instead).
-constexpr uint32_t kHwCap = 512;
-struct HeadWalkParams {
-    const uint16_t* text;
-    int64_t n_units;
-    DfaWalkDev a;                // table in shared memory
-    uint32_t* tile_counts;       // [n_tiles] newlines per kNlTile units (as K1)
-    uint32_t* masks;             // [n_tiles * 256] newline masks (as K1)
-    uint16_t* cand;              // [n_tiles * kHwCap]
-    uint32_t* scalars;           // [0] ticket (zeroed by the caller), [1] dense flag (zeroed), [2] candidate of the line at offset 0
-};
-bool k1h_plan(const DfaWalkDev&);
-void k1h_count_headwalk(const Launch&, const HeadWalkParams&);
 bool k2b_linewalk_plan(const DfaWalkDev&, uint32_t* threads, bool* in_smem);
 void k2b_linewalk_scan(const Launch&, const LineWalkParams&, uint32_t threads, bool in_smem);
 

@@ -5,8 +5,8 @@
 // JDKRegexpCookedExtraction.match/_constructMatch (jdkre/JDKRegexpCookedExtraction.java:36-59).
 //
 // Work decomposition = kernels/capwalk.cu (lines bucketed by candidate extraction, a CTA takes work items of <= 4096
-// lines of ONE extraction, lanes claim lines from the CTA's cursor one line ahead), the per-unit step = kernels/
-// chunkwalk.cu: the extraction's table lives in shared memory as directly ASCII-indexed rows of u16 entries,
+// lines of ONE extraction, lanes claim lines from the CTA's cursor one line ahead). The extraction's table lives in shared
+// memory as directly ASCII-indexed rows of u16 entries,
 //
 //   per unit :  ent = LDS.U16[row(ent) + 2*unit]          one shared-memory lookup, the only dependent chain
 //               STS.U16 slot(ent)[thread] = position + 1    "last position at which command list `slot` fired"

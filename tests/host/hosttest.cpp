@@ -126,7 +126,7 @@ extern "C" int ht_run(const void* blob, size_t len, const uint16_t* text, const 
     }
 }
 
-// The one-pass automaton (host/fused.hpp) interpreted the way kernels/chunkwalk.cu runs it: one table lookup per unit,
+// The one-pass automaton (host/fused.hpp) interpreted one unit at a time: one table lookup per unit,
 // "last position" per op slot, group boundaries resolved from the outcome at end of line.
 // stats: [0] available, [1] states, [2] joint classes, [3] op slots, [4] outcomes. Returns 1 when not available.
 extern "C" int ht_run_fused(const void* blob, size_t len, const uint16_t* text, const int64_t* starts, const int64_t* ends,
@@ -233,7 +233,7 @@ extern "C" int ht_compact_dfa(const void* blob, size_t len, int32_t* trans, int6
     }
 }
 
-// The big-definition text path interpreted the way kernels/dfawalk.cu (K0d / K2b) and kernels/capwalk.cu (K4b) run it:
+// The big-definition text path interpreted the way kernels/dfawalk.cu (K2b) and kernels/capwalk.cu (K4b) run it:
 // '\n' split, combined DFA over the class-indexed table with SKIP / DEADSCAN / FIN rows in 16-unit blocks starting at
 // the aligned block that holds the line start, then the capture walk over the extraction's table image (smem_variant:
 // ids beyond DEAD read the DEAD row and the highest id seen survives; otherwise the physical FRZ rows), SLOW blocks

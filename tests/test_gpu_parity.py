@@ -136,19 +136,13 @@ def test_config_corpora(name, n, monkeypatch):
     table), #5 non-ASCII UTF-16 + divergence characters + 10 KB outliers."""
     d, gen = corpus.CONFIGS[name]
     text = gen(n)
-    if name in ("weblog", "syslog200", "utf16mix"):  # both DFA tiers of the big-definition path (K0d / K1 + K2b) ...
-        for tier in ("1", "2"):
-            monkeypatch.setenv("GORP_DFA_TIER", tier)
+    if name in ("weblog", "syslog200", "utf16mix"):  # the big-definition path with and without the early exit / tail automata
+        for no_tails in ("0", "1"):
+            if no_tails == "1":
+                monkeypatch.setenv("GORP_NO_TAILS", "1")
             check_against_oracle(d, text=text)
-        monkeypatch.setenv("GORP_NO_TAILS", "1")  # ... and the two-walk path without the early exit / tail automata
-        check_against_oracle(d, text=text)
+            check_against_oracle(d, text=text[:-1])  # last line not terminated
         monkeypatch.delenv("GORP_NO_TAILS")
-        monkeypatch.delenv("GORP_DFA_TIER")
-        for cut in ("1", "0"):  # the early-exit walk as chunk owner (one pass, newline masks) / over the line index (K1 + K2b)
-            monkeypatch.setenv("GORP_CUT_WALK", cut)
-            check_against_oracle(d, text=text)
-            check_against_oracle(d, text=text[:-1])
-        monkeypatch.delenv("GORP_CUT_WALK")
     _, b, oe = check_against_oracle(d, text=text)
     assert b.n_lines == n and (oe >= 0).sum() > n // 3
     if name == "utf16mix":
@@ -251,22 +245,18 @@ def test_full_size_properties_big_definitions(name, n, reps):
     assert (np.diff(b.line_off).reshape(reps, -1) == np.diff(b1.line_off)[None, :]).all()
 
 
-TIERS = {"k1_fusedwalk": {}, "chunkwalk": {"GORP_SMALL_PATH": "chunkwalk"},
-         "dfawalk_capwalk_notails": {"GORP_FORCE_TWOPASS": "1", "GORP_DFA_TIER": "1", "GORP_NO_TAILS": "1"},
-         "linewalk_capwalk_notails": {"GORP_FORCE_TWOPASS": "1", "GORP_DFA_TIER": "2", "GORP_NO_TAILS": "1"},
-         "linewalk_tailwalk_flush1": {"GORP_FORCE_TWOPASS": "1", "GORP_DFA_TIER": "2", "GORP_TAIL_FLUSH": "1"},
-         "cutwalk_tailwalk": {"GORP_FORCE_TWOPASS": "1", "GORP_CUT_WALK": "1", "GORP_TAIL_THREADS": "512"},
-         "linewalk_cut_tailwalk384": {"GORP_FORCE_TWOPASS": "1", "GORP_CUT_WALK": "0", "GORP_TAIL_THREADS": "384"},
-         "k1h_tailwalk": {"GORP_FORCE_TWOPASS": "1", "GORP_DFA_TIER": "3"},
-         "k1h_capwalk_notails": {"GORP_FORCE_TWOPASS": "1", "GORP_DFA_TIER": "3", "GORP_NO_TAILS": "1"},
-         "dfawalk_capwalk": {"GORP_FORCE_TWOPASS": "1", "GORP_DFA_TIER": "1"},
-         "linewalk_capwalk": {"GORP_FORCE_TWOPASS": "1", "GORP_DFA_TIER": "2"},
-         "dfawalk_k4": {"GORP_FORCE_TWOPASS": "1", "GORP_DFA_TIER": "1", "GORP_FORCE_K4": "1"},
+TIERS = {"k1_fusedwalk": {},
+         "linewalk_capwalk_notails": {"GORP_FORCE_TWOPASS": "1", "GORP_NO_TAILS": "1"},
+         "linewalk_tailwalk_flush1": {"GORP_FORCE_TWOPASS": "1", "GORP_TAIL_FLUSH": "1"},
+         "linewalk_tailwalk512": {"GORP_FORCE_TWOPASS": "1", "GORP_TAIL_THREADS": "512"},
+         "linewalk_cut_tailwalk384": {"GORP_FORCE_TWOPASS": "1", "GORP_TAIL_THREADS": "384"},
+         "linewalk_capwalk": {"GORP_FORCE_TWOPASS": "1"},
+         "linewalk_k4": {"GORP_FORCE_TWOPASS": "1", "GORP_FORCE_K4": "1"},
          "k1k2_capwalk": {"GORP_FORCE_TWOPASS": "1", "GORP_FORCE_K1K2": "1"},
          "twopass_fast": {"GORP_FORCE_TWOPASS": "1", "GORP_FORCE_K1K2": "1", "GORP_FORCE_K4": "1"},
          "general": {"GORP_FORCE_GENERAL": "1"}}
-_TIER_ENV = ("GORP_FORCE_TWOPASS", "GORP_FORCE_GENERAL", "GORP_FORCE_K1K2", "GORP_FORCE_K4", "GORP_DFA_TIER",
-             "GORP_NO_TAILS", "GORP_TAIL_FLUSH", "GORP_CUT_WALK", "GORP_TAIL_THREADS", "GORP_SMALL_PATH")
+_TIER_ENV = ("GORP_FORCE_TWOPASS", "GORP_FORCE_GENERAL", "GORP_FORCE_K1K2", "GORP_FORCE_K4", "GORP_NO_TAILS", "GORP_TAIL_FLUSH",
+             "GORP_TAIL_THREADS")
 
 
 @pytest.mark.parametrize("tier", list(TIERS))
@@ -324,8 +314,7 @@ def test_pike_vm_fallback(monkeypatch):
 def test_tail_walk_very_long_lines(monkeypatch):
     """Lines of 65 000 units and more leave the 16-bit tail walk for the one-thread-per-line kernel with 32-bit positions;
     results stay exact (spans far beyond 65 535, non-ASCII content, a candidate that ends as MISS / CAPTURE_FAIL)."""
-    monkeypatch.setenv("GORP_FORCE_TWOPASS", "1")  # the README definition would otherwise take the one-pass kernel
-    monkeypatch.setenv("GORP_DFA_TIER", "2")
+    monkeypatch.setenv("GORP_FORCE_TWOPASS", "1")  # the README definition would otherwise take the fused walk
     rng = np.random.default_rng(17)
     lines = corpus.weblog_lines(300, seed=8)
     body = "".join(rng.choice(list("abcdefghij0123456789/"), size=70000))
@@ -381,20 +370,16 @@ def test_latin1_text_form(monkeypatch):
     assert g.extract_batch_text_latin1(b"[1]: GET 2ms /a").ext_id.tolist() == [1]
 
 
-@pytest.mark.parametrize("small_path", ["fusedwalk", pytest.param("chunkwalk", marks=pytest.mark.xfail(
-    strict=False, reason="the chunk-owner kernel K0c is bistable (1.43 or 2.1 ms per launch here; profiles/README.md round 1): kept "
-                         "as a tier for A/B, the default path of small definitions is the fused walk"))])
-def test_chunkwalk_launch_times_are_stable(small_path, monkeypatch):
-    """Round 1 found the one-pass kernel bistable (11.5 or 17.4 ms per launch, depending on unrelated allocation sizes).
-    Every launch of a series must run in the fast mode whatever the sizes of the result allocations are: the row arrays are
-    padded by 0 / 64 K / 1 M rows (GORP_PAD_ROWS shifts every allocation that follows), 25 launches each. The default path
-    of small definitions (K1 + fused walk: no look-back, no phase coupling between CTAs) is held to the same bound."""
+def test_fused_walk_launch_times_are_stable(monkeypatch):
+    """Round 1 found the chunk-owner one-pass kernel of that time bistable (11.5 or 17.4 ms per launch, depending on unrelated
+    allocation sizes). Every launch of a series of the default path of small definitions (K1 + fused walk) must run at the
+    same speed whatever the sizes of the result allocations are: the row arrays are padded by 0 / 64 K / 1 M rows
+    (GORP_PAD_ROWS shifts every allocation that follows), 25 launches each."""
     import ctypes as C
     import torch
     from gorp_b200 import _ffi, corpusgen
     from gorp_b200.api import Blob, _check
     dev = torch.device("cuda", 0)
-    monkeypatch.setenv("GORP_SMALL_PATH", small_path)
     d_text = corpusgen.device_text("readme", 0, 12_000_000, dev)
     blob = Blob.from_definition(V.README_DEF)
     times = {}

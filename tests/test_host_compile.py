@@ -62,7 +62,7 @@ def test_config_definitions_reproduce_oracle(name):
 
 @pytest.mark.parametrize("case", ALL_DEFS)
 def test_one_pass_automaton_reproduces_oracle(case):
-    """host/fused.hpp: DFA x capture automata folded into one automaton, interpreted as kernels/chunkwalk.cu runs it."""
+    """host/fused.hpp: DFA x capture automata folded into one automaton, interpreted one table lookup per unit."""
     stats = compare_host_tables(case[0], [c[0] for c in case[1]] + TRICKY_LINES, fused=True)
     assert stats[0] == 1
 

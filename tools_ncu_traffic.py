@@ -14,11 +14,10 @@ import json
 import os
 import sys
 
-TIMER_OF = [("chunkwalk", "k0_chunkwalk_extract"), ("dfawalk_kernel", "k0_dfawalk"), ("nl_count", "k1_count_newlines"),
-            ("scan_", "scan_tiles"), ("nl_scatter", "k1_scatter_newlines"), ("nl_finish", "k1_scatter_newlines"), ("k1_finish", "k1_scatter_newlines"),
-            ("linewalk", "k2b_linewalk_scan"), ("histogram", "k3_histogram"), ("bucket_", "k4b_bucket"), ("tailwalk", "k4c_tailwalk"),
-            ("tail_long", "k4c_tailwalk"), ("capwalk", "k4b_capwalk"), ("dfa_direct", "k2_dfa_scan"), ("dfa_scan", "k2_dfa_scan"),
-            ("tdfa", "k4_tdfa_capture")]
+TIMER_OF = [("nl_count", "k1_count_newlines"), ("scan_", "scan_tiles"), ("nl_scatter", "k1_scatter_newlines"), ("nl_finish", "k1_scatter_newlines"),
+            ("k1_finish", "k1_scatter_newlines"), ("linewalk", "k2b_linewalk_scan"), ("histogram", "k3_histogram"), ("bucket_", "k4b_bucket"),
+            ("tailwalk", "k4c_tailwalk"), ("tail_long", "k4c_tailwalk"), ("capwalk", "k4b_capwalk"), ("dfa_direct", "k2_dfa_scan"),
+            ("dfa_scan", "k2_dfa_scan"), ("tdfa", "k4_tdfa_capture")]
 
 
 def main():
@@ -40,8 +39,6 @@ def main():
     agg = {}
     for name, m in last.items():
         timer = next((t for k, t in TIMER_OF if k in name), None)
-        if timer == "k0_dfawalk":
-            timer = "k0_dfawalk_cut" if "k0_dfawalk_cut" in timers else "k0_dfawalk_scan"
         if timer == "k4c_tailwalk" and "k4c_fusedwalk" in timers:  # the same kernel in "all" mode (small definitions)
             timer = "k4c_fusedwalk"
         if timer is None or timer not in timers:
