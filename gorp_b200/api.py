@@ -194,11 +194,13 @@ class ExtractionResult:
 
 
 class ExtractionBatch:
-    """Columnar result of one batch call: numpy copies of the gorp_result arrays + lazy ExtractionResult views."""
+    """Columnar result of one batch call: numpy copies of the gorp_result arrays + lazy ExtractionResult views.
+    `units` is the text the offsets index, in `encoding`: UTF-16 units, or the caller's UTF-8 bytes (byte coordinates);
+    a line or a value is decoded from its own slice only."""
 
-    def __init__(self, gorp, units, res: _ffi.Result, sep):
+    def __init__(self, gorp, units, res: _ffi.Result, sep, encoding="utf-16-le"):
         n = res.n_lines
-        self.gorp, self.units, self.sep, self.n_lines = gorp, units, sep, n
+        self.gorp, self.units, self.sep, self.n_lines, self.encoding = gorp, units, sep, n, encoding
         self.ext_id = np.ctypeslib.as_array(res.ext_id, (max(n, 1),))[:n].copy()
         self.line_off = np.ctypeslib.as_array(res.line_off, (n + 1,)).copy()
         self.span_stride = w = int(res.span_stride)
@@ -211,7 +213,7 @@ class ExtractionBatch:
 
     def line(self, i) -> str:
         a, b = int(self.line_off[i]), int(self.line_off[i + 1]) - self.sep
-        return self.units[a:b].tobytes().decode("utf-16-le", "surrogatepass")
+        return self.units[a:b].tobytes().decode(self.encoding, "surrogatepass")
 
     def spans_of(self, i):
         e = int(self.ext_id[i])
@@ -236,7 +238,7 @@ class ExtractionBatch:
         a = int(self.line_off[i])
         vals = []
         for (s, t) in self.spans_of(i):
-            vals.append(None if s < 0 else self.units[a + s:a + t].tobytes().decode("utf-16-le", "surrogatepass"))
+            vals.append(None if s < 0 else self.units[a + s:a + t].tobytes().decode(self.encoding, "surrogatepass"))
         return x.constructMatch(self.line(i), vals)
 
     def results(self, safe=False):
@@ -310,11 +312,19 @@ class Gorp:
         finally:
             lib.gorp_result_release(self._eng(), C.byref(res))
 
-    def extract_batch_text_utf8(self, data) -> ExtractionBatch:
+    def extract_batch_text_utf8(self, data, byte_offsets=False) -> ExtractionBatch:
         """'\n'-separated text held as UTF-8 bytes (a log file as it is on disk): decoded to UTF-16 on the device, results are
-        those of extract_batch_text on the decoded text (offsets in UTF-16 units). Malformed UTF-8 raises ValueError."""
+        those of extract_batch_text on the decoded text (offsets in UTF-16 units). Malformed UTF-8 raises ValueError.
+        byte_offsets=True: line_off and spans are byte offsets into `data` (gorp_extract_text_utf8_bytes, all of the engine's
+        devices); the batch slices `data` and decodes only what a line(), spans_of() or result() asks for."""
         b = np.ascontiguousarray(np.frombuffer(data, dtype=np.uint8) if isinstance(data, (bytes, bytearray)) else data, dtype=np.uint8)
         res = _ffi.Result()
+        if byte_offsets:
+            _check(lib.gorp_extract_text_utf8_bytes(self._eng(), b.ctypes.data, len(b), C.byref(res)))
+            try:
+                return ExtractionBatch(self, b, res, 1, encoding="utf-8")
+            finally:
+                lib.gorp_result_release(self._eng(), C.byref(res))
         _check(lib.gorp_extract_text_utf8(self._eng(), b.ctypes.data, len(b), C.byref(res)))
         try:
             units = np.frombuffer(b.tobytes().decode("utf-8").encode("utf-16-le"), dtype=np.uint16)

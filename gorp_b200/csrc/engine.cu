@@ -159,6 +159,7 @@ struct DeviceCtx {
     cudaEvent_t ev_in[2]{}, ev_free[2]{}, ev_rows = nullptr;
     cudaEvent_t ev_done = nullptr;  // end of the last call on this context: the next call's stream waits for it (shared scratch)
     DevBuf textbuf[2], offbuf[2], bytebuf[2], acc_ext, acc_off, acc_spans, acc_hist;
+    DevBuf byte_off;  // byte line offsets of a UTF-8 piece (byte coordinates)
     // per-call scratch, serialised by `mu`
     std::mutex mu;
     DevBuf text, off_in, line_off, tile_counts, tile_base, scan_scratch, ext_id, spans, hist, scalars;
@@ -976,8 +977,10 @@ struct DeviceRun {  // what one device produced for its pieces
 // Processes pieces [p0, p1) on device context c. Rows accumulate in c.acc_*; when `hr` is given (single-device call) the
 // rows of every finished piece are copied to the host arrays at once, overlapping the next pieces.
 // `text8` (ISO-8859-1 bytes, text form only) replaces `text`: the bytes are staged and widened to UTF-16 on the device.
+// `utf8`: the bytes are UTF-8, decoded on the device; offsets count UTF-16 units of the decoded text, or with `byte_coords`
+// bytes of `text8` (then the pieces are independent, as for ISO-8859-1).
 // The caller holds c.mu (a multi-device call keeps every participating device locked until its rows are copied out).
-void run_pieces(gorp_engine* e, DeviceCtx& c, const uint16_t* text, const uint8_t* text8, bool utf8, const int64_t* off,
+void run_pieces(gorp_engine* e, DeviceCtx& c, const uint16_t* text, const uint8_t* text8, bool utf8, bool byte_coords, const int64_t* off,
                 const std::vector<Piece>& pieces, size_t p0, size_t p1, HostResult* hr, DeviceRun& run) {
     CK(cudaSetDevice(c.device));
     CK(cudaStreamWaitEvent(c.stream, c.ev_done, 0));  // a device-resident call on another stream may still use the scratch
@@ -1075,7 +1078,7 @@ void run_pieces(gorp_engine* e, DeviceCtx& c, const uint16_t* text, const uint8_
                 c.launches += 1;
             }
             nl = run_pipeline(c, c.textbuf[b].as<uint16_t>(), n_units_piece, nullptr, 0, c.stream, false, &dr);
-            if (utf8) {
+            if (utf8 && !byte_coords) {
                 piece_bias = utf8_base;
                 utf8_base += n_units_piece;
             }
@@ -1088,12 +1091,42 @@ void run_pieces(gorp_engine* e, DeviceCtx& c, const uint16_t* text, const uint8_
         }
         // gather: rows [rows, rows + nl) of the batch
         if (nl) CK(cudaMemcpyAsync(c.acc_ext.as<int32_t>() + rows, dr.d_ext_id, static_cast<size_t>(nl) * 4, cudaMemcpyDeviceToDevice, c.stream));
-        k_bias_copy(L, c.acc_off.as<int64_t>() + rows, dr.d_line_off, nl + 1, off ? 0 : piece_bias);
-        if (nl && stride)
-            CK(cudaMemcpyAsync(c.acc_spans.as<int32_t>() + static_cast<size_t>(rows) * stride, dr.d_spans, static_cast<size_t>(nl) * stride * 4,
-                               cudaMemcpyDeviceToDevice, c.stream));
+        if (utf8 && byte_coords) {
+            // byte '\n' index of the piece, built after run_pipeline (which reuses tile_counts, tile_base, scan_scratch and
+            // nl_masks); line k of the bytes is line k of the decoded text (same '\n' characters). Then the gather converts
+            // the rows from the piece's unit offsets to byte offsets.
+            const int64_t n_tiles = (units + kNlTile - 1) / kNlTile;
+            c.tile_counts.reserve(static_cast<size_t>(n_tiles + 1) * 4);
+            c.tile_base.reserve(static_cast<size_t>(n_tiles + 2) * 8);
+            c.scan_scratch.reserve(static_cast<size_t>(n_tiles / 4096 + 8) * 8);
+            c.nl_masks.reserve(static_cast<size_t>(n_tiles + 4) * 256 * 4);
+            c.byte_off.reserve(static_cast<size_t>(nl + 2) * 8);
+            k_utf8_count_newlines_masks(L, c.bytebuf[b].as<uint8_t>(), units, c.tile_counts.as<uint32_t>(), c.nl_masks.as<uint32_t>());
+            scan_u32_to_i64(L, c.tile_counts.as<uint32_t>(), n_tiles, c.tile_base.as<int64_t>(), c.scan_scratch.as<int64_t>());
+            k1_scatter_masks(L, c.nl_masks.as<uint32_t>(), units, c.tile_base.as<int64_t>(), c.byte_off.as<int64_t>());
+            if (stride > 64) throw std::logic_error("result rows wider than 64 entries");  // (31 groups at most: 62)
+            Utf8RowsParams P{};
+            P.bytes = c.bytebuf[b].as<uint8_t>();
+            P.unit_off = dr.d_line_off;
+            P.byte_off = c.byte_off.as<int64_t>();
+            P.spans = dr.d_spans;
+            P.n_lines = nl;
+            P.end_off = units + (units > 0 && text8[pc.u1 - 1] != 0x0A ? 1 : 0);
+            P.bias = piece_bias;
+            P.stride = stride;
+            P.out_off = c.acc_off.as<int64_t>() + rows;
+            P.out_spans = c.acc_spans.as<int32_t>() + static_cast<size_t>(rows) * stride;
+            k_utf8_rows(L, P);
+            c.launches += units > 0 ? 6 : 3;
+        } else {
+            k_bias_copy(L, c.acc_off.as<int64_t>() + rows, dr.d_line_off, nl + 1, off ? 0 : piece_bias);
+            if (nl && stride)
+                CK(cudaMemcpyAsync(c.acc_spans.as<int32_t>() + static_cast<size_t>(rows) * stride, dr.d_spans, static_cast<size_t>(nl) * stride * 4,
+                                   cudaMemcpyDeviceToDevice, c.stream));
+            c.launches += 1;
+        }
         k_accumulate(L, c.acc_hist.as<int64_t>(), dr.d_histogram, static_cast<int>(E2));
-        c.launches += 2;
+        c.launches += 1;
         CK(cudaEventRecord(c.ev_free[b], c.stream));
         if (hr) {
             CK(cudaEventRecord(c.ev_rows, c.stream));
@@ -1121,7 +1154,7 @@ void run_pieces(gorp_engine* e, DeviceCtx& c, const uint16_t* text, const uint8_
 }
 
 int extract_host(gorp_engine* e, const uint16_t* text, const uint8_t* text8, int64_t n_units, const int64_t* off, int64_t n_lines,
-                 gorp_result* out, bool utf8 = false) {
+                 gorp_result* out, bool utf8 = false, bool byte_coords = false) {
     if (!e || !out || (!text && !text8 && n_units > 0) || n_units < 0 || n_lines < 0) return fail(GORP_E_ARG, "bad argument");
     if (e->devs.empty()) return fail(GORP_E_CUDA, "engine has no CUDA device");
     return guarded([&]() -> int {
@@ -1146,15 +1179,16 @@ int extract_host(gorp_engine* e, const uint16_t* text, const uint8_t* text8, int
             hr->numa_node = e->devs[0]->numa_node;
         }
         const size_t E2 = e->def.extractions.size() + 2;
-        // UTF-8 input: offsets are in decoded units, known only piece after piece — one device per call
-        const size_t G = utf8 ? 1 : std::min(e->devs.size(), pieces.size());
+        // UTF-8 input with offsets in decoded units: those are known only piece after piece — one device per call
+        // (in byte coordinates the host knows every piece's position, as for ISO-8859-1)
+        const size_t G = utf8 && !byte_coords ? 1 : std::min(e->devs.size(), pieces.size());
         int64_t nl = 0;
         int32_t stride = 0;
         DeviceGuard restore_device;
         if (G <= 1) {
             DeviceRun run;
             std::lock_guard<std::mutex> lock(e->devs[0]->mu);
-            run_pieces(e, *e->devs[0], text, text8, utf8, off, pieces, 0, pieces.size(), hr.get(), run);
+            run_pieces(e, *e->devs[0], text, text8, utf8, byte_coords, off, pieces, 0, pieces.size(), hr.get(), run);
             nl = run.n_rows;
             stride = run.stride;
         } else {
@@ -1171,12 +1205,13 @@ int extract_host(gorp_engine* e, const uint16_t* text, const uint8_t* text8, int
             for (size_t d = 0; d < G; ++d)
                 th.emplace_back([&, d]() {
                     runs[d].status = guarded([&]() -> int {
-                        run_pieces(e, *e->devs[d], text, text8, false, off, pieces, first[d], first[d + 1], nullptr, runs[d]);
+                        run_pieces(e, *e->devs[d], text, text8, utf8, byte_coords, off, pieces, first[d], first[d + 1], nullptr, runs[d]);
                         return GORP_OK;
                     });
                     if (runs[d].status != GORP_OK) runs[d].error = g_error;
                 });
             for (auto& t : th) t.join();
+            // (the first device that failed: for malformed UTF-8 that is the lowest offending byte, the ranges being in byte order)
             for (size_t d = 0; d < G; ++d)
                 if (runs[d].status != GORP_OK) return fail(runs[d].status, runs[d].error);
             std::vector<int64_t> base(G + 1, 0);
@@ -1503,6 +1538,10 @@ int gorp_extract_text_latin1(gorp_engine* e, const uint8_t* text, int64_t n_byte
 
 int gorp_extract_text_utf8(gorp_engine* e, const uint8_t* text, int64_t n_bytes, gorp_result* out) {
     return extract_host(e, nullptr, text, n_bytes, nullptr, 0, out, true);
+}
+
+int gorp_extract_text_utf8_bytes(gorp_engine* e, const uint8_t* text, int64_t n_bytes, gorp_result* out) {
+    return extract_host(e, nullptr, text, n_bytes, nullptr, 0, out, true, true);
 }
 
 int gorp_match_all_lines(gorp_engine* e, const uint16_t* text, const int64_t* off, int64_t n_lines, gorp_match_result* out) {

@@ -297,6 +297,25 @@ void k_widen_latin1(const Launch&, const uint8_t* src, uint16_t* dst, int64_t n)
 int64_t utf8_tiles(int64_t n_bytes);
 void k_utf8_count(const Launch&, const uint8_t* src, int64_t n, uint32_t* tile_counts, unsigned long long* first_bad);
 void k_utf8_write(const Launch&, const uint8_t* src, int64_t n, const int64_t* tile_base, uint16_t* dst);
+// Byte coordinates of the UTF-8 input (gorp_extract_text_utf8_bytes), kernels/utf8.cu.
+// Count pass of K1 over the bytes (utf8_nl_count_mask_kernel): tile_counts[ceil(n / kNlTile)], masks[ceil(n / kNlTile) * 256]
+// in the layout of k1_count_newlines_masks, so k1_scatter_masks(masks, n, ...) writes the byte line offsets (entries 1..).
+void k_utf8_count_newlines_masks(const Launch&, const uint8_t* src, int64_t n, uint32_t* tile_counts, uint32_t* masks);
+// Gather of one piece's rows in byte coordinates (utf8_rows_kernel): out_off[i] = byte start of line i + bias (i <= n_lines,
+// out_off[n_lines] = end_off + bias), out_spans = the unit rows with every boundary moved to the byte offset of its sequence.
+struct Utf8RowsParams {
+    const uint8_t* bytes;        // the piece's UTF-8 bytes (16-byte aligned, readable up to the next 32-byte boundary)
+    const int64_t* unit_off;     // [n_lines + 1] line offsets of the decoded piece (K1)
+    const int64_t* byte_off;     // entries 1 .. of the byte line offsets (entry 0 is 0, entry n_lines is end_off)
+    const int32_t* spans;        // [n_lines * stride] rows in unit offsets
+    int64_t n_lines;
+    int64_t end_off;             // n_bytes, + 1 when the piece does not end in '\n'
+    int64_t bias;                // byte position of the piece in the caller's buffer
+    uint32_t stride;             // <= 64
+    int64_t* out_off;
+    int32_t* out_spans;
+};
+void k_utf8_rows(const Launch&, const Utf8RowsParams&);
 
 // matchAll (kernels/matchall.cu): the reference's own tables on the device
 struct MatchAllDev {

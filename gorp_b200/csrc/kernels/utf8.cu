@@ -9,6 +9,9 @@
 //           scan         exclusive prefix of the tile counts (scan_u32_to_i64)
 //   pass 2  utf8_write   block scan inside the tile, every thread decodes the sequences that START in its 16 bytes
 // Both passes are plain HBM streams (1 byte read per unit in pass 1, 1 byte read + 2 bytes written in pass 2).
+//
+// gorp_extract_text_utf8_bytes gives the same results in byte coordinates of the caller's buffer: a byte '\n' index of
+// the piece (utf8_nl_count_mask_kernel + K1's scatter) and a gather that converts the unit rows (utf8_rows_kernel).
 #include "device_common.cuh"
 
 namespace gorp {
@@ -156,9 +159,180 @@ __global__ void __launch_bounds__(kUtf8Threads) utf8_write_kernel(const uint8_t*
     }
 }
 
+// ------------------------------------------------------------------ byte coordinates (gorp_extract_text_utf8_bytes)
+// 0x01 per byte of w whose __vcmp*4 result byte is 0xFF, packed to bits 0..3
+__device__ __forceinline__ uint32_t byte_bits(uint32_t m) {
+    return ((m >> 7) & 1u) | ((m >> 14) & 2u) | ((m >> 21) & 4u) | ((m >> 28) & 8u);
+}
+
+// K1's count pass over BYTES: 32 bytes per thread (two 128-bit loads), '\n' found four bytes at a time (__vcmpeq4), one
+// 32-bit mask word per thread — the layout of nl_count_mask_kernel, so its scatter pass (nl_scatter_mask_kernel) turns the
+// masks into byte line offsets unchanged.
+__global__ void __launch_bounds__(kUtf8Threads) utf8_nl_count_mask_kernel(const uint8_t* __restrict__ src, int64_t n,
+                                                                         uint32_t* __restrict__ tile_counts, uint32_t* __restrict__ masks) {
+    static_assert(kNlTile == kUtf8Threads * 32, "one mask word = 32 bytes");
+    const int64_t mine = static_cast<int64_t>(blockIdx.x) * kNlTile + static_cast<int64_t>(threadIdx.x) * 32;
+    uint32_t mask = 0;  // bit k: byte mine+k is '\n'
+    if (mine + 32 <= n) {
+        const uint4* p = reinterpret_cast<const uint4*>(src + mine);
+        const uint4 a = __ldg(p), b = __ldg(p + 1);
+        const uint32_t w[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+#pragma unroll
+        for (int j = 0; j < 8; ++j) mask |= byte_bits(__vcmpeq4(w[j], 0x0A0A0A0Au)) << (4 * j);
+    } else {
+        for (int k = 0; k < 32; ++k)
+            if (mine + k < n && src[mine + k] == 0x0A) mask |= 1u << k;
+    }
+    masks[static_cast<int64_t>(blockIdx.x) * kUtf8Threads + threadIdx.x] = mask;
+    __shared__ uint32_t s_warp[kUtf8Threads / 32];
+    const uint32_t total = block_sum(static_cast<uint32_t>(__popc(mask)), s_warp);
+    if (threadIdx.x == 0) tile_counts[blockIdx.x] = total;
+}
+
+// Result rows of one piece in byte coordinates: ONE WARP per group of 32 lines.
+//  - lane l takes line 32 g + l: writes its byte offset (+ bias); the line is ASCII exactly when its byte length equals its
+//    unit length (a 2- or 3-byte sequence is 1 unit, a 4-byte sequence 2), and then its row is valid as it is: the warp
+//    copies the rows of the group's ASCII lines (coalesced).
+//  - every other line of the group is converted by the whole warp: the row's boundaries (unit offsets) are sorted in
+//    shared memory (bitonic, <= 64 keys), then the warp walks the line in 1024-byte windows, lane l counting the units of
+//    32 bytes; a warp scan gives the unit offset at each lane's slice, and the lane places the sorted boundaries that fall
+//    in its slice at the sequence starts that carry them. The walk stops once the last boundary is placed.
+//    Work per line: O(len / 32) per lane + the sort; a 100 KB line is 100 window steps of the warp, not a serial walk.
+// A boundary never falls inside a surrogate pair of text decoded from well-formed UTF-8 (no lone surrogates; capture
+// automata consume whole pairs), so every boundary lands on a sequence start.
+constexpr int kRowsThreads = 256;
+
+__global__ void __launch_bounds__(kRowsThreads) utf8_rows_kernel(Utf8RowsParams P) {
+    __shared__ unsigned long long s_keys[kRowsThreads / 32][64];
+    const uint32_t lane = threadIdx.x & 31u;
+    unsigned long long* keys = s_keys[threadIdx.x >> 5];
+    const uint32_t stride = P.stride;
+    const int64_t n = P.n_lines;
+    if (n == 0 && blockIdx.x == 0 && threadIdx.x == 0) P.out_off[0] = P.bias + P.end_off;
+    const int64_t n_groups = (n + 31) / 32;
+    const int64_t warps = static_cast<int64_t>(gridDim.x) * (kRowsThreads / 32);
+    for (int64_t g = static_cast<int64_t>(blockIdx.x) * (kRowsThreads / 32) + (threadIdx.x >> 5); g < n_groups; g += warps) {
+        const int64_t line = g * 32 + lane;
+        const bool valid = line < n;
+        int64_t u0 = 0, u1 = 0, b0 = 0, b1 = 0;
+        if (valid) {
+            u0 = P.unit_off[line];
+            u1 = P.unit_off[line + 1];
+            b0 = line == 0 ? 0 : P.byte_off[line];
+            b1 = line + 1 == n ? P.end_off : P.byte_off[line + 1];
+            P.out_off[line] = b0 + P.bias;
+            if (line + 1 == n) P.out_off[n] = b1 + P.bias;
+        }
+        if (stride == 0) continue;
+        uint32_t other = __ballot_sync(0xffffffffu, valid && b1 - b0 != u1 - u0);
+        {   // rows of the ASCII lines: as they are
+            const int64_t r0 = g * 32, cnt = (n - r0 < 32 ? n - r0 : 32) * stride;
+            const int32_t* __restrict__ in = P.spans + r0 * stride;
+            int32_t* __restrict__ out = P.out_spans + r0 * stride;
+            for (uint32_t i = lane; i < cnt; i += 32)
+                if (!((other >> (i / stride)) & 1u)) out[i] = in[i];
+        }
+        while (other) {
+            const int j = __ffs(other) - 1;
+            other &= other - 1;
+            const int64_t ln = g * 32 + j;
+            const int64_t lu0 = __shfl_sync(0xffffffffu, u0, j), lu1 = __shfl_sync(0xffffffffu, u1, j);
+            const int64_t lb0 = __shfl_sync(0xffffffffu, b0, j), lb1 = __shfl_sync(0xffffffffu, b1, j);
+            const int64_t len_u = lu1 - lu0 - 1, len_b = lb1 - lb0 - 1;
+            const int32_t* __restrict__ in = P.spans + ln * stride;
+            int32_t* __restrict__ out = P.out_spans + ln * stride;
+            // keys (unit offset << 8 | slot) of the boundaries inside the line; -1 stays -1, the line's end maps to its byte length
+            uint32_t m = 0;
+#pragma unroll
+            for (int r = 0; r < 2; ++r) {
+                const uint32_t s = lane + 32u * r;
+                const int32_t v = s < stride ? in[s] : -1;
+                const bool key = v >= 0 && v < len_u;
+                keys[s] = key ? (static_cast<unsigned long long>(v) << 8) | s : ~0ull;
+                if (s < stride && !key) out[s] = v < 0 ? -1 : static_cast<int32_t>(len_b);
+                m += __popc(__ballot_sync(0xffffffffu, key));
+            }
+            __syncwarp();
+            for (uint32_t k = 2; k <= 64; k <<= 1)  // bitonic sort of the 64 keys (padding ~0 sorts last)
+                for (uint32_t h = k >> 1; h > 0; h >>= 1) {
+                    const uint32_t i = (lane / h) * 2 * h + (lane % h), p = i + h;
+                    const unsigned long long x = keys[i], y = keys[p];
+                    if (((i & k) == 0) == (x > y)) {
+                        keys[i] = y;
+                        keys[p] = x;
+                    }
+                    __syncwarp();
+                }
+            if (m == 0) continue;
+            const int64_t last = static_cast<int64_t>(keys[m - 1] >> 8);
+            int64_t base = 0;  // units of the line before the current window
+            for (int64_t w = lb0 & ~int64_t(31); w < lb0 + len_b && base <= last; w += 1024) {
+                const int64_t s0 = w + 32 * static_cast<int64_t>(lane);
+                uint32_t lead = 0, four = 0;
+                if (s0 < lb0 + len_b && s0 + 32 > lb0) {
+                    const uint4* p = reinterpret_cast<const uint4*>(P.bytes + s0);
+                    const uint4 a = __ldg(p), b = __ldg(p + 1);
+                    const uint32_t x[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+#pragma unroll
+                    for (int q = 0; q < 8; ++q) {
+                        lead |= (byte_bits(__vcmpeq4(x[q] & 0xC0C0C0C0u, 0x80808080u)) ^ 0xFu) << (4 * q);
+                        four |= byte_bits(__vcmpgeu4(x[q], 0xF0F0F0F0u)) << (4 * q);
+                    }
+                    // only the bytes of the line
+                    const int64_t lo = lb0 - s0, hi = lb0 + len_b - s0;
+                    const uint32_t keep = (lo > 0 ? ~0u << lo : ~0u) & (hi < 32 ? (1u << hi) - 1u : ~0u);
+                    lead &= keep;
+                    four &= lead;
+                }
+                const uint32_t units = __popc(lead) + __popc(four);
+                uint32_t incl = units;
+#pragma unroll
+                for (int o = 1; o < 32; o <<= 1) {
+                    const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o);
+                    if (lane >= static_cast<uint32_t>(o)) incl += t;
+                }
+                int64_t c = base + (incl - units);  // unit offset of the first sequence that starts in this lane's slice
+                const int64_t c_end = c + units;
+                // first key >= c (binary search over the m sorted keys)
+                uint32_t lo = 0, hi = m;
+                while (lo < hi) {
+                    const uint32_t mid = (lo + hi) >> 1;
+                    if (static_cast<int64_t>(keys[mid] >> 8) < c) lo = mid + 1;
+                    else hi = mid;
+                }
+                if (lo < m && static_cast<int64_t>(keys[lo] >> 8) < c_end) {
+                    uint32_t bits = lead;
+                    while (bits && lo < m) {
+                        const int k = __ffs(bits) - 1;
+                        bits &= bits - 1;
+                        unsigned long long key;
+                        while (lo < m && static_cast<int64_t>((key = keys[lo]) >> 8) <= c) {
+                            out[key & 0xFFu] = static_cast<int32_t>(s0 + k - lb0);
+                            ++lo;
+                        }
+                        c += 1 + ((four >> k) & 1u);
+                    }
+                }
+                base += __shfl_sync(0xffffffffu, incl, 31);
+            }
+            __syncwarp();
+        }
+    }
+}
+
 }  // namespace
 
 int64_t utf8_tiles(int64_t n_bytes) { return (n_bytes + kUtf8Tile - 1) / kUtf8Tile; }
+
+void k_utf8_count_newlines_masks(const Launch& L, const uint8_t* src, int64_t n, uint32_t* tile_counts, uint32_t* masks) {
+    if (n <= 0) return;
+    utf8_nl_count_mask_kernel<<<static_cast<int>((n + kNlTile - 1) / kNlTile), kUtf8Threads, 0, L.stream>>>(src, n, tile_counts, masks);
+}
+
+void k_utf8_rows(const Launch& L, const Utf8RowsParams& P) {
+    const int64_t want = ((P.n_lines + 31) / 32 + kRowsThreads / 32 - 1) / (kRowsThreads / 32), cap = static_cast<int64_t>(L.sm_count) * 8;
+    utf8_rows_kernel<<<static_cast<int>(want < 1 ? 1 : want < cap ? want : cap), kRowsThreads, 0, L.stream>>>(P);
+}
 
 void k_utf8_count(const Launch& L, const uint8_t* src, int64_t n, uint32_t* tile_counts, unsigned long long* first_bad) {
     if (n <= 0) return;

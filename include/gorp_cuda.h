@@ -125,6 +125,11 @@ int gorp_extract_text_latin1(gorp_engine* e, const uint8_t* text, int64_t n_byte
  * sequence fails the call with GORP_E_ARG and the byte offset in gorp_last_error() — no replacement characters are
  * invented. Runs on the engine's first device. */
 int gorp_extract_text_utf8(gorp_engine* e, const uint8_t* text, int64_t n_bytes, gorp_result* out);
+/* Same call as gorp_extract_text_utf8, with the results in BYTE coordinates of the caller's buffer: line i is bytes
+ * [line_off[i], line_off[i+1] - 1) (line_off[n_lines] = n_bytes, + 1 when the text does not end in '\n'), spans are
+ * (start, end) byte offsets relative to the line's first byte. ext_id and histogram are those of gorp_extract_text_utf8.
+ * Runs on all of the engine's devices (contiguous line-aligned byte ranges, rows concatenated in device order). */
+int gorp_extract_text_utf8_bytes(gorp_engine* e, const uint8_t* text, int64_t n_bytes, gorp_result* out);
 void gorp_result_release(gorp_engine* e, gorp_result* r);
 
 /* PolyMatcher.match for a batch (reference autom/PolyMatcher.java:123-133, reached through Gorp.getMatcher(), Gorp.java:135-137):

@@ -21,7 +21,8 @@ import com.salesforce.gorp.model.CookedExtraction;
 public final class ExtractionBatch {
     /** extraction index per line: >= 0 matched, -1 miss (Gorp.extract returns null), <= -2: capture failure of extraction -2-e */
     public final int[] extId;
-    /** UTF-16 unit offsets of the lines in the batch text ('\n'-separated forms: line i = [lineOff[i], lineOff[i+1] - 1)) */
+    /** UTF-16 unit offsets of the lines in the batch text ('\n'-separated forms: line i = [lineOff[i], lineOff[i+1] - 1)); byte
+     *  offsets in the caller's buffer for a byte-coordinate batch ({@link GorpCuda#extractBatchUtf8Bytes}), spans too */
     public final long[] lineOff;
     /** spanStride ints per line: (start, end) of group 1..n relative to the line start, -1 = group did not participate */
     public final int[] spans;
@@ -32,9 +33,18 @@ public final class ExtractionBatch {
     private final CookedExtraction[] extractions;
     private final int[] groups;
     private final LongFunction<String> lines;
+    private final ByteSource bytes;
+
+    /** Decodes bytes [from, to) of the caller's buffer (byte-coordinate batches). */
+    interface ByteSource { String decode(long from, long to); }
 
     ExtractionBatch(int[] extId, long[] lineOff, int[] spans, int spanStride, long[] histogram, CookedExtraction[] extractions,
                     int[] groups, LongFunction<String> lines) {
+        this(extId, lineOff, spans, spanStride, histogram, extractions, groups, lines, null);
+    }
+
+    ExtractionBatch(int[] extId, long[] lineOff, int[] spans, int spanStride, long[] histogram, CookedExtraction[] extractions,
+                    int[] groups, LongFunction<String> lines, ByteSource bytes) {
         this.extId = extId;
         this.lineOff = lineOff;
         this.spans = spans;
@@ -43,6 +53,7 @@ public final class ExtractionBatch {
         this.extractions = extractions;
         this.groups = groups;
         this.lines = lines;
+        this.bytes = bytes;
     }
 
     public int size() { return extId.length; }
@@ -55,13 +66,18 @@ public final class ExtractionBatch {
     public CookedExtraction extraction(int i) { return extId[i] >= 0 ? extractions[extId[i]] : null; }
 
     /** Text of line i (decoded lazily from the caller's buffer). */
-    public String line(int i) { return lines.apply(i); }
+    public String line(int i) { return bytes != null ? bytes.decode(lineOff[i], lineOff[i + 1] - 1) : lines.apply(i); }
+
+    /** Text [a, b) of line i: a substring of the line, or in a byte-coordinate batch the decoded bytes [start + a, start + b). */
+    private String cut(int i, String line, int a, int b) {
+        return bytes != null ? bytes.decode(lineOff[i] + a, lineOff[i] + b) : line.substring(a, b);
+    }
 
     /** Value of capture group g (0-based) of line i without building an ExtractionResult; null when absent. */
     public String value(int i, int g) {
         if (extId[i] < 0 || g >= groups[extId[i]]) return null;
         int a = spans[i * spanStride + 2 * g], b = spans[i * spanStride + 2 * g + 1];
-        return a < 0 ? null : line(i).substring(a, b);
+        return a < 0 ? null : cut(i, bytes != null ? null : line(i), a, b);
     }
 
     /** What Gorp.extract(line i) returns: null for a miss; throws for a capture failure (Gorp.java:173-177). */
@@ -90,7 +106,7 @@ public final class ExtractionBatch {
         String[] values = new String[groups[e]];
         for (int g = 0; g < values.length; ++g) {
             int a = spans[i * spanStride + 2 * g], b = spans[i * spanStride + 2 * g + 1];
-            values[g] = a < 0 ? null : input.substring(a, b);
+            values[g] = a < 0 ? null : cut(i, input, a, b);
         }
         return extractions[e].constructMatch(input, values);
     }

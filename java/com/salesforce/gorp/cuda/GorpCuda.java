@@ -56,6 +56,8 @@ public final class GorpCuda implements AutoCloseable {
             FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS));
     private static final MethodHandle EXTRACT_TEXT_UTF8 = fn("gorp_extract_text_utf8",
             FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS));
+    private static final MethodHandle EXTRACT_TEXT_UTF8_BYTES = fn("gorp_extract_text_utf8_bytes",
+            FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS));
     // struct gorp_match_result { int64 n_lines; const int64* accept_off; const int32* accept; void* owner; }
     private static final StructLayout MATCH_RESULT = MemoryLayout.structLayout(
             JAVA_LONG.withName("n_lines"), ADDRESS.withName("accept_off"), ADDRESS.withName("accept"), ADDRESS.withName("owner"));
@@ -223,6 +225,38 @@ public final class GorpCuda implements AutoCloseable {
         }
     }
 
+    /**
+     * Same call as {@link #extractBatchUtf8}, with the results in BYTE coordinates of {@code text}: {@code lineOff} are byte
+     * offsets relative to the buffer's position and spans byte offsets relative to the line start, so neither the lines nor
+     * the offsets are rebuilt on the host; {@link ExtractionBatch#value} decodes only the value's bytes. Runs on all of the
+     * engine's devices. Malformed UTF-8 fails the call.
+     */
+    public ExtractionBatch extractBatchUtf8Bytes(java.nio.ByteBuffer text) throws Throwable {
+        try (Arena a = Arena.ofConfined()) {
+            MemorySegment seg;
+            if (text.isDirect()) {
+                seg = MemorySegment.ofBuffer(text);
+            } else {
+                seg = a.allocate(Math.max(text.remaining(), 1), 16);
+                MemorySegment.copy(MemorySegment.ofBuffer(text), 0, seg, 0, text.remaining());
+            }
+            final java.nio.ByteBuffer view = text.duplicate();
+            final int base = view.position();
+            MemorySegment res = a.allocate(RESULT);
+            check((int) EXTRACT_TEXT_UTF8_BYTES.invokeExact(engine, seg, (long) text.remaining(), res));
+            try {
+                final int n = (int) res.get(JAVA_LONG, 0);
+                return batch(res, n, null, (from, to) -> {
+                    byte[] b = new byte[(int) (to - from)];
+                    view.get(base + (int) from, b);
+                    return new String(b, java.nio.charset.StandardCharsets.UTF_8);
+                });
+            } finally {
+                RESULT_RELEASE.invokeExact(engine, res);
+            }
+        }
+    }
+
     /** Columnar batch over a List&lt;String&gt; (Gorp.extractAll without materialising every ExtractionResult). */
     public ExtractionBatch extractBatch(List<String> lines) throws Throwable {
         final int n = lines.size();
@@ -286,12 +320,17 @@ public final class GorpCuda implements AutoCloseable {
 
     /** Copies the native result columns into heap arrays (the native buffers go back to the engine's pool). */
     private ExtractionBatch batch(MemorySegment res, int n, java.util.function.LongFunction<String> lines) {
+        return batch(res, n, lines, null);
+    }
+
+    /** With {@code bytes} (byte-coordinate results): lines and values are cut from the caller's buffer. */
+    private ExtractionBatch batch(MemorySegment res, int n, java.util.function.LongFunction<String> lines, ExtractionBatch.ByteSource bytes) {
         final int stride = res.get(JAVA_INT, 12), nExt = res.get(JAVA_INT, 8);
         int[] extId = res.get(ADDRESS, 16).reinterpret(4L * Math.max(n, 1)).asSlice(0, 4L * n).toArray(JAVA_INT);
         long[] lineOff = res.get(ADDRESS, 24).reinterpret(8L * (n + 1)).toArray(JAVA_LONG);
         int[] spans = res.get(ADDRESS, 32).reinterpret(4L * Math.max((long) n * stride, 1)).asSlice(0, 4L * n * stride).toArray(JAVA_INT);
         long[] hist = res.get(ADDRESS, 40).reinterpret(8L * (nExt + 2)).toArray(JAVA_LONG);
-        return new ExtractionBatch(extId, lineOff, spans, stride, hist, extractions, groups, lines);
+        return new ExtractionBatch(extId, lineOff, spans, stride, hist, extractions, groups, lines, bytes);
     }
 
     private interface LineSource { String line(long i); }
