@@ -52,7 +52,7 @@ class DeviceResult(C.Structure):
 SYMBOLS = [
     "gorp_abi_version", "gorp_last_error", "gorp_device_count", "gorp_compile_definition", "gorp_compile_patterns",
     "gorp_blob_free", "gorp_blob_get_info", "gorp_blob_get_extraction", "gorp_blob_get_extractor_name",
-    "gorp_blob_get_tables", "gorp_engine_create", "gorp_engine_destroy", "gorp_extract_lines", "gorp_extract_text", "gorp_extract_text_latin1", "gorp_extract_text_utf8", "gorp_extract_text_utf8_bytes", "gorp_match_all_lines", "gorp_match_result_release",
+    "gorp_blob_get_tables", "gorp_engine_create", "gorp_engine_destroy", "gorp_extract_lines", "gorp_extract_text", "gorp_extract_text_latin1", "gorp_extract_text_utf8", "gorp_extract_text_utf8_bytes", "gorp_extract_lines_utf8", "gorp_match_all_lines", "gorp_match_result_release",
     "gorp_result_release", "gorp_extract_text_device", "gorp_extract_lines_device", "gorp_kernel_times",
 ]
 
@@ -79,6 +79,7 @@ lib.gorp_extract_text.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(R
 lib.gorp_extract_text_latin1.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(Result)]
 lib.gorp_extract_text_utf8.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(Result)]
 lib.gorp_extract_text_utf8_bytes.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(Result)]
+lib.gorp_extract_lines_utf8.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(Result)]
 lib.gorp_match_all_lines.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(MatchResult)]
 lib.gorp_match_result_release.argtypes = [C.c_void_p, C.POINTER(MatchResult)]
 lib.gorp_match_result_release.restype = None

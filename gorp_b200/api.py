@@ -291,6 +291,33 @@ class Gorp:
         finally:
             lib.gorp_result_release(self._eng(), C.byref(res))
 
+    def extract_batch_lines_utf8(self, lines, offsets=None) -> ExtractionBatch:
+        """extract_batch_lines for strings held as UTF-8 bytes (gorp_extract_lines_utf8, all of the engine's devices): a '\\n'
+        inside a string is data. `lines` is a sequence of bytes / str (str is UTF-8-encoded), or with `offsets` a bytes-like
+        buffer in which string i is bytes [offsets[i], offsets[i+1]) (int64; offsets[0] may be > 0, as in an Arrow slice).
+        line_off and spans are byte offsets into that buffer; the batch decodes only what a line(), spans_of() or result()
+        asks for. A string that is not well-formed UTF-8 on its own raises ValueError."""
+        if offsets is None:
+            parts = [s.encode("utf-8") if isinstance(s, str) else bytes(s) for s in lines]
+            off = np.zeros(len(parts) + 1, dtype=np.int64)
+            if parts:
+                np.cumsum([len(p) for p in parts], out=off[1:])
+            b = np.frombuffer(b"".join(parts), dtype=np.uint8)
+        else:
+            b = np.ascontiguousarray(np.frombuffer(lines, dtype=np.uint8) if isinstance(lines, (bytes, bytearray, memoryview)) else lines,
+                                     dtype=np.uint8)
+            off = np.ascontiguousarray(offsets, dtype=np.int64)
+            if off.ndim != 1 or len(off) < 1:
+                raise ValueError("offsets must hold n_lines + 1 entries")
+            if int(off[-1]) > len(b):
+                raise ValueError("offsets reach past the end of the buffer")
+        res = _ffi.Result()
+        _check(lib.gorp_extract_lines_utf8(self._eng(), b.ctypes.data, off.ctypes.data, len(off) - 1, C.byref(res)))
+        try:
+            return ExtractionBatch(self, b, res, 0, encoding="utf-8")
+        finally:
+            lib.gorp_result_release(self._eng(), C.byref(res))
+
     def extract_batch_text(self, text) -> ExtractionBatch:
         """Gorp.extractAll(CharBuffer): '\\n'-separated UTF-16 text (str or uint16 array)."""
         units = np.ascontiguousarray(to_units(text), dtype=np.uint16)

@@ -160,6 +160,7 @@ struct DeviceCtx {
     cudaEvent_t ev_done = nullptr;  // end of the last call on this context: the next call's stream waits for it (shared scratch)
     DevBuf textbuf[2], offbuf[2], bytebuf[2], acc_ext, acc_off, acc_spans, acc_hist;
     DevBuf byte_off;  // byte line offsets of a UTF-8 piece (byte coordinates)
+    DevBuf unit_off, slice_units;  // UTF-8 strings (gorp_extract_lines_utf8): unit offsets of the piece's strings, count-pass slice prefixes
     // per-call scratch, serialised by `mu`
     std::mutex mu;
     DevBuf text, off_in, line_off, tile_counts, tile_base, scan_scratch, ext_id, spans, hist, scalars;
@@ -978,7 +979,9 @@ struct DeviceRun {  // what one device produced for its pieces
 // rows of every finished piece are copied to the host arrays at once, overlapping the next pieces.
 // `text8` (ISO-8859-1 bytes, text form only) replaces `text`: the bytes are staged and widened to UTF-16 on the device.
 // `utf8`: the bytes are UTF-8, decoded on the device; offsets count UTF-16 units of the decoded text, or with `byte_coords`
-// bytes of `text8` (then the pieces are independent, as for ISO-8859-1).
+// bytes of `text8` (then the pieces are independent, as for ISO-8859-1). `utf8` with `off` (always in byte coordinates): the
+// caller's strings are bytes [off[i], off[i+1]) of `text8`; the piece is decoded at textbuf + kTextPad, its strings' unit
+// offsets (relative to the piece) feed the lines form of the pipeline, and the rows go back to the caller's byte offsets.
 // The caller holds c.mu (a multi-device call keeps every participating device locked until its rows are copied out).
 void run_pieces(gorp_engine* e, DeviceCtx& c, const uint16_t* text, const uint8_t* text8, bool utf8, bool byte_coords, const int64_t* off,
                 const std::vector<Piece>& pieces, size_t p0, size_t p1, HostResult* hr, DeviceRun& run) {
@@ -1000,6 +1003,10 @@ void run_pieces(gorp_engine* e, DeviceCtx& c, const uint16_t* text, const uint8_
         c.textbuf[b].reserve((max_units + kTextPad + 64) * 2);
         if (text8) c.bytebuf[b].reserve(max_units + 64);
         if (off) c.offbuf[b].reserve((max_lines + 1) * 8);
+    }
+    if (off && utf8) {
+        c.unit_off.reserve((max_lines + 1) * 8);
+        c.slice_units.reserve((max_units / 16 + 1) * 2);
     }
     // row capacity: exact for the lines form; for the text form sized for the first piece from the running density
     // estimate, then (below) for the whole range from the density actually seen
@@ -1046,7 +1053,33 @@ void run_pieces(gorp_engine* e, DeviceCtx& c, const uint16_t* text, const uint8_
         int64_t piece_bias = pc.u0;  // what turns the piece's line offsets into offsets of the whole batch
         gorp_device_result dr{};
         int64_t nl;
-        if (off) {
+        if (off && utf8) {
+            // UTF-8 strings: count + validate, scan, unit offsets of the strings + boundary validation, (one host round trip:
+            // total + first malformed byte), decode; then the lines form over the decoded piece
+            const int64_t tiles = utf8_tiles(units), n_lines_piece = pc.l1 - pc.l0;
+            c.tile_counts.reserve(static_cast<size_t>(tiles + 1) * 4);
+            c.tile_base.reserve(static_cast<size_t>(tiles + 2) * 8);
+            c.scan_scratch.reserve(static_cast<size_t>(tiles / 4096 + 8) * 8);
+            c.scalars.reserve(128);
+            unsigned long long* d_bad = reinterpret_cast<unsigned long long*>(c.scalars.as<int64_t>() + 6);
+            unsigned long long bad = ~0ull;
+            int64_t total = 0;
+            CK(cudaMemsetAsync(d_bad, 0xFF, 8, c.stream));
+            k_utf8_count(L, c.bytebuf[b].as<uint8_t>(), units, c.tile_counts.as<uint32_t>(), d_bad, c.slice_units.as<uint16_t>());
+            scan_u32_to_i64(L, c.tile_counts.as<uint32_t>(), tiles, c.tile_base.as<int64_t>(), c.scan_scratch.as<int64_t>());
+            k_utf8_line_units(L, c.bytebuf[b].as<uint8_t>(), units, c.offbuf[b].as<int64_t>(), n_lines_piece + 1, pc.u0, c.tile_base.as<int64_t>(),
+                              c.slice_units.as<uint16_t>(), c.unit_off.as<int64_t>(), d_bad);
+            if (units > 0) CK(cudaMemcpyAsync(&total, c.tile_base.as<int64_t>() + tiles, 8, cudaMemcpyDeviceToHost, c.stream));
+            CK(cudaMemcpyAsync(&bad, d_bad, 8, cudaMemcpyDeviceToHost, c.stream));
+            CK(cudaStreamSynchronize(c.stream));
+            if (bad != ~0ull)
+                throw ArgError(strfmt("malformed UTF-8 at byte %lld (every string must be well-formed UTF-8)",
+                                      static_cast<long long>(pc.u0 + static_cast<int64_t>(bad))));
+            uint16_t* piece_text = c.textbuf[b].as<uint16_t>() + kTextPad;  // (device address - unit index) a multiple of 32 bytes
+            k_utf8_write(L, c.bytebuf[b].as<uint8_t>(), units, c.tile_base.as<int64_t>(), piece_text);
+            c.launches += 6;
+            nl = run_pipeline(c, piece_text, total, c.unit_off.as<int64_t>(), n_lines_piece, c.stream, false, &dr);
+        } else if (off) {
             const uint16_t* vbase = c.textbuf[b].as<uint16_t>() + kTextPad + (pc.u0 & 15) - pc.u0;  // text[i] lives at vbase + i
             nl = run_pipeline(c, vbase, pc.u1, c.offbuf[b].as<int64_t>(), pc.l1 - pc.l0, c.stream, false, &dr);  // text[i] valid for i < u1
         } else {
@@ -1091,7 +1124,22 @@ void run_pieces(gorp_engine* e, DeviceCtx& c, const uint16_t* text, const uint8_
         }
         // gather: rows [rows, rows + nl) of the batch
         if (nl) CK(cudaMemcpyAsync(c.acc_ext.as<int32_t>() + rows, dr.d_ext_id, static_cast<size_t>(nl) * 4, cudaMemcpyDeviceToDevice, c.stream));
-        if (utf8 && byte_coords) {
+        if (off && utf8) {
+            // rows back to the caller's byte offsets (line_off is a copy of the caller's offsets)
+            if (stride > 64) throw std::logic_error("result rows wider than 64 entries");  // (31 groups at most: 62)
+            Utf8RowsParams P{};
+            P.bytes = c.bytebuf[b].as<uint8_t>();
+            P.unit_off = dr.d_line_off;
+            P.byte_off = c.offbuf[b].as<int64_t>();
+            P.spans = dr.d_spans;
+            P.n_lines = nl;
+            P.bias = pc.u0;
+            P.stride = stride;
+            P.out_off = c.acc_off.as<int64_t>() + rows;
+            P.out_spans = c.acc_spans.as<int32_t>() + static_cast<size_t>(rows) * stride;
+            k_utf8_rows(L, P, true);
+            c.launches += 1;
+        } else if (utf8 && byte_coords) {
             // byte '\n' index of the piece, built after run_pipeline (which reuses tile_counts, tile_base, scan_scratch and
             // nl_masks); line k of the bytes is line k of the decoded text (same '\n' characters). Then the gather converts
             // the rows from the piece's unit offsets to byte offsets.
@@ -1163,7 +1211,7 @@ int extract_host(gorp_engine* e, const uint16_t* text, const uint8_t* text8, int
         // round 2): 149 -> 132 ms per 100 M lines of Latin-1 input
         int64_t piece_units = text8 ? 4 * kPieceUnits : kPieceUnits;
         // (the lines form pays two copies and a longer kernel chain per piece: larger pieces once the batch has 16 of them)
-        if (off && n_lines > 0) piece_units = std::min<int64_t>(4 * kPieceUnits, std::max<int64_t>(kPieceUnits, n_units / 16));
+        if (off && n_lines > 0 && !text8) piece_units = std::min<int64_t>(4 * kPieceUnits, std::max<int64_t>(kPieceUnits, n_units / 16));
         if (const char* f = std::getenv("GORP_PIECE_UNITS")) piece_units = std::max<int64_t>(std::atoll(f), 1024);
         const std::vector<Piece> pieces = text8 ? plan_pieces(text8, n_units, off, n_lines, piece_units) : plan_pieces(text, n_units, off, n_lines, piece_units);
         std::unique_ptr<HostResult> hr;
@@ -1542,6 +1590,14 @@ int gorp_extract_text_utf8(gorp_engine* e, const uint8_t* text, int64_t n_bytes,
 
 int gorp_extract_text_utf8_bytes(gorp_engine* e, const uint8_t* text, int64_t n_bytes, gorp_result* out) {
     return extract_host(e, nullptr, text, n_bytes, nullptr, 0, out, true, true);
+}
+
+int gorp_extract_lines_utf8(gorp_engine* e, const uint8_t* text, const int64_t* off, int64_t n_lines, gorp_result* out) {
+    if (!e || !out || !off || n_lines < 0) return fail(GORP_E_ARG, "bad argument");
+    if (off[0] < 0) return fail(GORP_E_ARG, "offsets must start at >= 0");
+    if (const int64_t i = first_decreasing_offset(off, n_lines); i >= 0)
+        return fail(GORP_E_ARG, strfmt("offsets must be non-decreasing (line %lld)", static_cast<long long>(i)));
+    return extract_host(e, nullptr, text, n_lines > 0 ? off[n_lines] : 0, off, n_lines, out, true, true);
 }
 
 int gorp_match_all_lines(gorp_engine* e, const uint16_t* text, const int64_t* off, int64_t n_lines, gorp_match_result* out) {

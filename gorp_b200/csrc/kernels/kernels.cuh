@@ -295,7 +295,8 @@ void k_widen_latin1(const Launch&, const uint8_t* src, uint16_t* dst, int64_t n)
 // count: tile_counts[utf8_tiles(n)] = UTF-16 units per 4096-byte tile, *first_bad = offset of the first malformed byte (preset
 // to ~0 by the caller); write: tile_base = exclusive scan of tile_counts.
 int64_t utf8_tiles(int64_t n_bytes);
-void k_utf8_count(const Launch&, const uint8_t* src, int64_t n, uint32_t* tile_counts, unsigned long long* first_bad);
+// slice_units (lines form, else nullptr): [ceil(n / 16)] units of the 4096-byte tile before each 16-byte slice
+void k_utf8_count(const Launch&, const uint8_t* src, int64_t n, uint32_t* tile_counts, unsigned long long* first_bad, uint16_t* slice_units = nullptr);
 void k_utf8_write(const Launch&, const uint8_t* src, int64_t n, const int64_t* tile_base, uint16_t* dst);
 // Byte coordinates of the UTF-8 input (gorp_extract_text_utf8_bytes), kernels/utf8.cu.
 // Count pass of K1 over the bytes (utf8_nl_count_mask_kernel): tile_counts[ceil(n / kNlTile)], masks[ceil(n / kNlTile) * 256]
@@ -315,7 +316,14 @@ struct Utf8RowsParams {
     int64_t* out_off;
     int32_t* out_spans;
 };
-void k_utf8_rows(const Launch&, const Utf8RowsParams&);
+// lines = true: the List<String> form over UTF-8 strings (gorp_extract_lines_utf8): no separator, byte_off is the caller's
+// offsets [n_lines + 1] (the piece's bytes start at caller byte `bias`), out_off their copy; end_off is not used.
+void k_utf8_rows(const Launch&, const Utf8RowsParams&, bool lines = false);
+// Unit offsets of the strings of a UTF-8 piece (utf8_line_units_kernel): unit_off[i] = UTF-16 units of the decoded piece
+// before byte byte_off[i] - base, from the count pass's tile_base (scanned) and slice_units; an interior offset that cuts a
+// sequence or starts with a continuation byte sets first_bad (atomicMin) to the byte at which a string fails on its own.
+void k_utf8_line_units(const Launch&, const uint8_t* src, int64_t n, const int64_t* byte_off, int64_t n_off, int64_t base, const int64_t* tile_base,
+                       const uint16_t* slice_units, int64_t* unit_off, unsigned long long* first_bad);
 
 // matchAll (kernels/matchall.cu): the reference's own tables on the device
 struct MatchAllDev {

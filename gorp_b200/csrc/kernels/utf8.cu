@@ -12,6 +12,11 @@
 //
 // gorp_extract_text_utf8_bytes gives the same results in byte coordinates of the caller's buffer: a byte '\n' index of
 // the piece (utf8_nl_count_mask_kernel + K1's scatter) and a gather that converts the unit rows (utf8_rows_kernel).
+//
+// gorp_extract_lines_utf8 (strings as UTF-8 bytes + offsets): pass 1 also leaves a unit prefix per 16-byte slice, then
+// utf8_line_units_kernel turns each string's byte offset into its unit offset and checks that no string boundary cuts a
+// sequence; after pass 2 the lines form of the pipeline runs on the decoded piece and utf8_rows_kernel<true> maps its rows
+// back to the caller's bytes.
 #include "device_common.cuh"
 
 namespace gorp {
@@ -24,6 +29,11 @@ constexpr int kUtf8Tile = kUtf8Threads * kUtf8PerThread;
 
 __device__ __forceinline__ uint32_t byte_at(const uint8_t* __restrict__ src, int64_t i, int64_t n) {
     return i < n ? static_cast<uint32_t>(__ldg(src + i)) : 0x100u;  // 0x100: "no byte" (never a continuation byte)
+}
+
+// 0x01 per byte of w whose __vcmp*4 result byte is 0xFF, packed to bits 0..3
+__device__ __forceinline__ uint32_t byte_bits(uint32_t m) {
+    return ((m >> 7) & 1u) | ((m >> 14) & 2u) | ((m >> 21) & 4u) | ((m >> 28) & 8u);
 }
 
 // length of the well-formed sequence that starts with lead byte b0 at position i (1..4), or 0 when malformed
@@ -54,8 +64,11 @@ __device__ __forceinline__ uint32_t block_sum(uint32_t v, uint32_t* s_warp) {
     return t;
 }
 
+// kLines (gorp_extract_lines_utf8): also writes slice_units[i] = units of the tile before the 16-byte slice i (exclusive,
+// tile-relative: < 4096, a u16), so that a string's unit offset is one lookup away (utf8_line_units_kernel).
+template <bool kLines>
 __global__ void __launch_bounds__(kUtf8Threads) utf8_count_kernel(const uint8_t* __restrict__ src, int64_t n, uint32_t* __restrict__ tile_counts,
-                                                                 unsigned long long* __restrict__ first_bad) {
+                                                                 unsigned long long* __restrict__ first_bad, uint16_t* __restrict__ slice_units) {
     __shared__ uint32_t s_warp[kUtf8Threads / 32];
     const int64_t n_tiles = (n + kUtf8Tile - 1) / kUtf8Tile;
     for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
@@ -99,8 +112,74 @@ __global__ void __launch_bounds__(kUtf8Threads) utf8_count_kernel(const uint8_t*
                 units += c >= 0xF0u ? 2u : 1u;
             }
         }
-        const uint32_t total = block_sum(units, s_warp);
-        if (threadIdx.x == 0) tile_counts[tile] = total;
+        if constexpr (kLines) {
+            const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+            uint32_t incl = units;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o);
+                if (lane >= static_cast<uint32_t>(o)) incl += t;
+            }
+            if (lane == 31) s_warp[warp] = incl;
+            __syncthreads();
+            uint32_t before = 0, total = 0;
+            for (uint32_t w = 0; w < kUtf8Threads / 32; ++w) {
+                before += w < warp ? s_warp[w] : 0u;
+                total += s_warp[w];
+            }
+            __syncthreads();
+            if (p0 < n) slice_units[p0 / kUtf8PerThread] = static_cast<uint16_t>(before + incl - units);
+            if (threadIdx.x == 0) tile_counts[tile] = total;
+        } else {
+            const uint32_t total = block_sum(units, s_warp);
+            if (threadIdx.x == 0) tile_counts[tile] = total;
+        }
+    }
+}
+
+// Unit offsets of the strings of one piece (gorp_extract_lines_utf8), one thread per offset: byte offset b (relative to the
+// piece) -> tile_base[b / 4096] + slice_units[b / 16] + units of bytes [b & ~15, b) (one 16-byte load), O(1) per string.
+// It also checks the boundaries the count pass cannot see: a string that ends inside a sequence the next string completes
+// (the concatenation is well-formed, the strings are not). For an interior offset b whose byte is a continuation byte, the
+// string before b fails at the lead p of the cut sequence (p in [b - 3, b), the sequence reaching past b); with no such lead,
+// the string that starts at b fails at b. The lowest offending byte goes to first_bad (atomicMin, as the count pass).
+__global__ void __launch_bounds__(kUtf8Threads) utf8_line_units_kernel(const uint8_t* __restrict__ src, int64_t n, const int64_t* __restrict__ byte_off,
+                                                                      int64_t n_off, int64_t base, const int64_t* __restrict__ tile_base,
+                                                                      const uint16_t* __restrict__ slice_units, int64_t* __restrict__ unit_off,
+                                                                      unsigned long long* __restrict__ first_bad) {
+    const int64_t n_tiles = (n + kUtf8Tile - 1) / kUtf8Tile;
+    for (int64_t i = static_cast<int64_t>(blockIdx.x) * kUtf8Threads + threadIdx.x; i < n_off; i += static_cast<int64_t>(gridDim.x) * kUtf8Threads) {
+        const int64_t b = byte_off[i] - base;
+        int64_t u;
+        if (b <= 0 || n <= 0) {  // (an empty piece: its offsets all equal the piece start, nothing was scanned)
+            u = 0;
+        } else if (b >= n) {
+            u = tile_base[n_tiles];
+        } else {
+            const uint4 v = __ldg(reinterpret_cast<const uint4*>(src + (b & ~int64_t(15))));
+            const uint32_t x[4] = {v.x, v.y, v.z, v.w};
+            uint32_t lead = 0, four = 0;
+#pragma unroll
+            for (int q = 0; q < 4; ++q) {
+                lead |= (byte_bits(__vcmpeq4(x[q] & 0xC0C0C0C0u, 0x80808080u)) ^ 0xFu) << (4 * q);
+                four |= byte_bits(__vcmpgeu4(x[q], 0xF0F0F0F0u)) << (4 * q);
+            }
+            const uint32_t k = static_cast<uint32_t>(b & 15), before = (1u << k) - 1u;
+            u = tile_base[b / kUtf8Tile] + slice_units[b / kUtf8PerThread] + __popc(lead & before) + __popc(four & lead & before);
+            if (!((lead >> k) & 1u)) {  // b cuts a sequence, or starts with a stray continuation byte
+                int64_t bad = b;
+                for (int back = 1; back <= 3 && b - back >= 0; ++back) {
+                    const uint32_t pb = __ldg(src + b - back);
+                    if ((pb & 0xC0u) != 0x80u) {
+                        const int len = pb >= 0xF0u ? 4 : pb >= 0xE0u ? 3 : pb >= 0xC0u ? 2 : 1;
+                        if (len > back) bad = b - back;
+                        break;
+                    }
+                }
+                atomicMin(first_bad, static_cast<unsigned long long>(bad));
+            }
+        }
+        unit_off[i] = u;
     }
 }
 
@@ -160,10 +239,6 @@ __global__ void __launch_bounds__(kUtf8Threads) utf8_write_kernel(const uint8_t*
 }
 
 // ------------------------------------------------------------------ byte coordinates (gorp_extract_text_utf8_bytes)
-// 0x01 per byte of w whose __vcmp*4 result byte is 0xFF, packed to bits 0..3
-__device__ __forceinline__ uint32_t byte_bits(uint32_t m) {
-    return ((m >> 7) & 1u) | ((m >> 14) & 2u) | ((m >> 21) & 4u) | ((m >> 28) & 8u);
-}
 
 // K1's count pass over BYTES: 32 bytes per thread (two 128-bit loads), '\n' found four bytes at a time (__vcmpeq4), one
 // 32-bit mask word per thread — the layout of nl_count_mask_kernel, so its scatter pass (nl_scatter_mask_kernel) turns the
@@ -200,15 +275,18 @@ __global__ void __launch_bounds__(kUtf8Threads) utf8_nl_count_mask_kernel(const 
 //    Work per line: O(len / 32) per lane + the sort; a 100 KB line is 100 window steps of the warp, not a serial walk.
 // A boundary never falls inside a surrogate pair of text decoded from well-formed UTF-8 (no lone surrogates; capture
 // automata consume whole pairs), so every boundary lands on a sequence start.
+// kLines (gorp_extract_lines_utf8): no separator; byte_off is the caller's offsets [n_lines + 1] (the piece starts at byte
+// `bias` of the caller's buffer), and out_off is a copy of them.
 constexpr int kRowsThreads = 256;
 
+template <bool kLines>
 __global__ void __launch_bounds__(kRowsThreads) utf8_rows_kernel(Utf8RowsParams P) {
     __shared__ unsigned long long s_keys[kRowsThreads / 32][64];
     const uint32_t lane = threadIdx.x & 31u;
     unsigned long long* keys = s_keys[threadIdx.x >> 5];
     const uint32_t stride = P.stride;
     const int64_t n = P.n_lines;
-    if (n == 0 && blockIdx.x == 0 && threadIdx.x == 0) P.out_off[0] = P.bias + P.end_off;
+    if (n == 0 && blockIdx.x == 0 && threadIdx.x == 0) P.out_off[0] = kLines ? P.byte_off[0] : P.bias + P.end_off;
     const int64_t n_groups = (n + 31) / 32;
     const int64_t warps = static_cast<int64_t>(gridDim.x) * (kRowsThreads / 32);
     for (int64_t g = static_cast<int64_t>(blockIdx.x) * (kRowsThreads / 32) + (threadIdx.x >> 5); g < n_groups; g += warps) {
@@ -218,8 +296,13 @@ __global__ void __launch_bounds__(kRowsThreads) utf8_rows_kernel(Utf8RowsParams 
         if (valid) {
             u0 = P.unit_off[line];
             u1 = P.unit_off[line + 1];
-            b0 = line == 0 ? 0 : P.byte_off[line];
-            b1 = line + 1 == n ? P.end_off : P.byte_off[line + 1];
+            if constexpr (kLines) {
+                b0 = P.byte_off[line] - P.bias;
+                b1 = P.byte_off[line + 1] - P.bias;
+            } else {
+                b0 = line == 0 ? 0 : P.byte_off[line];
+                b1 = line + 1 == n ? P.end_off : P.byte_off[line + 1];
+            }
             P.out_off[line] = b0 + P.bias;
             if (line + 1 == n) P.out_off[n] = b1 + P.bias;
         }
@@ -238,7 +321,8 @@ __global__ void __launch_bounds__(kRowsThreads) utf8_rows_kernel(Utf8RowsParams 
             const int64_t ln = g * 32 + j;
             const int64_t lu0 = __shfl_sync(0xffffffffu, u0, j), lu1 = __shfl_sync(0xffffffffu, u1, j);
             const int64_t lb0 = __shfl_sync(0xffffffffu, b0, j), lb1 = __shfl_sync(0xffffffffu, b1, j);
-            const int64_t len_u = lu1 - lu0 - 1, len_b = lb1 - lb0 - 1;
+            constexpr int64_t sep = kLines ? 0 : 1;
+            const int64_t len_u = lu1 - lu0 - sep, len_b = lb1 - lb0 - sep;
             const int32_t* __restrict__ in = P.spans + ln * stride;
             int32_t* __restrict__ out = P.out_spans + ln * stride;
             // keys (unit offset << 8 | slot) of the boundaries inside the line; -1 stays -1, the line's end maps to its byte length
@@ -329,15 +413,27 @@ void k_utf8_count_newlines_masks(const Launch& L, const uint8_t* src, int64_t n,
     utf8_nl_count_mask_kernel<<<static_cast<int>((n + kNlTile - 1) / kNlTile), kUtf8Threads, 0, L.stream>>>(src, n, tile_counts, masks);
 }
 
-void k_utf8_rows(const Launch& L, const Utf8RowsParams& P) {
+void k_utf8_rows(const Launch& L, const Utf8RowsParams& P, bool lines) {
     const int64_t want = ((P.n_lines + 31) / 32 + kRowsThreads / 32 - 1) / (kRowsThreads / 32), cap = static_cast<int64_t>(L.sm_count) * 8;
-    utf8_rows_kernel<<<static_cast<int>(want < 1 ? 1 : want < cap ? want : cap), kRowsThreads, 0, L.stream>>>(P);
+    const int grid = static_cast<int>(want < 1 ? 1 : want < cap ? want : cap);
+    if (lines) utf8_rows_kernel<true><<<grid, kRowsThreads, 0, L.stream>>>(P);
+    else utf8_rows_kernel<false><<<grid, kRowsThreads, 0, L.stream>>>(P);
 }
 
-void k_utf8_count(const Launch& L, const uint8_t* src, int64_t n, uint32_t* tile_counts, unsigned long long* first_bad) {
+void k_utf8_count(const Launch& L, const uint8_t* src, int64_t n, uint32_t* tile_counts, unsigned long long* first_bad, uint16_t* slice_units) {
     if (n <= 0) return;
     const int64_t tiles = utf8_tiles(n), cap = static_cast<int64_t>(L.sm_count) * 8;
-    utf8_count_kernel<<<static_cast<int>(tiles < cap ? tiles : cap), kUtf8Threads, 0, L.stream>>>(src, n, tile_counts, first_bad);
+    const int grid = static_cast<int>(tiles < cap ? tiles : cap);
+    if (slice_units) utf8_count_kernel<true><<<grid, kUtf8Threads, 0, L.stream>>>(src, n, tile_counts, first_bad, slice_units);
+    else utf8_count_kernel<false><<<grid, kUtf8Threads, 0, L.stream>>>(src, n, tile_counts, first_bad, nullptr);
+}
+
+void k_utf8_line_units(const Launch& L, const uint8_t* src, int64_t n, const int64_t* byte_off, int64_t n_off, int64_t base, const int64_t* tile_base,
+                       const uint16_t* slice_units, int64_t* unit_off, unsigned long long* first_bad) {
+    if (n_off <= 0) return;
+    const int64_t want = (n_off + kUtf8Threads - 1) / kUtf8Threads, cap = static_cast<int64_t>(L.sm_count) * 16;
+    utf8_line_units_kernel<<<static_cast<int>(want < cap ? want : cap), kUtf8Threads, 0, L.stream>>>(src, n, byte_off, n_off, base, tile_base,
+                                                                                                    slice_units, unit_off, first_bad);
 }
 
 void k_utf8_write(const Launch& L, const uint8_t* src, int64_t n, const int64_t* tile_base, uint16_t* dst) {

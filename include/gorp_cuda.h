@@ -130,6 +130,14 @@ int gorp_extract_text_utf8(gorp_engine* e, const uint8_t* text, int64_t n_bytes,
  * (start, end) byte offsets relative to the line's first byte. ext_id and histogram are those of gorp_extract_text_utf8.
  * Runs on all of the engine's devices (contiguous line-aligned byte ranges, rows concatenated in device order). */
 int gorp_extract_text_utf8_bytes(gorp_engine* e, const uint8_t* text, int64_t n_bytes, gorp_result* out);
+/* Gorp.extractAll(List<String>) for strings held as UTF-8 bytes, e.g. an Arrow/Parquet string column (int64 offsets) or a
+ * batch of byte[] records: string i is bytes [off[i], off[i+1]) of `text`; a '\n' inside a string is data. Results are
+ * those of gorp_extract_lines on the UTF-16 of `new String(bytes_i, UTF_8)` for every string, in BYTE coordinates:
+ * line_off is a copy of `off` (sep = 0), spans are (start, end) byte offsets relative to the string's first byte;
+ * ext_id and histogram are unchanged. Every string must be well-formed UTF-8 on its own (Unicode table 3-7): otherwise
+ * GORP_E_ARG, "malformed UTF-8 at byte N", N = the lowest byte of `text` at which decoding some string on its own fails.
+ * Bytes outside [off[0], off[n_lines]) are never read. Runs on all of the engine's devices. */
+int gorp_extract_lines_utf8(gorp_engine* e, const uint8_t* text, const int64_t* off, int64_t n_lines, gorp_result* out);
 void gorp_result_release(gorp_engine* e, gorp_result* r);
 
 /* PolyMatcher.match for a batch (reference autom/PolyMatcher.java:123-133, reached through Gorp.getMatcher(), Gorp.java:135-137):

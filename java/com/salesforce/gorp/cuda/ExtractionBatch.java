@@ -22,7 +22,8 @@ public final class ExtractionBatch {
     /** extraction index per line: >= 0 matched, -1 miss (Gorp.extract returns null), <= -2: capture failure of extraction -2-e */
     public final int[] extId;
     /** UTF-16 unit offsets of the lines in the batch text ('\n'-separated forms: line i = [lineOff[i], lineOff[i+1] - 1)); byte
-     *  offsets in the caller's buffer for a byte-coordinate batch ({@link GorpCuda#extractBatchUtf8Bytes}), spans too */
+     *  offsets in the caller's buffer for a byte-coordinate batch ({@link GorpCuda#extractBatchUtf8Bytes}; for
+     *  {@link GorpCuda#extractBatchUtf8Lines} line i = [lineOff[i], lineOff[i+1]), no separator), spans too */
     public final long[] lineOff;
     /** spanStride ints per line: (start, end) of group 1..n relative to the line start, -1 = group did not participate */
     public final int[] spans;
@@ -34,6 +35,7 @@ public final class ExtractionBatch {
     private final int[] groups;
     private final LongFunction<String> lines;
     private final ByteSource bytes;
+    private final int sep;  // units between a line's end and the next line's start in a byte-coordinate batch ('\n': 1, strings: 0)
 
     /** Decodes bytes [from, to) of the caller's buffer (byte-coordinate batches). */
     interface ByteSource { String decode(long from, long to); }
@@ -45,6 +47,11 @@ public final class ExtractionBatch {
 
     ExtractionBatch(int[] extId, long[] lineOff, int[] spans, int spanStride, long[] histogram, CookedExtraction[] extractions,
                     int[] groups, LongFunction<String> lines, ByteSource bytes) {
+        this(extId, lineOff, spans, spanStride, histogram, extractions, groups, lines, bytes, 1);
+    }
+
+    ExtractionBatch(int[] extId, long[] lineOff, int[] spans, int spanStride, long[] histogram, CookedExtraction[] extractions,
+                    int[] groups, LongFunction<String> lines, ByteSource bytes, int sep) {
         this.extId = extId;
         this.lineOff = lineOff;
         this.spans = spans;
@@ -54,6 +61,7 @@ public final class ExtractionBatch {
         this.groups = groups;
         this.lines = lines;
         this.bytes = bytes;
+        this.sep = sep;
     }
 
     public int size() { return extId.length; }
@@ -66,7 +74,7 @@ public final class ExtractionBatch {
     public CookedExtraction extraction(int i) { return extId[i] >= 0 ? extractions[extId[i]] : null; }
 
     /** Text of line i (decoded lazily from the caller's buffer). */
-    public String line(int i) { return bytes != null ? bytes.decode(lineOff[i], lineOff[i + 1] - 1) : lines.apply(i); }
+    public String line(int i) { return bytes != null ? bytes.decode(lineOff[i], lineOff[i + 1] - sep) : lines.apply(i); }
 
     /** Text [a, b) of line i: a substring of the line, or in a byte-coordinate batch the decoded bytes [start + a, start + b). */
     private String cut(int i, String line, int a, int b) {

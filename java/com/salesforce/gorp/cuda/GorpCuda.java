@@ -58,6 +58,8 @@ public final class GorpCuda implements AutoCloseable {
             FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS));
     private static final MethodHandle EXTRACT_TEXT_UTF8_BYTES = fn("gorp_extract_text_utf8_bytes",
             FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS));
+    private static final MethodHandle EXTRACT_LINES_UTF8 = fn("gorp_extract_lines_utf8",
+            FunctionDescriptor.of(JAVA_INT, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS));
     // struct gorp_match_result { int64 n_lines; const int64* accept_off; const int32* accept; void* owner; }
     private static final StructLayout MATCH_RESULT = MemoryLayout.structLayout(
             JAVA_LONG.withName("n_lines"), ADDRESS.withName("accept_off"), ADDRESS.withName("accept"), ADDRESS.withName("owner"));
@@ -257,6 +259,47 @@ public final class GorpCuda implements AutoCloseable {
         }
     }
 
+    /**
+     * Columnar batch over records held as UTF-8 bytes (a batch of Kafka records, a {@code List<byte[]>} of events): what
+     * {@link #extractBatch(List)} gives on {@code new String(record, UTF_8)} for every record, in BYTE coordinates: lineOff
+     * are offsets into the records laid end to end (record i = [lineOff[i], lineOff[i+1])), spans byte offsets relative to
+     * the record's first byte. A '\n' inside a record is data. The records are copied to native memory as they are (no
+     * decoding, no String per record) and decoded on the device; lines and values are decoded later from the records
+     * themselves, which must not change while the batch is in use. Runs on all of the engine's devices. A record that is not
+     * well-formed UTF-8 fails the call.
+     */
+    public ExtractionBatch extractBatchUtf8Lines(List<byte[]> records) throws Throwable {
+        final int n = records.size();
+        final long[] start = new long[n + 1];
+        for (int i = 0; i < n; ++i) start[i + 1] = start[i] + records.get(i).length;
+        try (Arena a = Arena.ofConfined()) {
+            MemorySegment text = a.allocate(Math.max(start[n], 1), 16);
+            MemorySegment off = a.allocate(8L * (n + 1), 8);
+            for (int i = 0; i < n; ++i) {
+                byte[] r = records.get(i);
+                MemorySegment.copy(r, 0, text, java.lang.foreign.ValueLayout.JAVA_BYTE, start[i], r.length);
+            }
+            MemorySegment.copy(start, 0, off, JAVA_LONG, 0, n + 1);
+            MemorySegment res = a.allocate(RESULT);
+            check((int) EXTRACT_LINES_UTF8.invokeExact(engine, text, off, (long) n, res));
+            try {
+                // bytes [from, to) lie in one record: the first record that ends after `from` (the arena is gone by then)
+                return batch(res, n, null, (from, to) -> {
+                    if (to <= from) return "";
+                    int lo = 0, hi = n;
+                    while (lo < hi) {
+                        int mid = (lo + hi) >>> 1;
+                        if (start[mid + 1] <= from) lo = mid + 1;
+                        else hi = mid;
+                    }
+                    return new String(records.get(lo), (int) (from - start[lo]), (int) (to - from), java.nio.charset.StandardCharsets.UTF_8);
+                }, 0);
+            } finally {
+                RESULT_RELEASE.invokeExact(engine, res);
+            }
+        }
+    }
+
     /** Columnar batch over a List&lt;String&gt; (Gorp.extractAll without materialising every ExtractionResult). */
     public ExtractionBatch extractBatch(List<String> lines) throws Throwable {
         final int n = lines.size();
@@ -325,12 +368,17 @@ public final class GorpCuda implements AutoCloseable {
 
     /** With {@code bytes} (byte-coordinate results): lines and values are cut from the caller's buffer. */
     private ExtractionBatch batch(MemorySegment res, int n, java.util.function.LongFunction<String> lines, ExtractionBatch.ByteSource bytes) {
+        return batch(res, n, lines, bytes, 1);
+    }
+
+    /** {@code sep}: bytes between a line's end and the next line's start ('\n'-separated text: 1, records: 0). */
+    private ExtractionBatch batch(MemorySegment res, int n, java.util.function.LongFunction<String> lines, ExtractionBatch.ByteSource bytes, int sep) {
         final int stride = res.get(JAVA_INT, 12), nExt = res.get(JAVA_INT, 8);
         int[] extId = res.get(ADDRESS, 16).reinterpret(4L * Math.max(n, 1)).asSlice(0, 4L * n).toArray(JAVA_INT);
         long[] lineOff = res.get(ADDRESS, 24).reinterpret(8L * (n + 1)).toArray(JAVA_LONG);
         int[] spans = res.get(ADDRESS, 32).reinterpret(4L * Math.max((long) n * stride, 1)).asSlice(0, 4L * n * stride).toArray(JAVA_INT);
         long[] hist = res.get(ADDRESS, 40).reinterpret(8L * (nExt + 2)).toArray(JAVA_LONG);
-        return new ExtractionBatch(extId, lineOff, spans, stride, hist, extractions, groups, lines, bytes);
+        return new ExtractionBatch(extId, lineOff, spans, stride, hist, extractions, groups, lines, bytes, sep);
     }
 
     private interface LineSource { String line(long i); }
