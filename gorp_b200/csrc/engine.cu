@@ -806,8 +806,9 @@ int64_t run_pipeline_tables(DeviceCtx& c, const uint16_t* d_text, int64_t n_unit
     const uint32_t stride = c.max_slots;
     c.spans.reserve((nl * stride + 4) * 4);
     bool hist_done = false;
+    // K4b walks 32-byte blocks with 256-bit loads, like the walkers above: a text base that is only 16-byte aligned takes K4
     if (!c.cap.match_only && stride > 0 && (sep == 1 || with_tails) && c.capimg.enabled && !c.force_general && !c.force_k4 && n_lines > 0 &&
-        n_lines < (1ll << 32)) {
+        n_lines < (1ll << 32) && (reinterpret_cast<uintptr_t>(d_text) & 31) == 0) {
         // K4b: histogram -> buckets by extraction -> one warp per work item (kernels/capwalk.cu)
         const uint32_t E = c.n_ext;
         CK(cudaMemsetAsync(c.hist.p, 0, (E + 2) * 8, stream));

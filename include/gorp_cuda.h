@@ -154,7 +154,8 @@ int gorp_match_all_lines(gorp_engine* e, const uint16_t* text, const int64_t* of
 void gorp_match_result_release(gorp_engine* e, gorp_match_result* r);
 
 /* --- device-resident variants: `d_text` (and `d_off`) already live in the HBM of the engine's device `dev_index`
- * (index into the `devices` array given at creation) and must be 16-byte aligned; results stay in device memory
+ * (index into the `devices` array given at creation) and must be 16-byte aligned; only a 32-byte aligned `d_text` gets
+ * the walkers that read 32-byte blocks (256-bit loads), any other takes the 16-byte-load kernels. Results stay in device memory
  * owned by the engine until the next call on the same (engine, dev_index). `stream` is a cudaStream_t (NULL = the
  * CUDA default stream, as everywhere in CUDA). The call enqueues the kernels on that stream; the text form waits once for the newline
  * count (it sizes the per-line arrays). Used by bench.py for the HBM-resident `value`. */

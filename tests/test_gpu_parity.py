@@ -15,20 +15,30 @@ pytestmark = pytest.mark.gpu
 
 def check_against_oracle(definition, text=None, lines=None, gorp=None):
     g = gorp or DefinitionReader.reader(definition).read()
+    b = g.extract_batch_lines(lines) if lines is not None else g.extract_batch_text(text)
+    oe = assert_matches_oracle(definition, b, text=text, lines=lines)
+    return g, b, oe
+
+
+def assert_matches_oracle(definition, b, text=None, lines=None, expect=None, line_off0=0):
+    """Holds a batch result `b` (anything with n_lines, span_stride, ext_id, line_off, spans and histogram as numpy arrays)
+    to the oracle on the same input: '\\n'-separated UTF-16 `text`, or `lines` (str or uint16 arrays) for the List<String>
+    form, whose offsets start at `line_off0`. `expect` = the oracle's (ext_id, spans) when the caller has them already.
+    Returns the oracle's ext_id."""
     o = gorp_oracle.Gorp(definition)
     G = max(len(x.extractor_names) for x in o.extractions)
     if lines is not None:
-        b = g.extract_batch_lines(lines)
-        units = [np.asarray(jdkre.to_units(s), dtype=np.uint16) for s in lines]
+        units = [s.astype(np.uint16, copy=False) if isinstance(s, np.ndarray) else np.asarray(jdkre.to_units(s), dtype=np.uint16)
+                 for s in lines]
         off = np.zeros(len(lines) + 1, dtype=np.int64)
         np.cumsum([len(u) for u in units], out=off[1:])
         flat = np.concatenate(units) if units else np.zeros(0, np.uint16)
-        oe, osp = o.extract_batch(flat, off, threads=0)
-        assert (b.line_off == off).all()
+        oe, osp = expect or o.extract_batch(flat, off, threads=0)
+        assert b.n_lines == len(lines)
+        assert (b.line_off == off + line_off0).all(), np.flatnonzero(b.line_off != off + line_off0)[:10]
     else:
-        b = g.extract_batch_text(text)
         starts, ends = gorp_oracle.split_lines(text)
-        oe, osp = o.extract_batch(text, (starts, ends), threads=0)
+        oe, osp = expect or o.extract_batch(text, (starts, ends), threads=0)
         assert b.n_lines == len(starts)
         assert (b.line_off[:-1] == starts).all() and (b.line_off[1:] - 1 == ends).all()
     assert (b.ext_id == oe).all(), np.flatnonzero(b.ext_id != oe)[:10]
@@ -40,7 +50,7 @@ def check_against_oracle(definition, text=None, lines=None, gorp=None):
     hist = np.zeros(E + 2, dtype=np.int64)
     np.add.at(hist, np.where(oe >= 0, oe, np.where(oe == -1, E, E + 1)), 1)
     assert (b.histogram == hist).all()
-    return g, b, oe
+    return oe
 
 
 # ---------------------------------------------------------------- the reference's own vectors through the GPU
