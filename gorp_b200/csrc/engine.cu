@@ -120,7 +120,7 @@ T* upload(const std::vector<T>& v, std::vector<void*>& owned) {
     return static_cast<T*>(p);
 }
 
-constexpr int kMaxTimed = 12;
+constexpr int kMaxTimed = 16;
 struct DeviceCtx {
     int device = 0;
     int numa_node = -1;
@@ -637,18 +637,19 @@ struct Timer {
     }
 };
 
-// Runs the device pipeline. Text form when d_off == nullptr. Caller holds c.mu and has set the device.
+// Runs the device pipeline. Text form when d_off == nullptr. Caller holds c.mu and has set the device; `tm` times the
+// stages of the caller's call on `stream`.
 // Returns n_lines (synchronises once for the text form to size the per-line arrays).
 int64_t run_pipeline_tables(DeviceCtx& c, const uint16_t* d_text, int64_t n_units, const int64_t* d_off, int64_t n_lines,
-                            cudaStream_t stream, bool timed, gorp_device_result* out);
+                            cudaStream_t stream, Timer& tm, gorp_device_result* out);
 
 // The table-driven pipeline, then (only for definitions that have such extractions) the simulated Pike VM over the lines
 // that came out as CAPTURE_FAIL of an extraction without a determinised capture automaton.
 int64_t run_pipeline(DeviceCtx& c, const uint16_t* d_text, int64_t n_units, const int64_t* d_off, int64_t n_lines,
-                     cudaStream_t stream, bool timed, gorp_device_result* out) {
+                     cudaStream_t stream, Timer& tm, gorp_device_result* out) {
     gorp_device_result local{};
     gorp_device_result* r = out ? out : &local;
-    const int64_t nl = run_pipeline_tables(c, d_text, n_units, d_off, n_lines, stream, timed, r);
+    const int64_t nl = run_pipeline_tables(c, d_text, n_units, d_off, n_lines, stream, tm, r);
     if (c.pike.enabled && nl > 0 && !c.cap.match_only && c.max_slots > 0) {
         Launch L{stream, c.sm_count};
         const size_t per_thread = pike_scratch_ints_per_thread(c.pike) * 4;
@@ -667,9 +668,8 @@ int64_t run_pipeline(DeviceCtx& c, const uint16_t* d_text, int64_t n_units, cons
 }
 
 int64_t run_pipeline_tables(DeviceCtx& c, const uint16_t* d_text, int64_t n_units, const int64_t* d_off, int64_t n_lines,
-                            cudaStream_t stream, bool timed, gorp_device_result* out) {
+                            cudaStream_t stream, Timer& tm, gorp_device_result* out) {
     Launch L{stream, c.sm_count};
-    Timer tm(c, stream, timed);
     c.scalars.reserve(128);
     int64_t* d_n_lines = c.scalars.as<int64_t>();
     const int64_t* d_line_off;
@@ -932,6 +932,129 @@ int64_t run_pipeline_tables(DeviceCtx& c, const uint16_t* d_text, int64_t n_unit
     return n_lines;
 }
 
+// ------------------------------------------------------------------ UTF-8 input: the steps around run_pipeline
+// Shared by the host piece loop (run_pieces, on a staged piece) and the device-resident UTF-8 calls (on the caller's HBM).
+// `bytes` is 16-byte aligned; the caller holds c.mu and has set the device.
+
+// Text form, before the pipeline: UTF-16 units per tile + validation, scan, one host round trip ({decoded total, first
+// malformed byte}, and the last byte when `last` is given), decode to `dst`. Returns the decoded total. `at` is the position
+// of `bytes` in the caller's buffer (the error names a byte of the caller's buffer).
+int64_t utf8_text_decode(DeviceCtx& c, const Launch& L, Timer& tm, const uint8_t* bytes, int64_t n, int64_t at, uint16_t* dst, uint8_t* last) {
+    const int64_t tiles = utf8_tiles(n);
+    c.tile_counts.reserve(static_cast<size_t>(tiles + 1) * 4);
+    c.tile_base.reserve(static_cast<size_t>(tiles + 2) * 8);
+    c.scan_scratch.reserve(static_cast<size_t>(tiles / 4096 + 8) * 8);
+    c.scalars.reserve(128);
+    unsigned long long* d_bad = reinterpret_cast<unsigned long long*>(c.scalars.as<int64_t>() + 6);
+    unsigned long long bad = ~0ull;
+    int64_t total = 0;
+    CK(cudaMemsetAsync(d_bad, 0xFF, 8, L.stream));
+    k_utf8_count(L, bytes, n, c.tile_counts.as<uint32_t>(), d_bad);
+    scan_u32_to_i64(L, c.tile_counts.as<uint32_t>(), tiles, c.tile_base.as<int64_t>(), c.scan_scratch.as<int64_t>());
+    tm.mark("utf8_count", 4);
+    if (n > 0) CK(cudaMemcpyAsync(&total, c.tile_base.as<int64_t>() + tiles, 8, cudaMemcpyDeviceToHost, L.stream));
+    CK(cudaMemcpyAsync(&bad, d_bad, 8, cudaMemcpyDeviceToHost, L.stream));
+    if (last && n > 0) CK(cudaMemcpyAsync(last, bytes + n - 1, 1, cudaMemcpyDeviceToHost, L.stream));
+    CK(cudaStreamSynchronize(L.stream));
+    if (bad != ~0ull)
+        throw ArgError(strfmt("malformed UTF-8 at byte %lld (the input must be well-formed UTF-8)", static_cast<long long>(at + static_cast<int64_t>(bad))));
+    k_utf8_write(L, bytes, n, c.tile_base.as<int64_t>(), dst);
+    tm.mark("utf8_decode", 1);
+    return total;
+}
+
+// Text form, after the pipeline: the byte '\n' index of `bytes` (built here because run_pipeline reuses tile_counts,
+// tile_base, scan_scratch and nl_masks; line k of the bytes is line k of the decoded text: the same '\n' characters), then
+// the rows `dr` moved from unit to byte offsets: out_off = byte line offsets + bias, out_spans = byte spans.
+void utf8_text_rows(DeviceCtx& c, const Launch& L, Timer& tm, const uint8_t* bytes, int64_t n, bool ends_with_nl, const gorp_device_result& dr,
+                    int64_t bias, uint32_t stride, int64_t* out_off, int32_t* out_spans) {
+    const int64_t n_tiles = (n + kNlTile - 1) / kNlTile;
+    c.tile_counts.reserve(static_cast<size_t>(n_tiles + 1) * 4);
+    c.tile_base.reserve(static_cast<size_t>(n_tiles + 2) * 8);
+    c.scan_scratch.reserve(static_cast<size_t>(n_tiles / 4096 + 8) * 8);
+    c.nl_masks.reserve(static_cast<size_t>(n_tiles + 4) * 256 * 4);
+    c.byte_off.reserve(static_cast<size_t>(dr.n_lines + 2) * 8);
+    k_utf8_count_newlines_masks(L, bytes, n, c.tile_counts.as<uint32_t>(), c.nl_masks.as<uint32_t>());
+    scan_u32_to_i64(L, c.tile_counts.as<uint32_t>(), n_tiles, c.tile_base.as<int64_t>(), c.scan_scratch.as<int64_t>());
+    k1_scatter_masks(L, c.nl_masks.as<uint32_t>(), n, c.tile_base.as<int64_t>(), c.byte_off.as<int64_t>());
+    tm.mark("utf8_nl_index", n > 0 ? 5 : 2);
+    if (stride > 64) throw std::logic_error("result rows wider than 64 entries");  // (31 groups at most: 62)
+    Utf8RowsParams P{};
+    P.bytes = bytes;
+    P.unit_off = dr.d_line_off;
+    P.byte_off = c.byte_off.as<int64_t>();
+    P.spans = dr.d_spans;
+    P.n_lines = dr.n_lines;
+    P.end_off = n + (ends_with_nl ? 0 : 1);
+    P.bias = bias;
+    P.stride = stride;
+    P.out_off = out_off;
+    P.out_spans = out_spans;
+    k_utf8_rows(L, P);
+    tm.mark("utf8_rows", 1);
+}
+
+// Lines form, before the pipeline: `bytes` holds bytes [at, at + n) of the caller's buffer, `d_off` the caller's n_lines + 1
+// offsets (device memory). UTF-16 units per tile + slice prefixes + validation, scan, the strings' unit offsets (c.unit_off,
+// relative to the piece) with the boundary check and, with `check_order`, the offset-order check; one host round trip;
+// decode to `dst`. Returns the decoded total.
+int64_t utf8_lines_decode(DeviceCtx& c, const Launch& L, Timer& tm, const uint8_t* bytes, int64_t n, int64_t at, const int64_t* d_off, int64_t n_lines,
+                          uint16_t* dst, bool check_order) {
+    const int64_t tiles = utf8_tiles(n);
+    c.tile_counts.reserve(static_cast<size_t>(tiles + 1) * 4);
+    c.tile_base.reserve(static_cast<size_t>(tiles + 2) * 8);
+    c.scan_scratch.reserve(static_cast<size_t>(tiles / 4096 + 8) * 8);
+    c.scalars.reserve(128);
+    unsigned long long* d_bad = reinterpret_cast<unsigned long long*>(c.scalars.as<int64_t>() + 6);
+    unsigned long long* d_order = check_order ? d_bad + 1 : nullptr;
+    unsigned long long bad = ~0ull, order = ~0ull;
+    int64_t total = 0;
+    CK(cudaMemsetAsync(d_bad, 0xFF, check_order ? 16 : 8, L.stream));
+    k_utf8_count(L, bytes, n, c.tile_counts.as<uint32_t>(), d_bad, c.slice_units.as<uint16_t>());
+    scan_u32_to_i64(L, c.tile_counts.as<uint32_t>(), tiles, c.tile_base.as<int64_t>(), c.scan_scratch.as<int64_t>());
+    tm.mark("utf8_count", 4);
+    k_utf8_line_units(L, bytes, n, d_off, n_lines + 1, at, c.tile_base.as<int64_t>(), c.slice_units.as<uint16_t>(), c.unit_off.as<int64_t>(), d_bad,
+                      d_order);
+    tm.mark("utf8_line_units", 1);
+    if (n > 0) CK(cudaMemcpyAsync(&total, c.tile_base.as<int64_t>() + tiles, 8, cudaMemcpyDeviceToHost, L.stream));
+    CK(cudaMemcpyAsync(&bad, d_bad, 8, cudaMemcpyDeviceToHost, L.stream));
+    if (check_order) CK(cudaMemcpyAsync(&order, d_order, 8, cudaMemcpyDeviceToHost, L.stream));
+    CK(cudaStreamSynchronize(L.stream));
+    if (order != ~0ull) throw ArgError(strfmt("offsets must be non-decreasing (line %lld)", static_cast<long long>(order)));
+    if (bad != ~0ull)
+        throw ArgError(strfmt("malformed UTF-8 at byte %lld (every string must be well-formed UTF-8)", static_cast<long long>(at + static_cast<int64_t>(bad))));
+    k_utf8_write(L, bytes, n, c.tile_base.as<int64_t>(), dst);
+    tm.mark("utf8_decode", 1);
+    return total;
+}
+
+// Lines form, after the pipeline: the rows `dr` moved back to the caller's byte offsets (out_off = a copy of d_off, or
+// nullptr when the call returns d_off itself).
+void utf8_lines_rows(const Launch& L, Timer& tm, const uint8_t* bytes, int64_t at, const int64_t* d_off, const gorp_device_result& dr, uint32_t stride,
+                     int64_t* out_off, int32_t* out_spans) {
+    if (stride > 64) throw std::logic_error("result rows wider than 64 entries");  // (31 groups at most: 62)
+    Utf8RowsParams P{};
+    P.bytes = bytes;
+    P.unit_off = dr.d_line_off;
+    P.byte_off = d_off;
+    P.spans = dr.d_spans;
+    P.n_lines = dr.n_lines;
+    P.bias = at;
+    P.stride = stride;
+    P.out_off = out_off;
+    P.out_spans = out_spans;
+    k_utf8_rows(L, P, true);
+    tm.mark("utf8_rows", 1);
+}
+
+// The UTF-8 device-resident calls write their rows in byte coordinates to acc_spans (and the text form its byte line
+// offsets to acc_off): the accumulators of the host-buffer calls, idle outside those calls. utf8_rows_kernel reads the
+// pipeline's unit rows while it writes, so it cannot write them in place.
+void reserve_byte_rows(DeviceCtx& c, int64_t n_lines, uint32_t stride, bool offsets) {
+    if (offsets) c.acc_off.reserve(static_cast<size_t>(n_lines + 2) * 8);
+    c.acc_spans.reserve((static_cast<size_t>(n_lines) * stride + 4) * 4);
+}
+
 // ------------------------------------------------------------------ host-buffer calls: pieces, pipelining, devices
 constexpr int64_t kPieceUnits = 32ll << 20;  // 64 MB of text per piece
 constexpr int kTextPad = 32;                 // units in front of a staged piece (aligned chunk reads of the lines form)
@@ -987,8 +1110,12 @@ struct DeviceRun {  // what one device produced for its pieces
 void run_pieces(gorp_engine* e, DeviceCtx& c, const uint16_t* text, const uint8_t* text8, bool utf8, bool byte_coords, const int64_t* off,
                 const std::vector<Piece>& pieces, size_t p0, size_t p1, HostResult* hr, DeviceRun& run) {
     CK(cudaSetDevice(c.device));
-    CK(cudaStreamWaitEvent(c.stream, c.ev_done, 0));  // a device-resident call on another stream may still use the scratch
+    // a device-resident call on another stream may still use the scratch: the kernels wait for it, and so do the staging
+    // copies (the UTF-8 device calls decode into textbuf[0] and stage into bytebuf[0], which the first piece's copy overwrites)
+    CK(cudaStreamWaitEvent(c.stream, c.ev_done, 0));
+    CK(cudaStreamWaitEvent(c.s_in, c.ev_done, 0));
     Launch L{c.stream, c.sm_count};
+    Timer tm(c, c.stream, false);  // (untimed: counts the launches)
     const size_t E2 = e->def.extractions.size() + 2;
     const uint32_t stride = e->match_only ? 0u : c.max_slots;
     int64_t units_total = 0, lines_total = 0;
@@ -1055,63 +1182,25 @@ void run_pieces(gorp_engine* e, DeviceCtx& c, const uint16_t* text, const uint8_
         gorp_device_result dr{};
         int64_t nl;
         if (off && utf8) {
-            // UTF-8 strings: count + validate, scan, unit offsets of the strings + boundary validation, (one host round trip:
-            // total + first malformed byte), decode; then the lines form over the decoded piece
-            const int64_t tiles = utf8_tiles(units), n_lines_piece = pc.l1 - pc.l0;
-            c.tile_counts.reserve(static_cast<size_t>(tiles + 1) * 4);
-            c.tile_base.reserve(static_cast<size_t>(tiles + 2) * 8);
-            c.scan_scratch.reserve(static_cast<size_t>(tiles / 4096 + 8) * 8);
-            c.scalars.reserve(128);
-            unsigned long long* d_bad = reinterpret_cast<unsigned long long*>(c.scalars.as<int64_t>() + 6);
-            unsigned long long bad = ~0ull;
-            int64_t total = 0;
-            CK(cudaMemsetAsync(d_bad, 0xFF, 8, c.stream));
-            k_utf8_count(L, c.bytebuf[b].as<uint8_t>(), units, c.tile_counts.as<uint32_t>(), d_bad, c.slice_units.as<uint16_t>());
-            scan_u32_to_i64(L, c.tile_counts.as<uint32_t>(), tiles, c.tile_base.as<int64_t>(), c.scan_scratch.as<int64_t>());
-            k_utf8_line_units(L, c.bytebuf[b].as<uint8_t>(), units, c.offbuf[b].as<int64_t>(), n_lines_piece + 1, pc.u0, c.tile_base.as<int64_t>(),
-                              c.slice_units.as<uint16_t>(), c.unit_off.as<int64_t>(), d_bad);
-            if (units > 0) CK(cudaMemcpyAsync(&total, c.tile_base.as<int64_t>() + tiles, 8, cudaMemcpyDeviceToHost, c.stream));
-            CK(cudaMemcpyAsync(&bad, d_bad, 8, cudaMemcpyDeviceToHost, c.stream));
-            CK(cudaStreamSynchronize(c.stream));
-            if (bad != ~0ull)
-                throw ArgError(strfmt("malformed UTF-8 at byte %lld (every string must be well-formed UTF-8)",
-                                      static_cast<long long>(pc.u0 + static_cast<int64_t>(bad))));
+            // UTF-8 strings (the host checked the offsets): decoded behind the lines-form padding, then the lines form over
+            // the decoded piece
+            const int64_t n_lines_piece = pc.l1 - pc.l0;
             uint16_t* piece_text = c.textbuf[b].as<uint16_t>() + kTextPad;  // (device address - unit index) a multiple of 32 bytes
-            k_utf8_write(L, c.bytebuf[b].as<uint8_t>(), units, c.tile_base.as<int64_t>(), piece_text);
-            c.launches += 6;
-            nl = run_pipeline(c, piece_text, total, c.unit_off.as<int64_t>(), n_lines_piece, c.stream, false, &dr);
+            const int64_t total = utf8_lines_decode(c, L, tm, c.bytebuf[b].as<uint8_t>(), units, pc.u0, c.offbuf[b].as<int64_t>(), n_lines_piece,
+                                                    piece_text, false);
+            nl = run_pipeline(c, piece_text, total, c.unit_off.as<int64_t>(), n_lines_piece, c.stream, tm, &dr);
         } else if (off) {
             const uint16_t* vbase = c.textbuf[b].as<uint16_t>() + kTextPad + (pc.u0 & 15) - pc.u0;  // text[i] lives at vbase + i
-            nl = run_pipeline(c, vbase, pc.u1, c.offbuf[b].as<int64_t>(), pc.l1 - pc.l0, c.stream, false, &dr);  // text[i] valid for i < u1
+            nl = run_pipeline(c, vbase, pc.u1, c.offbuf[b].as<int64_t>(), pc.l1 - pc.l0, c.stream, tm, &dr);  // text[i] valid for i < u1
         } else {
             int64_t n_units_piece = units;
             if (text8 && utf8) {
-                // bytes -> UTF-16 on the device: units per tile, scan, (one host round trip: total + first malformed byte), decode
-                const int64_t tiles = utf8_tiles(units);
-                c.tile_counts.reserve(static_cast<size_t>(tiles + 1) * 4);
-                c.tile_base.reserve(static_cast<size_t>(tiles + 2) * 8);
-                c.scan_scratch.reserve(static_cast<size_t>(tiles / 4096 + 8) * 8);
-                c.scalars.reserve(64);
-                unsigned long long* d_bad = reinterpret_cast<unsigned long long*>(c.scalars.as<int64_t>() + 6);
-                unsigned long long bad = ~0ull;
-                int64_t total = 0;
-                CK(cudaMemsetAsync(d_bad, 0xFF, 8, c.stream));
-                k_utf8_count(L, c.bytebuf[b].as<uint8_t>(), units, c.tile_counts.as<uint32_t>(), d_bad);
-                scan_u32_to_i64(L, c.tile_counts.as<uint32_t>(), tiles, c.tile_base.as<int64_t>(), c.scan_scratch.as<int64_t>());
-                if (units > 0) CK(cudaMemcpyAsync(&total, c.tile_base.as<int64_t>() + tiles, 8, cudaMemcpyDeviceToHost, c.stream));
-                CK(cudaMemcpyAsync(&bad, d_bad, 8, cudaMemcpyDeviceToHost, c.stream));
-                CK(cudaStreamSynchronize(c.stream));
-                if (bad != ~0ull)
-                    throw ArgError(strfmt("malformed UTF-8 at byte %lld (the input must be well-formed UTF-8)",
-                                          static_cast<long long>(pc.u0 + static_cast<int64_t>(bad))));
-                k_utf8_write(L, c.bytebuf[b].as<uint8_t>(), units, c.tile_base.as<int64_t>(), c.textbuf[b].as<uint16_t>());
-                c.launches += 5;
-                n_units_piece = total;
+                n_units_piece = utf8_text_decode(c, L, tm, c.bytebuf[b].as<uint8_t>(), units, pc.u0, c.textbuf[b].as<uint16_t>(), nullptr);
             } else if (text8) {
                 k_widen_latin1(L, c.bytebuf[b].as<uint8_t>(), c.textbuf[b].as<uint16_t>(), units);
                 c.launches += 1;
             }
-            nl = run_pipeline(c, c.textbuf[b].as<uint16_t>(), n_units_piece, nullptr, 0, c.stream, false, &dr);
+            nl = run_pipeline(c, c.textbuf[b].as<uint16_t>(), n_units_piece, nullptr, 0, c.stream, tm, &dr);
             if (utf8 && !byte_coords) {
                 piece_bias = utf8_base;
                 utf8_base += n_units_piece;
@@ -1127,46 +1216,11 @@ void run_pieces(gorp_engine* e, DeviceCtx& c, const uint16_t* text, const uint8_
         if (nl) CK(cudaMemcpyAsync(c.acc_ext.as<int32_t>() + rows, dr.d_ext_id, static_cast<size_t>(nl) * 4, cudaMemcpyDeviceToDevice, c.stream));
         if (off && utf8) {
             // rows back to the caller's byte offsets (line_off is a copy of the caller's offsets)
-            if (stride > 64) throw std::logic_error("result rows wider than 64 entries");  // (31 groups at most: 62)
-            Utf8RowsParams P{};
-            P.bytes = c.bytebuf[b].as<uint8_t>();
-            P.unit_off = dr.d_line_off;
-            P.byte_off = c.offbuf[b].as<int64_t>();
-            P.spans = dr.d_spans;
-            P.n_lines = nl;
-            P.bias = pc.u0;
-            P.stride = stride;
-            P.out_off = c.acc_off.as<int64_t>() + rows;
-            P.out_spans = c.acc_spans.as<int32_t>() + static_cast<size_t>(rows) * stride;
-            k_utf8_rows(L, P, true);
-            c.launches += 1;
+            utf8_lines_rows(L, tm, c.bytebuf[b].as<uint8_t>(), pc.u0, c.offbuf[b].as<int64_t>(), dr, stride, c.acc_off.as<int64_t>() + rows,
+                            c.acc_spans.as<int32_t>() + static_cast<size_t>(rows) * stride);
         } else if (utf8 && byte_coords) {
-            // byte '\n' index of the piece, built after run_pipeline (which reuses tile_counts, tile_base, scan_scratch and
-            // nl_masks); line k of the bytes is line k of the decoded text (same '\n' characters). Then the gather converts
-            // the rows from the piece's unit offsets to byte offsets.
-            const int64_t n_tiles = (units + kNlTile - 1) / kNlTile;
-            c.tile_counts.reserve(static_cast<size_t>(n_tiles + 1) * 4);
-            c.tile_base.reserve(static_cast<size_t>(n_tiles + 2) * 8);
-            c.scan_scratch.reserve(static_cast<size_t>(n_tiles / 4096 + 8) * 8);
-            c.nl_masks.reserve(static_cast<size_t>(n_tiles + 4) * 256 * 4);
-            c.byte_off.reserve(static_cast<size_t>(nl + 2) * 8);
-            k_utf8_count_newlines_masks(L, c.bytebuf[b].as<uint8_t>(), units, c.tile_counts.as<uint32_t>(), c.nl_masks.as<uint32_t>());
-            scan_u32_to_i64(L, c.tile_counts.as<uint32_t>(), n_tiles, c.tile_base.as<int64_t>(), c.scan_scratch.as<int64_t>());
-            k1_scatter_masks(L, c.nl_masks.as<uint32_t>(), units, c.tile_base.as<int64_t>(), c.byte_off.as<int64_t>());
-            if (stride > 64) throw std::logic_error("result rows wider than 64 entries");  // (31 groups at most: 62)
-            Utf8RowsParams P{};
-            P.bytes = c.bytebuf[b].as<uint8_t>();
-            P.unit_off = dr.d_line_off;
-            P.byte_off = c.byte_off.as<int64_t>();
-            P.spans = dr.d_spans;
-            P.n_lines = nl;
-            P.end_off = units + (units > 0 && text8[pc.u1 - 1] != 0x0A ? 1 : 0);
-            P.bias = piece_bias;
-            P.stride = stride;
-            P.out_off = c.acc_off.as<int64_t>() + rows;
-            P.out_spans = c.acc_spans.as<int32_t>() + static_cast<size_t>(rows) * stride;
-            k_utf8_rows(L, P);
-            c.launches += units > 0 ? 6 : 3;
+            utf8_text_rows(c, L, tm, c.bytebuf[b].as<uint8_t>(), units, units == 0 || text8[pc.u1 - 1] == 0x0A, dr, piece_bias, stride,
+                           c.acc_off.as<int64_t>() + rows, c.acc_spans.as<int32_t>() + static_cast<size_t>(rows) * stride);
         } else {
             k_bias_copy(L, c.acc_off.as<int64_t>() + rows, dr.d_line_off, nl + 1, off ? 0 : piece_bias);
             if (nl && stride)
@@ -1683,7 +1737,8 @@ int gorp_extract_text_device(gorp_engine* e, int dev_index, const uint16_t* d_te
         CK(cudaSetDevice(c.device));
         cudaStream_t st = static_cast<cudaStream_t>(stream);
         CK(cudaStreamWaitEvent(st, c.ev_done, 0));  // the previous call on this context (any stream) used the same scratch
-        run_pipeline(c, d_text, n_units, nullptr, 0, st, (flags & GORP_FLAG_TIME_KERNELS) != 0, out);
+        Timer tm(c, st, (flags & GORP_FLAG_TIME_KERNELS) != 0);
+        run_pipeline(c, d_text, n_units, nullptr, 0, st, tm, out);
         CK(cudaEventRecord(c.ev_done, st));
         if (flags & GORP_FLAG_SYNC) CK(cudaStreamSynchronize(st));
         return GORP_OK;
@@ -1707,7 +1762,90 @@ int gorp_extract_lines_device(gorp_engine* e, int dev_index, const uint16_t* d_t
             CK(cudaMemcpyAsync(&n_units, d_off + n_lines, 8, cudaMemcpyDeviceToHost, st));
             CK(cudaStreamSynchronize(st));
         }
-        run_pipeline(c, d_text, n_units, d_off, n_lines, st, (flags & GORP_FLAG_TIME_KERNELS) != 0, out);
+        Timer tm(c, st, (flags & GORP_FLAG_TIME_KERNELS) != 0);
+        run_pipeline(c, d_text, n_units, d_off, n_lines, st, tm, out);
+        CK(cudaEventRecord(c.ev_done, st));
+        if (flags & GORP_FLAG_SYNC) CK(cudaStreamSynchronize(st));
+        return GORP_OK;
+    });
+}
+
+int gorp_extract_text_utf8_device(gorp_engine* e, int dev_index, const uint8_t* d_text, int64_t n_bytes, void* stream, int flags,
+                                  gorp_device_result* out) {
+    if (!e || dev_index < 0 || dev_index >= static_cast<int>(e->devs.size()) || n_bytes < 0 || (reinterpret_cast<uintptr_t>(d_text) & 15))
+        return fail(GORP_E_ARG, "bad argument (d_text must be 16-byte aligned)");
+    return guarded([&]() -> int {
+        DeviceCtx& c = *e->devs[dev_index];
+        std::lock_guard<std::mutex> lock(c.mu);
+        DeviceGuard restore_device;
+        CK(cudaSetDevice(c.device));
+        cudaStream_t st = static_cast<cudaStream_t>(stream);
+        CK(cudaStreamWaitEvent(st, c.ev_done, 0));  // the previous call on this context (any stream) used the same scratch
+        Launch L{st, c.sm_count};
+        Timer tm(c, st, (flags & GORP_FLAG_TIME_KERNELS) != 0);
+        // round trip 1: {decoded total, first malformed byte, last byte}; round trip 2: the newline count (run_pipeline)
+        c.textbuf[0].reserve(static_cast<size_t>(n_bytes + 64) * 2);
+        uint16_t* text = c.textbuf[0].as<uint16_t>();
+        uint8_t last = 0x0A;
+        const int64_t n_units = utf8_text_decode(c, L, tm, d_text, n_bytes, 0, text, &last);
+        gorp_device_result dr{};
+        run_pipeline(c, text, n_units, nullptr, 0, st, tm, &dr);
+        const uint32_t stride = static_cast<uint32_t>(dr.span_stride);
+        reserve_byte_rows(c, dr.n_lines, stride, true);
+        utf8_text_rows(c, L, tm, d_text, n_bytes, last == 0x0A, dr, 0, stride, c.acc_off.as<int64_t>(), c.acc_spans.as<int32_t>());
+        CK(cudaGetLastError());
+        dr.d_line_off = c.acc_off.as<int64_t>();
+        dr.d_spans = c.acc_spans.as<int32_t>();
+        if (out) *out = dr;
+        CK(cudaEventRecord(c.ev_done, st));
+        if (flags & GORP_FLAG_SYNC) CK(cudaStreamSynchronize(st));
+        return GORP_OK;
+    });
+}
+
+int gorp_extract_lines_utf8_device(gorp_engine* e, int dev_index, const uint8_t* d_text, const int64_t* d_off, int64_t n_lines, void* stream,
+                                   int flags, gorp_device_result* out) {
+    if (!e || dev_index < 0 || dev_index >= static_cast<int>(e->devs.size()) || !d_off || n_lines < 0 ||
+        (reinterpret_cast<uintptr_t>(d_text) & 15))
+        return fail(GORP_E_ARG, "bad argument (d_text must be 16-byte aligned)");
+    return guarded([&]() -> int {
+        DeviceCtx& c = *e->devs[dev_index];
+        std::lock_guard<std::mutex> lock(c.mu);
+        DeviceGuard restore_device;
+        CK(cudaSetDevice(c.device));
+        cudaStream_t st = static_cast<cudaStream_t>(stream);
+        CK(cudaStreamWaitEvent(st, c.ev_done, 0));  // the previous call on this context (any stream) used the same scratch
+        Launch L{st, c.sm_count};
+        Timer tm(c, st, (flags & GORP_FLAG_TIME_KERNELS) != 0);
+        // round trip 1: d_off[0] and d_off[n_lines] size the copy and the decode buffer
+        int64_t ends[2] = {0, 0};
+        CK(cudaMemcpyAsync(&ends[0], d_off, 8, cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(&ends[1], d_off + n_lines, 8, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        if (ends[0] < 0) throw ArgError("offsets must start at >= 0");
+        // (d_off[n] < d_off[0]: some offset decreases, which the order check of utf8_lines_decode reports; nothing is read)
+        const int64_t at = ends[0], n_bytes = std::max<int64_t>(ends[1] - at, 0);
+        // the strings' bytes are copied to the 16-byte aligned staging buffer, so every kernel sees the layout of a staged
+        // host piece whatever the alignment of d_off[0], and no byte outside [d_off[0], d_off[n]) is read
+        c.bytebuf[0].reserve(static_cast<size_t>(n_bytes) + 64);
+        c.textbuf[0].reserve(static_cast<size_t>(n_bytes + kTextPad + 64) * 2);
+        c.unit_off.reserve(static_cast<size_t>(n_lines + 1) * 8);
+        c.slice_units.reserve(static_cast<size_t>(n_bytes / 16 + 1) * 2);
+        const uint8_t* bytes = c.bytebuf[0].as<uint8_t>();
+        if (n_bytes) CK(cudaMemcpyAsync(c.bytebuf[0].p, d_text + at, static_cast<size_t>(n_bytes), cudaMemcpyDeviceToDevice, st));
+        tm.mark("utf8_copy", 0);
+        // round trip 2: {decoded total, first malformed byte, first decreasing offset}
+        uint16_t* text = c.textbuf[0].as<uint16_t>() + kTextPad;  // (device address - unit index) a multiple of 32 bytes
+        const int64_t n_units = utf8_lines_decode(c, L, tm, bytes, n_bytes, at, d_off, n_lines, text, true);
+        gorp_device_result dr{};
+        run_pipeline(c, text, n_units, c.unit_off.as<int64_t>(), n_lines, st, tm, &dr);
+        const uint32_t stride = static_cast<uint32_t>(dr.span_stride);
+        reserve_byte_rows(c, n_lines, stride, false);
+        utf8_lines_rows(L, tm, bytes, at, d_off, dr, stride, nullptr, c.acc_spans.as<int32_t>());  // (d_line_off is d_off itself)
+        CK(cudaGetLastError());
+        dr.d_line_off = d_off;
+        dr.d_spans = c.acc_spans.as<int32_t>();
+        if (out) *out = dr;
         CK(cudaEventRecord(c.ev_done, st));
         if (flags & GORP_FLAG_SYNC) CK(cudaStreamSynchronize(st));
         return GORP_OK;

@@ -305,7 +305,7 @@ void k_utf8_count_newlines_masks(const Launch&, const uint8_t* src, int64_t n, u
 // Gather of one piece's rows in byte coordinates (utf8_rows_kernel): out_off[i] = byte start of line i + bias (i <= n_lines,
 // out_off[n_lines] = end_off + bias), out_spans = the unit rows with every boundary moved to the byte offset of its sequence.
 struct Utf8RowsParams {
-    const uint8_t* bytes;        // the piece's UTF-8 bytes (16-byte aligned, readable up to the next 32-byte boundary)
+    const uint8_t* bytes;        // the piece's UTF-8 bytes (16-byte aligned; read up to the 16-byte block of the last line's end)
     const int64_t* unit_off;     // [n_lines + 1] line offsets of the decoded piece (K1)
     const int64_t* byte_off;     // entries 1 .. of the byte line offsets (entry 0 is 0, entry n_lines is end_off)
     const int32_t* spans;        // [n_lines * stride] rows in unit offsets
@@ -317,13 +317,16 @@ struct Utf8RowsParams {
     int32_t* out_spans;
 };
 // lines = true: the List<String> form over UTF-8 strings (gorp_extract_lines_utf8): no separator, byte_off is the caller's
-// offsets [n_lines + 1] (the piece's bytes start at caller byte `bias`), out_off their copy; end_off is not used.
+// offsets [n_lines + 1] (the piece's bytes start at caller byte `bias`), out_off their copy (nullptr: not written); end_off
+// is not used.
 void k_utf8_rows(const Launch&, const Utf8RowsParams&, bool lines = false);
 // Unit offsets of the strings of a UTF-8 piece (utf8_line_units_kernel): unit_off[i] = UTF-16 units of the decoded piece
 // before byte byte_off[i] - base, from the count pass's tile_base (scanned) and slice_units; an interior offset that cuts a
 // sequence or starts with a continuation byte sets first_bad (atomicMin) to the byte at which a string fails on its own.
+// order_bad (or nullptr): set (atomicMin, preset to ~0) to the first i with byte_off[i + 1] < byte_off[i]; offsets outside
+// [base, base + n] are not dereferenced.
 void k_utf8_line_units(const Launch&, const uint8_t* src, int64_t n, const int64_t* byte_off, int64_t n_off, int64_t base, const int64_t* tile_base,
-                       const uint16_t* slice_units, int64_t* unit_off, unsigned long long* first_bad);
+                       const uint16_t* slice_units, int64_t* unit_off, unsigned long long* first_bad, unsigned long long* order_bad = nullptr);
 
 // matchAll (kernels/matchall.cu): the reference's own tables on the device
 struct MatchAllDev {

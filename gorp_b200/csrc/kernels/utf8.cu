@@ -143,17 +143,22 @@ __global__ void __launch_bounds__(kUtf8Threads) utf8_count_kernel(const uint8_t*
 // (the concatenation is well-formed, the strings are not). For an interior offset b whose byte is a continuation byte, the
 // string before b fails at the lead p of the cut sequence (p in [b - 3, b), the sequence reaching past b); with no such lead,
 // the string that starts at b fails at b. The lowest offending byte goes to first_bad (atomicMin, as the count pass).
+// order_bad (offsets that come from device memory, gorp_extract_lines_utf8_device; nullptr when the host checked them): the
+// lowest i with byte_off[i + 1] < byte_off[i] (atomicMin), the index the host check reports. An offset outside
+// [base, base + n] is never dereferenced (its unit offset is left 0); such an offset implies a decreasing pair, so the
+// call fails on order_bad before anything reads unit_off.
 __global__ void __launch_bounds__(kUtf8Threads) utf8_line_units_kernel(const uint8_t* __restrict__ src, int64_t n, const int64_t* __restrict__ byte_off,
                                                                       int64_t n_off, int64_t base, const int64_t* __restrict__ tile_base,
                                                                       const uint16_t* __restrict__ slice_units, int64_t* __restrict__ unit_off,
-                                                                      unsigned long long* __restrict__ first_bad) {
+                                                                      unsigned long long* __restrict__ first_bad, unsigned long long* __restrict__ order_bad) {
     const int64_t n_tiles = (n + kUtf8Tile - 1) / kUtf8Tile;
     for (int64_t i = static_cast<int64_t>(blockIdx.x) * kUtf8Threads + threadIdx.x; i < n_off; i += static_cast<int64_t>(gridDim.x) * kUtf8Threads) {
-        const int64_t b = byte_off[i] - base;
+        const int64_t o = byte_off[i], b = o - base;
+        if (order_bad && i + 1 < n_off && byte_off[i + 1] < o) atomicMin(order_bad, static_cast<unsigned long long>(i));
         int64_t u;
-        if (b <= 0 || n <= 0) {  // (an empty piece: its offsets all equal the piece start, nothing was scanned)
+        if (b <= 0 || b > n) {  // the piece start (an empty piece too: nothing was scanned), or not an offset of the piece
             u = 0;
-        } else if (b >= n) {
+        } else if (b == n) {
             u = tile_base[n_tiles];
         } else {
             const uint4 v = __ldg(reinterpret_cast<const uint4*>(src + (b & ~int64_t(15))));
@@ -276,7 +281,7 @@ __global__ void __launch_bounds__(kUtf8Threads) utf8_nl_count_mask_kernel(const 
 // A boundary never falls inside a surrogate pair of text decoded from well-formed UTF-8 (no lone surrogates; capture
 // automata consume whole pairs), so every boundary lands on a sequence start.
 // kLines (gorp_extract_lines_utf8): no separator; byte_off is the caller's offsets [n_lines + 1] (the piece starts at byte
-// `bias` of the caller's buffer), and out_off is a copy of them.
+// `bias` of the caller's buffer), and out_off is a copy of them, or nullptr when the caller returns its own offsets.
 constexpr int kRowsThreads = 256;
 
 template <bool kLines>
@@ -286,7 +291,8 @@ __global__ void __launch_bounds__(kRowsThreads) utf8_rows_kernel(Utf8RowsParams 
     unsigned long long* keys = s_keys[threadIdx.x >> 5];
     const uint32_t stride = P.stride;
     const int64_t n = P.n_lines;
-    if (n == 0 && blockIdx.x == 0 && threadIdx.x == 0) P.out_off[0] = kLines ? P.byte_off[0] : P.bias + P.end_off;
+    const bool write_off = !kLines || P.out_off;
+    if (n == 0 && write_off && blockIdx.x == 0 && threadIdx.x == 0) P.out_off[0] = kLines ? P.byte_off[0] : P.bias + P.end_off;
     const int64_t n_groups = (n + 31) / 32;
     const int64_t warps = static_cast<int64_t>(gridDim.x) * (kRowsThreads / 32);
     for (int64_t g = static_cast<int64_t>(blockIdx.x) * (kRowsThreads / 32) + (threadIdx.x >> 5); g < n_groups; g += warps) {
@@ -303,8 +309,10 @@ __global__ void __launch_bounds__(kRowsThreads) utf8_rows_kernel(Utf8RowsParams 
                 b0 = line == 0 ? 0 : P.byte_off[line];
                 b1 = line + 1 == n ? P.end_off : P.byte_off[line + 1];
             }
-            P.out_off[line] = b0 + P.bias;
-            if (line + 1 == n) P.out_off[n] = b1 + P.bias;
+            if (write_off) {
+                P.out_off[line] = b0 + P.bias;
+                if (line + 1 == n) P.out_off[n] = b1 + P.bias;
+            }
         }
         if (stride == 0) continue;
         uint32_t other = __ballot_sync(0xffffffffu, valid && b1 - b0 != u1 - u0);
@@ -354,8 +362,9 @@ __global__ void __launch_bounds__(kRowsThreads) utf8_rows_kernel(Utf8RowsParams 
                 const int64_t s0 = w + 32 * static_cast<int64_t>(lane);
                 uint32_t lead = 0, four = 0;
                 if (s0 < lb0 + len_b && s0 + 32 > lb0) {
+                    // (the second half only when the line reaches into it: the bytes end where the caller's buffer may end)
                     const uint4* p = reinterpret_cast<const uint4*>(P.bytes + s0);
-                    const uint4 a = __ldg(p), b = __ldg(p + 1);
+                    const uint4 a = __ldg(p), b = s0 + 16 < lb0 + len_b ? __ldg(p + 1) : make_uint4(0, 0, 0, 0);
                     const uint32_t x[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
 #pragma unroll
                     for (int q = 0; q < 8; ++q) {
@@ -429,11 +438,11 @@ void k_utf8_count(const Launch& L, const uint8_t* src, int64_t n, uint32_t* tile
 }
 
 void k_utf8_line_units(const Launch& L, const uint8_t* src, int64_t n, const int64_t* byte_off, int64_t n_off, int64_t base, const int64_t* tile_base,
-                       const uint16_t* slice_units, int64_t* unit_off, unsigned long long* first_bad) {
+                       const uint16_t* slice_units, int64_t* unit_off, unsigned long long* first_bad, unsigned long long* order_bad) {
     if (n_off <= 0) return;
     const int64_t want = (n_off + kUtf8Threads - 1) / kUtf8Threads, cap = static_cast<int64_t>(L.sm_count) * 16;
     utf8_line_units_kernel<<<static_cast<int>(want < cap ? want : cap), kUtf8Threads, 0, L.stream>>>(src, n, byte_off, n_off, base, tile_base,
-                                                                                                    slice_units, unit_off, first_bad);
+                                                                                                    slice_units, unit_off, first_bad, order_bad);
 }
 
 void k_utf8_write(const Launch& L, const uint8_t* src, int64_t n, const int64_t* tile_base, uint16_t* dst) {

@@ -178,6 +178,22 @@ int gorp_extract_text_device(gorp_engine* e, int dev_index, const uint16_t* d_te
 int gorp_extract_lines_device(gorp_engine* e, int dev_index, const uint16_t* d_text, const int64_t* d_off,
                               int64_t n_lines, void* stream, int flags, gorp_device_result* out);
 
+/* The same device-resident calls for UTF-8 held in HBM: a log file read into device memory, a torch uint8 tensor, or a
+ * cuDF / Arrow string column (its bytes plus int64 offsets; widen int32 offsets first). Results are in BYTE coordinates,
+ * exactly those of gorp_extract_text_utf8_bytes (text form) and gorp_extract_lines_utf8 (lines form, d_line_off = the
+ * caller's d_off) on the same bytes; ext_id and histogram are unchanged. Malformed UTF-8 fails with GORP_E_ARG and
+ * "malformed UTF-8 at byte N" as in the host forms; in the lines form so do offsets that start below 0 or decrease
+ * ("offsets must be non-decreasing (line i)", checked on the device), and bytes outside [d_off[0], d_off[n_lines]) are
+ * never read. Conventions of the calls above (alignment, results, stream, flags). Host round trips: two per call —
+ * text form: {decoded total, first malformed byte} and the newline count; lines form: {d_off[0], d_off[n_lines]} and
+ * {decoded total, first malformed byte, first decreasing offset}. Engine scratch: the decoded UTF-16 text, 2 bytes per
+ * input byte (n_bytes, or d_off[n_lines] - d_off[0]); the lines form also copies its bytes into the engine (1 byte per
+ * byte), so that a first string at any byte offset meets the aligned kernels. */
+int gorp_extract_text_utf8_device(gorp_engine* e, int dev_index, const uint8_t* d_text, int64_t n_bytes, void* stream, int flags,
+                                  gorp_device_result* out);
+int gorp_extract_lines_utf8_device(gorp_engine* e, int dev_index, const uint8_t* d_text, const int64_t* d_off, int64_t n_lines,
+                                   void* stream, int flags, gorp_device_result* out);
+
 /* Device time per pipeline stage, summed over the calls made with GORP_FLAG_TIME_KERNELS on (e, dev_index) since the
  * last reset: names[i] / total_ms[i] for i < *n (at most `cap`), `calls` = timed calls, `launches` = kernels launched
  * by this context (all calls). Waits for the last timed call to finish. */
