@@ -281,7 +281,9 @@ __device__ __forceinline__ void cw_item(const CapWalkParams& P, const CapItem& i
     const uint32_t reg_stride = kCapWalkThreads * 4;
     const uint32_t lt_mask = (1u << lane) - 1u;
     const uint32_t stride = P.span_stride;
-    const uint32_t inv_stride = 65536u / stride + 1u;  // i / stride == (i * inv_stride) >> 16 for i < 32 * stride <= 2048
+    // i / stride == __umulhi(i, inv_stride) for every i < 2048 and stride <= 62 (checked exhaustively; a 16-bit reciprocal
+    // is not enough for i < 32 * stride: it is one too high from i = 1679 on for stride 56, 1499 for 60, 1115 for 62)
+    const uint32_t inv_stride = 0xFFFFFFFFu / stride + 1u;
     bool exhausted = false;  // warp-uniform: the item has no unclaimed line left
 
     // per-lane state: the line being walked, and the NEXT line of the lane, claimed one line ahead so that its id
@@ -392,7 +394,7 @@ __device__ __forceinline__ void cw_item(const CapWalkParams& P, const CapItem& i
             __syncwarp();  // staging area and the finished lanes' tag registers are read by the other lanes
             const uint32_t total = static_cast<uint32_t>(__popc(fin_mask)) * stride;
             for (uint32_t i = lane; i < total; i += 32) {
-                const uint32_t j = (i * inv_stride) >> 16, k = i - j * stride;
+                const uint32_t j = __umulhi(i, inv_stride), k = i - j * stride;
                 const uint4 f = s_fin[j];
                 int32_t val = -1;
                 if (f.y != 0xFFFFFFFFu && k < x.n_slots) {

@@ -135,16 +135,16 @@ template <bool kLines, int kT, bool kAll>
 __global__ void __launch_bounds__(kT, 2) tailwalk_kernel(TailWalkParams P) {
     constexpr uint32_t kSlotStride = SlotStride<kT>::value;
     constexpr int kTailWalkThreads = kT;
-    // [table][recipes][outcome codes][several-writer list][init list][slots: (max_slots + 2) x kSlotStride]
+    // [table][recipes][outcome codes][kAll: lines per outcome][several-writer list][init list][slots: (max_slots + 2) x kSlotStride]
     extern __shared__ __align__(16) unsigned char s_mem[];
     __shared__ uint32_t s_item, s_cursor, s_loaded, s_n_multi;
-    __shared__ uint32_t s_hist[kAll ? 256 : 1];  // kAll: lines per outcome of the one table
     const TailDev& T = P.t;
     const uint32_t stride = T.span_stride;
     const uint32_t tab_bytes = T.max_table_bytes;
     uint32_t* s_res = reinterpret_cast<uint32_t*>(s_mem + tab_bytes);
     int32_t* s_oext = reinterpret_cast<int32_t*>(s_res + T.max_res);
-    uint32_t* s_multi = reinterpret_cast<uint32_t*>(s_oext + T.max_outcomes);  // (outcome << 16 | k), packed writers
+    uint32_t* s_hist = reinterpret_cast<uint32_t*>(s_oext + T.max_outcomes);  // kAll: lines per outcome of the one table
+    uint32_t* s_multi = s_hist + (kAll ? T.max_outcomes : 0u);  // (outcome << 16 | k), packed writers
     uint8_t* s_init = reinterpret_cast<uint8_t*>(s_multi + 2 * kTwMaxMulti);
     unsigned char* s_slots = reinterpret_cast<unsigned char*>(s_init + 64);
     // [order: kCapItemLines x u16][length bins: kTwBins x u32] — the item's lines sorted by length (see below)
@@ -160,7 +160,7 @@ __global__ void __launch_bounds__(kT, 2) tailwalk_kernel(TailWalkParams P) {
     const uint32_t item_lines = kAll ? P.item_lines : kCapItemLines;
     const uint32_t n_items = kAll ? (n_all + item_lines - 1) / item_lines : *P.n_items;
     if (kAll)
-        for (uint32_t i = threadIdx.x; i < 256; i += kT) s_hist[i] = 0;
+        for (uint32_t i = threadIdx.x; i < T.max_outcomes; i += kT) s_hist[i] = 0;
     const uint32_t round_iters = P.round_iters;
     const bool pf_ahead = !(P.flags & 8u);
     if (threadIdx.x == 0) s_loaded = 0xFFFFFFFFu;
@@ -489,7 +489,7 @@ __global__ void __launch_bounds__(kT, 2) tailwalk_kernel(TailWalkParams P) {
     if (kAll) {  // per-outcome line counts of this CTA -> the histogram bins of their codes
         __syncthreads();
         const TailExt x = T.ext[0];
-        for (uint32_t o = threadIdx.x; o < x.n_outcomes && o < 256u; o += kT) {
+        for (uint32_t o = threadIdx.x; o < x.n_outcomes; o += kT) {
             const int32_t code = __ldg(T.oext + x.oext_off + o);
             const uint32_t bin = code >= 0 ? static_cast<uint32_t>(code) : (code == -1 ? P.n_ext : P.n_ext + 1u);
             if (s_hist[o]) atomicAdd(P.hist + bin, static_cast<unsigned long long>(s_hist[o]));
@@ -560,8 +560,9 @@ static bool tailwalk_sort_requested() {
 }
 
 size_t tailwalk_smem_bytes(const TailDev& t, int threads) {
+    // per outcome: its code and (fused walk) its line count — up to 1008 outcomes: rows are 10-bit ids
     const size_t sort_bytes = tailwalk_sort_requested() ? kCapItemLines * 2 + kTwBins * 4 : 0;
-    return static_cast<size_t>(t.max_table_bytes) + static_cast<size_t>(t.max_res) * 4 + static_cast<size_t>(t.max_outcomes) * 4 +
+    return static_cast<size_t>(t.max_table_bytes) + static_cast<size_t>(t.max_res) * 4 + static_cast<size_t>(t.max_outcomes) * 8 +
            2 * kTwMaxMulti * 4 + 64 + ((static_cast<size_t>(t.max_slots + 2) * (static_cast<size_t>(threads) * 2 + 64) + 15) & ~size_t(15)) +
            sort_bytes + 16;
 }

@@ -570,3 +570,62 @@ extern "C" int ht_run_fused_tail(const void* blob, size_t len, const uint16_t* t
         return -1;
     }
 }
+
+// Which side of each table limit a definition lands on (the choices engine.cu makes when it builds an engine, minus the
+// shared-memory budgets, which depend on the kernels' launch shapes). out[0..11] = largest tag-register count of the capture
+// automata, span stride (2 x the most groups), fused automaton available, its op slots, its outcomes, its several-writer
+// group boundaries, fused-walk table image available, its table bytes, capture image (K4b) available, fast capture image
+// (K4 fast) available, tails of any extraction, extractions that fall back to the Pike VM. tail[e] = the tail image of
+// extraction e is available. Returns the extraction count, or -1 (err).
+extern "C" int ht_layout(const void* blob, size_t len, uint32_t* out, uint8_t* tail, int cap, char* err, int errlen) {
+    try {
+        CompiledDefinition def = parse_blob(blob, len);
+        DeviceModel m = build_device_model(def);
+        const FusedAutomaton F = build_fused(m);
+        finalize_device_model(m, F);
+        const size_t E = m.n_groups.size();
+        uint32_t max_regs = 0, max_groups = 0, n_pike = 0;
+        for (const Tdfa& t : m.tdfas) max_regs = std::max(max_regs, t.n_regs);
+        for (uint32_t g : m.n_groups) max_groups = std::max(max_groups, g);
+        for (uint8_t p : m.pike_only) n_pike += p ? 1u : 0u;
+        const uint32_t stride = 2 * max_groups;
+        std::fill(out, out + 12, 0u);
+        out[0] = max_regs;
+        out[1] = stride;
+        out[2] = F.available ? 1u : 0u;
+        if (F.available) {
+            out[3] = F.n_op_slots;
+            out[4] = static_cast<uint32_t>(F.outcomes.size());
+            for (uint32_t r : F.res) out[5] += r >= 256u ? 1u : 0u;
+            if (stride > 0) {
+                const TailImage I = build_tail_image(build_fused_tailset(F, m, stride), stride);
+                out[6] = I.available && I.ext[0].available ? 1u : 0u;
+                out[7] = I.max_table_bytes;
+            }
+        }
+        out[8] = build_cap_image(m, 4096).available ? 1u : 0u;
+        // engine.cu, fast tier image: every table within 16-bit row offsets, image + registers within 160 KB
+        {
+            const uint32_t row_bytes = (m.symbols.n_classes + 1) * 4;
+            size_t words = 128;
+            bool ok = true;
+            for (const Tdfa& t : m.tdfas) {
+                const uint64_t rows = 2ull * t.n_states + 9;
+                ok = ok && rows * row_bytes <= 0xFFFC;
+                words += rows * (row_bytes / 4);
+            }
+            words = (words + 3) & ~size_t(3);
+            const size_t reg_stride = 512 * 4;  // kernels.cuh: kCapFastThreads x 4
+            out[9] = ok && words * 4 + (max_regs + 2) * reg_stride <= 160 * 1024 && (max_regs + 2) * reg_stride <= 0x10000 ? 1u : 0u;
+        }
+        const TailSet T = build_tails(def, m);
+        out[10] = T.any ? 1u : 0u;
+        out[11] = n_pike;
+        const TailImage TI = build_tail_image(T, stride);
+        for (size_t e = 0; e < E && static_cast<int>(e) < cap; ++e) tail[e] = T.any && TI.ext[e].available ? 1u : 0u;
+        return static_cast<int>(E);
+    } catch (const std::exception& e) {
+        std::snprintf(err, errlen, "%s", e.what());
+        return -1;
+    }
+}

@@ -108,3 +108,23 @@ def run_tails(blob_bytes: bytes, text: np.ndarray, stride: int):
     if n < 0:
         raise RuntimeError(err.value.decode())
     return ext[:n], spans[:n, :stride], stats
+
+
+LAYOUT_FIELDS = ("max_regs", "stride", "fused", "fused_slots", "fused_outcomes", "fused_multi", "fused_image", "fused_table_bytes",
+                 "capimg", "cap_fast", "tails", "pike")
+
+
+def layout(blob_bytes: bytes):
+    """Which side of each table limit a definition lands on (tests/host/hosttest.cpp: ht_layout): a dict of LAYOUT_FIELDS
+    and "tail", the per-extraction availability of the tail image."""
+    lib = load()
+    out = np.zeros(len(LAYOUT_FIELDS), dtype=np.uint32)
+    tail = np.zeros(4096, dtype=np.uint8)
+    err = C.create_string_buffer(1024)
+    P = C.c_void_p
+    n = lib.ht_layout(blob_bytes, C.c_size_t(len(blob_bytes)), P(out.ctypes.data), P(tail.ctypes.data), C.c_int(len(tail)), err, C.c_int(1024))
+    if n < 0:
+        raise RuntimeError(err.value.decode())
+    d = dict(zip(LAYOUT_FIELDS, (int(v) for v in out)))
+    d["tail"] = [bool(v) for v in tail[:n]]
+    return d
