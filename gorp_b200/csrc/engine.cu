@@ -650,7 +650,7 @@ int64_t run_pipeline(DeviceCtx& c, const uint16_t* d_text, int64_t n_units, cons
     gorp_device_result local{};
     gorp_device_result* r = out ? out : &local;
     const int64_t nl = run_pipeline_tables(c, d_text, n_units, d_off, n_lines, stream, tm, r);
-    if (c.pike.enabled && nl > 0 && !c.cap.match_only && c.max_slots > 0) {
+    if (c.pike.enabled && nl > 0 && !c.cap.match_only) {
         Launch L{stream, c.sm_count};
         const size_t per_thread = pike_scratch_ints_per_thread(c.pike) * 4;
         size_t threads = static_cast<size_t>(c.sm_count) * 128;
@@ -661,7 +661,7 @@ int64_t run_pipeline(DeviceCtx& c, const uint16_t* d_text, int64_t n_units, cons
         k_pike_fixup(L, c.pike, d_text, r->d_line_off, d_off ? 0 : 1, nl, c.max_slots, const_cast<int32_t*>(r->d_ext_id),
                      const_cast<int32_t*>(r->d_spans), reinterpret_cast<unsigned long long*>(const_cast<int64_t*>(r->d_histogram)), c.n_ext,
                      c.pike_scratch.as<int32_t>(), static_cast<uint32_t>(threads));
-        c.launches += 1;
+        tm.mark("pike_fixup", 1);
         CK(cudaGetLastError());
     }
     return nl;
@@ -900,7 +900,7 @@ int64_t run_pipeline_tables(DeviceCtx& c, const uint16_t* d_text, int64_t n_unit
             k4b_capwalk(L, W);
             tm.mark("k4b_capwalk", 1);
         }
-    } else if (!c.cap.match_only && stride > 0) {
+    } else if (!c.cap.match_only) {  // (also at stride 0: a definition without groups still has to fail the lines its regexes reject)
         if (sep == 1 && c.cap_fast.enabled && !c.force_general) {
             k4_tdfa_fast(L, c.cap_fast, c.cap, d_text, n_units, d_line_off, n_fast, stride, c.ext_id.as<int32_t>(), c.spans.as<int32_t>());
             if (n_fast < n_lines)
