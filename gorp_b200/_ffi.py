@@ -48,13 +48,23 @@ class DeviceResult(C.Structure):
                 ("d_n_lines", C.c_void_p)]
 
 
+class ValueTable(C.Structure):
+    _fields_ = [("n_rows", C.c_int64), ("n_columns", C.c_int32), ("reserved", C.c_int32),
+                ("d_row", C.c_void_p), ("d_offsets", C.POINTER(C.c_void_p)), ("d_data", C.POINTER(C.c_void_p)),
+                ("d_valid", C.POINTER(C.c_void_p)), ("null_count", C.POINTER(C.c_int64))]
+
+
+class DeviceTables(C.Structure):
+    _fields_ = [("n_tables", C.c_int32), ("unit_bytes", C.c_int32), ("tables", C.POINTER(ValueTable))]
+
+
 # every symbol include/gorp_cuda.h declares (tests/test_abi.py checks the list against the header)
 SYMBOLS = [
     "gorp_abi_version", "gorp_last_error", "gorp_device_count", "gorp_compile_definition", "gorp_compile_patterns",
     "gorp_blob_free", "gorp_blob_get_info", "gorp_blob_get_extraction", "gorp_blob_get_extractor_name",
     "gorp_blob_get_tables", "gorp_engine_create", "gorp_engine_destroy", "gorp_extract_lines", "gorp_extract_text", "gorp_extract_text_latin1", "gorp_extract_text_utf8", "gorp_extract_text_utf8_bytes", "gorp_extract_lines_utf8", "gorp_match_all_lines", "gorp_match_result_release",
     "gorp_result_release", "gorp_extract_text_device", "gorp_extract_lines_device", "gorp_extract_text_utf8_device",
-    "gorp_extract_lines_utf8_device", "gorp_kernel_times",
+    "gorp_extract_lines_utf8_device", "gorp_extract_tables_device", "gorp_kernel_times",
 ]
 
 lib.gorp_abi_version.restype = C.c_int
@@ -94,6 +104,7 @@ lib.gorp_extract_text_utf8_device.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C
                                               C.POINTER(DeviceResult)]
 lib.gorp_extract_lines_utf8_device.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int,
                                                C.POINTER(DeviceResult)]
+lib.gorp_extract_tables_device.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.POINTER(DeviceTables)]
 lib.gorp_kernel_times.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_char_p), C.POINTER(C.c_double), C.c_int,
                                   C.POINTER(C.c_int), C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.c_int]
 FLAG_SYNC, FLAG_TIME_KERNELS = 1, 2

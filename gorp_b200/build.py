@@ -21,7 +21,8 @@ HOST_SOURCES = [os.path.join(CSRC, "host", f) for f in
 CUDA_SOURCES = [os.path.join(CSRC, "engine.cu"), os.path.join(CSRC, "kernels", "kernels.cu"),
                 os.path.join(CSRC, "kernels", "fast.cu"),
                 os.path.join(CSRC, "kernels", "dfawalk.cu"),
-                os.path.join(CSRC, "kernels", "capwalk.cu"), os.path.join(CSRC, "kernels", "tailwalk.cu"), os.path.join(CSRC, "kernels", "utf8.cu"), os.path.join(CSRC, "kernels", "matchall.cu"), os.path.join(CSRC, "kernels", "pike.cu")]
+                os.path.join(CSRC, "kernels", "capwalk.cu"), os.path.join(CSRC, "kernels", "tailwalk.cu"), os.path.join(CSRC, "kernels", "utf8.cu"), os.path.join(CSRC, "kernels", "matchall.cu"), os.path.join(CSRC, "kernels", "pike.cu"),
+                os.path.join(CSRC, "kernels", "tables.cu")]
 OBJ_DIR = os.path.join(HERE, "_obj")
 COMPILE_FLAGS = ["-std=c++17", "-O3", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
                  "-Xcompiler", "-fPIC,-Wall", "-I", os.path.join(ROOT, "include")]

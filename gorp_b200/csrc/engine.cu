@@ -164,6 +164,18 @@ struct DeviceCtx {
     // per-call scratch, serialised by `mu`
     std::mutex mu;
     DevBuf text, off_in, line_off, tile_counts, tile_base, scan_scratch, ext_id, spans, hist, scalars;
+    // the result of the last successful device-resident extract call, which gorp_extract_tables_device reads; every other
+    // call that takes `mu` through CtxLock forgets it (its scratch may hold something else by then)
+    int last_unit_bytes = 0;  // 2: a UTF-16 call, 1: a UTF-8 call, 0: none
+    const void* last_text = nullptr;
+    gorp_device_result last{};
+    // value tables of gorp_extract_tables_device: device buffers, and the host descriptors the caller reads
+    DevBuf tb_counts, tb_starts, tb_scan, tb_layout, tb_rows, tb_lens, tb_valid, tb_stats, tb_offs, tb_colinfo, tb_data;
+    std::vector<gorp_value_table> tb_tables;
+    std::vector<const int64_t*> tb_off_ptr;
+    std::vector<const void*> tb_data_ptr;
+    std::vector<const uint8_t*> tb_valid_ptr;
+    std::vector<int64_t> tb_nulls;
     // per-kernel device time: CUDA events on the launching stream, accumulated over timed calls
     cudaEvent_t ev[kMaxTimed + 1]{};
     const char* ev_name[kMaxTimed]{};
@@ -188,6 +200,13 @@ struct DeviceCtx {
         if (s_in) cudaStreamDestroy(s_in);
         if (s_out) cudaStreamDestroy(s_out);
     }
+};
+
+// Holds c.mu for an extract or match call: the device-resident result that gorp_extract_tables_device reads does not
+// survive it (a device-resident call that succeeds records its own result again).
+struct CtxLock {
+    std::unique_lock<std::mutex> lock;
+    explicit CtxLock(DeviceCtx& c) : lock(c.mu) { c.last_unit_bytes = 0; }
 };
 
 // NUMA node of a CUDA device (sysfs numa_node of its PCI function), or -1 when the platform does not say
@@ -1290,7 +1309,7 @@ int extract_host(gorp_engine* e, const uint16_t* text, const uint8_t* text8, int
         DeviceGuard restore_device;
         if (G <= 1) {
             DeviceRun run;
-            std::lock_guard<std::mutex> lock(e->devs[0]->mu);
+            CtxLock lock(*e->devs[0]);
             run_pieces(e, *e->devs[0], text, text8, utf8, byte_coords, off, pieces, 0, pieces.size(), hr.get(), run);
             nl = run.n_rows;
             stride = run.stride;
@@ -1299,8 +1318,8 @@ int extract_host(gorp_engine* e, const uint16_t* text, const uint8_t* text8, int
             // host thread per device; the rows are copied out once every device's row base is known
             // every participating device stays locked (in device order) from the first kernel to the last row copied out:
             // a concurrent call on the same engine can neither overwrite the accumulators nor free them in between
-            std::vector<std::unique_lock<std::mutex>> locks;
-            for (size_t d = 0; d < G; ++d) locks.emplace_back(e->devs[d]->mu);
+            std::vector<CtxLock> locks;
+            for (size_t d = 0; d < G; ++d) locks.emplace_back(*e->devs[d]);
             std::vector<DeviceRun> runs(G);
             std::vector<size_t> first(G + 1);
             for (size_t d = 0; d <= G; ++d) first[d] = pieces.size() * d / G;
@@ -1663,7 +1682,7 @@ int gorp_match_all_lines(gorp_engine* e, const uint16_t* text, const int64_t* of
     if (!text && n_lines > 0 && off[n_lines] > off[0]) return fail(GORP_E_ARG, "null text");
     return guarded([&]() -> int {
         DeviceCtx& c = *e->devs[0];
-        std::lock_guard<std::mutex> lock(c.mu);
+        CtxLock lock(c);
         DeviceGuard restore_device;
         CK(cudaSetDevice(c.device));
         CK(cudaStreamWaitEvent(c.stream, c.ev_done, 0));
@@ -1732,14 +1751,17 @@ int gorp_extract_text_device(gorp_engine* e, int dev_index, const uint16_t* d_te
         return fail(GORP_E_ARG, "bad argument (d_text must be 16-byte aligned)");
     return guarded([&]() -> int {
         DeviceCtx& c = *e->devs[dev_index];
-        std::lock_guard<std::mutex> lock(c.mu);
+        CtxLock lock(c);
         DeviceGuard restore_device;
         CK(cudaSetDevice(c.device));
         cudaStream_t st = static_cast<cudaStream_t>(stream);
         CK(cudaStreamWaitEvent(st, c.ev_done, 0));  // the previous call on this context (any stream) used the same scratch
         Timer tm(c, st, (flags & GORP_FLAG_TIME_KERNELS) != 0);
-        run_pipeline(c, d_text, n_units, nullptr, 0, st, tm, out);
+        run_pipeline(c, d_text, n_units, nullptr, 0, st, tm, &c.last);
+        if (out) *out = c.last;
         CK(cudaEventRecord(c.ev_done, st));
+        c.last_unit_bytes = 2;
+        c.last_text = d_text;
         if (flags & GORP_FLAG_SYNC) CK(cudaStreamSynchronize(st));
         return GORP_OK;
     });
@@ -1752,7 +1774,7 @@ int gorp_extract_lines_device(gorp_engine* e, int dev_index, const uint16_t* d_t
         return fail(GORP_E_ARG, "bad argument (d_text must be 16-byte aligned)");
     return guarded([&]() -> int {
         DeviceCtx& c = *e->devs[dev_index];
-        std::lock_guard<std::mutex> lock(c.mu);
+        CtxLock lock(c);
         DeviceGuard restore_device;
         CK(cudaSetDevice(c.device));
         cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -1763,8 +1785,11 @@ int gorp_extract_lines_device(gorp_engine* e, int dev_index, const uint16_t* d_t
             CK(cudaStreamSynchronize(st));
         }
         Timer tm(c, st, (flags & GORP_FLAG_TIME_KERNELS) != 0);
-        run_pipeline(c, d_text, n_units, d_off, n_lines, st, tm, out);
+        run_pipeline(c, d_text, n_units, d_off, n_lines, st, tm, &c.last);
+        if (out) *out = c.last;
         CK(cudaEventRecord(c.ev_done, st));
+        c.last_unit_bytes = 2;
+        c.last_text = d_text;
         if (flags & GORP_FLAG_SYNC) CK(cudaStreamSynchronize(st));
         return GORP_OK;
     });
@@ -1776,7 +1801,7 @@ int gorp_extract_text_utf8_device(gorp_engine* e, int dev_index, const uint8_t* 
         return fail(GORP_E_ARG, "bad argument (d_text must be 16-byte aligned)");
     return guarded([&]() -> int {
         DeviceCtx& c = *e->devs[dev_index];
-        std::lock_guard<std::mutex> lock(c.mu);
+        CtxLock lock(c);
         DeviceGuard restore_device;
         CK(cudaSetDevice(c.device));
         cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -1798,6 +1823,9 @@ int gorp_extract_text_utf8_device(gorp_engine* e, int dev_index, const uint8_t* 
         dr.d_spans = c.acc_spans.as<int32_t>();
         if (out) *out = dr;
         CK(cudaEventRecord(c.ev_done, st));
+        c.last = dr;
+        c.last_unit_bytes = 1;
+        c.last_text = d_text;
         if (flags & GORP_FLAG_SYNC) CK(cudaStreamSynchronize(st));
         return GORP_OK;
     });
@@ -1810,7 +1838,7 @@ int gorp_extract_lines_utf8_device(gorp_engine* e, int dev_index, const uint8_t*
         return fail(GORP_E_ARG, "bad argument (d_text must be 16-byte aligned)");
     return guarded([&]() -> int {
         DeviceCtx& c = *e->devs[dev_index];
-        std::lock_guard<std::mutex> lock(c.mu);
+        CtxLock lock(c);
         DeviceGuard restore_device;
         CK(cudaSetDevice(c.device));
         cudaStream_t st = static_cast<cudaStream_t>(stream);
@@ -1846,6 +1874,119 @@ int gorp_extract_lines_utf8_device(gorp_engine* e, int dev_index, const uint8_t*
         dr.d_line_off = d_off;
         dr.d_spans = c.acc_spans.as<int32_t>();
         if (out) *out = dr;
+        CK(cudaEventRecord(c.ev_done, st));
+        c.last = dr;
+        c.last_unit_bytes = 1;
+        c.last_text = d_text;
+        if (flags & GORP_FLAG_SYNC) CK(cudaStreamSynchronize(st));
+        return GORP_OK;
+    });
+}
+
+int gorp_extract_tables_device(gorp_engine* e, int dev_index, void* stream, int flags, gorp_device_tables* out) {
+    if (!e || !out || dev_index < 0 || dev_index >= static_cast<int>(e->devs.size())) return fail(GORP_E_ARG, "bad argument");
+    return guarded([&]() -> int {
+        DeviceCtx& c = *e->devs[dev_index];
+        std::lock_guard<std::mutex> lock(c.mu);  // (not CtxLock: the tables leave the result they read as it is)
+        if (!c.last_unit_bytes)
+            throw ArgError("no device-resident result to make tables of: the last call on this engine and device must be a successful "
+                           "gorp_extract_*_device call");
+        DeviceGuard restore_device;
+        CK(cudaSetDevice(c.device));
+        cudaStream_t st = static_cast<cudaStream_t>(stream);
+        CK(cudaStreamWaitEvent(st, c.ev_done, 0));  // the previous call on this context (any stream) used the same scratch
+        Launch L{st, c.sm_count};
+        Timer tm(c, st, (flags & GORP_FLAG_TIME_KERNELS) != 0);
+        const gorp_device_result& r = c.last;
+        const uint32_t E = c.n_ext;
+        const int64_t n = r.n_lines;
+        const uint32_t stride = static_cast<uint32_t>(r.span_stride);
+        int64_t n_cols = 0;  // columns of all tables
+        for (const auto& x : e->def.extractions) n_cols += stride ? x.n_groups : 0;
+        // 1. rank: stable partition of the matched lines by extraction
+        const int64_t tile = tables_tile_lines(E), n_tiles = std::max<int64_t>(1, (n + tile - 1) / tile), cells = n_tiles * E;
+        c.tb_counts.reserve(static_cast<size_t>(cells) * 4 + 64);
+        c.tb_starts.reserve(static_cast<size_t>(cells + 1) * 8 + 64);
+        c.tb_layout.reserve((E + 1) * sizeof(TableLayout));
+        c.tb_rows.reserve(static_cast<size_t>(n + 8 * E + 8) * 8);
+        c.tb_stats.reserve(static_cast<size_t>(n_cols) * 16 + 64);
+        TableLayout* lay = c.tb_layout.as<TableLayout>();
+        k_tables_count(L, r.d_ext_id, n, E, tile, n_tiles, c.tb_counts.as<uint32_t>());
+        c.tb_scan.reserve(static_cast<size_t>(cells / 4096 + 8) * 8);
+        scan_u32_to_i64(L, c.tb_counts.as<uint32_t>(), cells, c.tb_starts.as<int64_t>(), c.tb_scan.as<int64_t>());
+        k_tables_layout(L, c.tb_starts.as<int64_t>(), n_tiles, E, c.d_slots, stride != 0, lay);
+        k_tables_scatter(L, r.d_ext_id, n, E, tile, n_tiles, c.tb_starts.as<int64_t>(), lay, c.tb_rows.as<int64_t>());
+        CK(cudaGetLastError());
+        tm.mark("tables_rank", 6);
+        // 2. lengths, validity, per-column totals and null counts (sized for every line in the widest extraction)
+        const int64_t slots_ub = n * (stride / 2) + 8 * n_cols + 8, words_ub = n * (stride / 2) / 32 + 17 * n_cols + 16;
+        c.tb_lens.reserve(static_cast<size_t>(slots_ub) * 4);
+        c.tb_valid.reserve(static_cast<size_t>(words_ub) * 4);
+        CK(cudaMemsetAsync(c.tb_valid.p, 0, static_cast<size_t>(words_ub) * 4, st));
+        if (n_cols) CK(cudaMemsetAsync(c.tb_stats.p, 0, static_cast<size_t>(n_cols) * 16, st));
+        k_tables_len(L, lay, E, c.tb_rows.as<int64_t>(), r.d_spans, stride, c.tb_lens.as<uint32_t>(), c.tb_valid.as<uint32_t>(),
+                     c.tb_stats.as<unsigned long long>());
+        CK(cudaGetLastError());
+        tm.mark("tables_len", 1);
+        // the one round trip: the layout and the column totals
+        std::vector<TableLayout> h_lay(E + 1);
+        std::vector<int64_t> h_stats(static_cast<size_t>(n_cols) * 2);
+        CK(cudaMemcpyAsync(h_lay.data(), lay, (E + 1) * sizeof(TableLayout), cudaMemcpyDeviceToHost, st));
+        if (n_cols) CK(cudaMemcpyAsync(h_stats.data(), c.tb_stats.p, h_stats.size() * 8, cudaMemcpyDeviceToHost, st));
+        CK(cudaStreamSynchronize(st));
+        if (h_lay[E].col_base != n_cols) throw std::runtime_error("value tables: column count mismatch");
+        // 3. offsets: one scan over the lengths of every column; 4. gather into 64-byte aligned columns
+        const int64_t n_off = h_lay[E].off_base;
+        const int ub = c.last_unit_bytes;
+        std::vector<int64_t> col_info(static_cast<size_t>(n_cols) * 2 + 2);
+        int64_t flat = 0, data_bytes = 0;
+        for (int64_t k = 0; k < n_cols; ++k) {
+            col_info[2 * k] = flat;
+            col_info[2 * k + 1] = data_bytes;
+            flat += h_stats[2 * k];
+            data_bytes += (h_stats[2 * k] * ub + 63) / 64 * 64;
+        }
+        c.tb_offs.reserve(static_cast<size_t>(n_off + 1) * 8 + 64);
+        c.tb_scan.reserve(static_cast<size_t>(n_off / 4096 + 8) * 8);
+        scan_u32_to_i64(L, c.tb_lens.as<uint32_t>(), n_off, c.tb_offs.as<int64_t>(), c.tb_scan.as<int64_t>());
+        CK(cudaGetLastError());
+        tm.mark("tables_scan", 3);
+        c.tb_colinfo.reserve(col_info.size() * 8);
+        CK(cudaMemcpyAsync(c.tb_colinfo.p, col_info.data(), col_info.size() * 8, cudaMemcpyHostToDevice, st));
+        c.tb_data.reserve(static_cast<size_t>(data_bytes) + 64);
+        k_tables_gather(L, lay, E, c.tb_rows.as<int64_t>(), r.d_line_off, r.d_spans, stride, c.last_text, ub, c.tb_lens.as<uint32_t>(),
+                        c.tb_offs.as<int64_t>(), c.tb_colinfo.as<int64_t>(), c.tb_data.as<uint8_t>());
+        CK(cudaGetLastError());
+        tm.mark("tables_gather", 1);
+        // (the host copy of col_info above is pageable: it has been staged by the time cudaMemcpyAsync returns)
+        c.tb_tables.assign(E, gorp_value_table{});
+        c.tb_off_ptr.assign(static_cast<size_t>(n_cols), nullptr);
+        c.tb_data_ptr.assign(static_cast<size_t>(n_cols), nullptr);
+        c.tb_valid_ptr.assign(static_cast<size_t>(n_cols), nullptr);
+        c.tb_nulls.assign(static_cast<size_t>(n_cols), 0);
+        for (uint32_t t = 0; t < E; ++t) {
+            const TableLayout& x = h_lay[t];
+            gorp_value_table& v = c.tb_tables[t];
+            v.n_rows = x.n_rows;
+            v.n_columns = static_cast<int32_t>(x.n_cols);
+            v.d_row = c.tb_rows.as<int64_t>() + x.row_base;
+            for (int64_t k = 0; k < x.n_cols; ++k) {
+                const int64_t col = x.col_base + k;
+                c.tb_off_ptr[col] = c.tb_offs.as<int64_t>() + x.off_base + k * x.seg;
+                c.tb_data_ptr[col] = c.tb_data.as<uint8_t>() + col_info[2 * col + 1];
+                c.tb_valid_ptr[col] = reinterpret_cast<const uint8_t*>(c.tb_valid.as<uint32_t>() + x.valid_base + k * x.vwords);
+                c.tb_nulls[col] = h_stats[2 * col + 1];
+            }
+            if (x.n_cols) {
+                v.d_offsets = c.tb_off_ptr.data() + x.col_base;
+                v.d_data = c.tb_data_ptr.data() + x.col_base;
+                v.d_valid = c.tb_valid_ptr.data() + x.col_base;
+                v.null_count = c.tb_nulls.data() + x.col_base;
+            }
+        }
+        out->n_tables = static_cast<int32_t>(E);
+        out->unit_bytes = ub;
+        out->tables = c.tb_tables.data();
         CK(cudaEventRecord(c.ev_done, st));
         if (flags & GORP_FLAG_SYNC) CK(cudaStreamSynchronize(st));
         return GORP_OK;

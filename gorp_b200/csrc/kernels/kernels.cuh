@@ -363,6 +363,34 @@ size_t pike_scratch_ints_per_thread(const PikeDev&);
 void k_pike_fixup(const Launch&, const PikeDev&, const uint16_t* text, const int64_t* line_off, int sep, int64_t n_lines, uint32_t span_stride,
                   int32_t* ext_id, int32_t* spans, unsigned long long* hist, uint32_t n_ext, int32_t* scratch, uint32_t scratch_threads);
 
+// Value tables of a device-resident result (kernels/tables.cu, gorp_extract_tables_device). Positions of table e in the
+// call's buffers, all in elements; entry E of the layout array holds the totals.
+struct TableLayout {
+    int64_t n_rows;              // matched lines of extraction e
+    int64_t row_base;            // of its row indexes (multiple of 8)
+    int64_t off_base;            // of column 0's offset segment; column k at off_base + k * seg
+    int64_t seg;                 // offset entries per column: round_up(n_rows + 1, 8)
+    int64_t valid_base;          // u32 words of column 0's bitmap; column k at valid_base + k * vwords
+    int64_t vwords;              // round_up(ceil(n_rows / 32), 16)
+    int64_t len_task, gather_task;  // first task of the table in the length and gather passes
+    int64_t col_base;            // index of column 0 among all columns
+    int64_t n_cols;              // groups of e
+};
+int64_t tables_tile_lines(uint32_t n_ext);  // lines per tile of the count / scatter passes
+// counts[e * n_tiles + t] = lines of extraction e in tile t
+void k_tables_count(const Launch&, const int32_t* ext_id, int64_t n_lines, uint32_t n_ext, int64_t tile_lines, int64_t n_tiles, uint32_t* counts);
+// starts = exclusive scan of counts; slots[e] = 2 * groups of e (ignored when !with_groups: every table has 0 columns)
+void k_tables_layout(const Launch&, const int64_t* starts, int64_t n_tiles, uint32_t n_ext, const uint32_t* slots, bool with_groups,
+                     TableLayout* lay);
+void k_tables_scatter(const Launch&, const int32_t* ext_id, int64_t n_lines, uint32_t n_ext, int64_t tile_lines, int64_t n_tiles,
+                      const int64_t* starts, const TableLayout* lay, int64_t* rows);
+// lens[lay.off_base total], valid (zeroed by the caller), stats[2 * columns] (zeroed: value units, nulls)
+void k_tables_len(const Launch&, const TableLayout* lay, uint32_t n_ext, const int64_t* rows, const int32_t* spans, uint32_t stride,
+                  uint32_t* lens, uint32_t* valid, unsigned long long* stats);
+// offs = scan of lens; col_info[2 * col] = offs at the column's entry 0, col_info[2 * col + 1] = byte offset of its data
+void k_tables_gather(const Launch&, const TableLayout* lay, uint32_t n_ext, const int64_t* rows, const int64_t* line_off, const int32_t* spans,
+                     uint32_t stride, const void* text, int unit_bytes, const uint32_t* lens, int64_t* offs, const int64_t* col_info, uint8_t* data);
+
 // K3: per-extraction histogram (E entries, then MISS, then capture failures).
 void k3_histogram(const Launch&, const int32_t* ext_id, int64_t n_lines, uint32_t n_ext, unsigned long long* hist);
 

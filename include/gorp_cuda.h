@@ -194,6 +194,51 @@ int gorp_extract_text_utf8_device(gorp_engine* e, int dev_index, const uint8_t* 
 int gorp_extract_lines_utf8_device(gorp_engine* e, int dev_index, const uint8_t* d_text, const int64_t* d_off, int64_t n_lines,
                                    void* stream, int flags, gorp_device_result* out);
 
+/* What ExtractionResult.asMap() gives per line, as columns in device memory: one table per extraction, one string column per
+ * extractor name, in Arrow layout (large_utf8 for the UTF-8 calls: 64-bit offsets, LSB-first validity bitmap), so that
+ * Arrow's C data interface, cuDF or torch can wrap the buffers without copying.
+ *
+ * Source: the result of the last successful device-resident extract call on (e, dev_index) — gorp_extract_text_device,
+ * gorp_extract_lines_device, gorp_extract_text_utf8_device or gorp_extract_lines_utf8_device. Every other extract or match
+ * call that reaches the context (the host forms reuse the same result scratch, gorp_match_all_lines, a device-resident call
+ * that fails) makes that result unreadable: the call then fails with GORP_E_ARG, as it does when no such call ran. A call
+ * refused for its arguments before it reaches the context, gorp_kernel_times and this call itself leave the result readable.
+ * The caller's d_text (and d_off of the lines forms) must hold the same contents, in stream order, until this call's kernels
+ * have run: the values are read from there.
+ *
+ * Rows: table e holds exactly the lines with ext_id == e, in ascending line order (n_rows == histogram[e]); MISS and
+ * CAPTURE_FAIL lines are in no table. Values: row r of column k, with span (s, t) of group k of the line, is code units
+ * [line_off[line] + s, line_off[line] + t) of the caller's d_text, not transcoded — UTF-16 units (Java `char` data) after
+ * the UTF-16 calls, bytes after the UTF-8 calls (every group boundary is a sequence start there, so each column is valid
+ * UTF-8); offsets count the same units. A group that did not participate, (-1, -1), is a null: bit r of the bitmap is 0
+ * and the value is empty. Bitmap padding bits are 0. An extraction without groups has 0 columns (null column arrays) and
+ * only d_row; a table without rows has offsets {0} in every column.
+ *
+ * Every device buffer is 64-byte aligned. The tables stay valid until the next extract call on (e, dev_index); a second
+ * tables call replaces them; the extract result they came from is not changed. Conventions of the device-resident calls
+ * (stream, GORP_FLAG_SYNC, GORP_FLAG_TIME_KERNELS: stages tables_rank, tables_len, tables_scan, tables_gather). Host round
+ * trips: one (the per-column totals that size the value buffers). Engine scratch: 8 B per line of the result (row
+ * indexes) and 12 B per (line, group of the widest extraction) for lengths and the offset scan, then 8 B per value
+ * (offsets), the values themselves and the bitmaps; plus 12 B per (extraction, tile of max(2048, 32 * extractions) lines). */
+typedef struct gorp_value_table {       /* the lines of extraction e, in line order */
+    int64_t n_rows;                     /* == histogram[e] of the call */
+    int32_t n_columns;                  /* == groups of e; column k = extractor name k (gorp_blob_get_extractor_name(e, k)) */
+    int32_t reserved;
+    const int64_t* d_row;               /* [n_rows] index of the line in the call's result, strictly ascending */
+    const int64_t* const* d_offsets;    /* host array [n_columns] of device pointers, each [n_rows + 1], offsets[0] = 0 */
+    const void* const* d_data;          /* host array [n_columns] of device pointers: the values, concatenated */
+    const uint8_t* const* d_valid;      /* host array [n_columns] of device pointers: Arrow validity bitmaps */
+    const int64_t* null_count;          /* host [n_columns] */
+} gorp_value_table;
+
+typedef struct gorp_device_tables {
+    int32_t n_tables;                   /* == n_extractions; table e = extraction e */
+    int32_t unit_bytes;                 /* 2 after the UTF-16 calls, 1 after the UTF-8 calls */
+    const gorp_value_table* tables;     /* host array [n_tables] */
+} gorp_device_tables;
+
+int gorp_extract_tables_device(gorp_engine* e, int dev_index, void* stream, int flags, gorp_device_tables* out);
+
 /* Device time per pipeline stage, summed over the calls made with GORP_FLAG_TIME_KERNELS on (e, dev_index) since the
  * last reset: names[i] / total_ms[i] for i < *n (at most `cap`), `calls` = timed calls, `launches` = kernels launched
  * by this context (all calls). Waits for the last timed call to finish. */
