@@ -64,7 +64,8 @@ SYMBOLS = [
     "gorp_blob_free", "gorp_blob_get_info", "gorp_blob_get_extraction", "gorp_blob_get_extractor_name",
     "gorp_blob_get_tables", "gorp_engine_create", "gorp_engine_destroy", "gorp_extract_lines", "gorp_extract_text", "gorp_extract_text_latin1", "gorp_extract_text_utf8", "gorp_extract_text_utf8_bytes", "gorp_extract_lines_utf8", "gorp_match_all_lines", "gorp_match_result_release",
     "gorp_result_release", "gorp_extract_text_device", "gorp_extract_lines_device", "gorp_extract_text_utf8_device",
-    "gorp_extract_lines_utf8_device", "gorp_extract_tables_device", "gorp_kernel_times",
+    "gorp_extract_lines_utf8_device", "gorp_extract_tables_device", "gorp_extract_text_utf8_tables", "gorp_extract_lines_utf8_tables",
+    "gorp_kernel_times",
 ]
 
 lib.gorp_abi_version.restype = C.c_int
@@ -105,6 +106,8 @@ lib.gorp_extract_text_utf8_device.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C
 lib.gorp_extract_lines_utf8_device.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int,
                                                C.POINTER(DeviceResult)]
 lib.gorp_extract_tables_device.argtypes = [C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.POINTER(DeviceTables)]
+lib.gorp_extract_text_utf8_tables.argtypes = [C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(Result), C.POINTER(DeviceTables)]
+lib.gorp_extract_lines_utf8_tables.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.POINTER(Result), C.POINTER(DeviceTables)]
 lib.gorp_kernel_times.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_char_p), C.POINTER(C.c_double), C.c_int,
                                   C.POINTER(C.c_int), C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.c_int]
 FLAG_SYNC, FLAG_TIME_KERNELS = 1, 2

@@ -193,14 +193,68 @@ class ExtractionResult:
         return out
 
 
+def _host_array(ptr, n, dtype):
+    """numpy copy of n elements at host address ptr."""
+    if n == 0:
+        return np.zeros(0, dtype=dtype)
+    return np.ctypeslib.as_array(C.cast(ptr, C.POINTER(np.ctypeslib.as_ctypes_type(dtype))), (n,)).copy()
+
+
+class ValueColumn:
+    """One extractor name of a ValueTable in Arrow large_string layout: value r is data[offsets[r]:offsets[r + 1]] (UTF-8),
+    null where bit r of `valid` (LSB first) is 0."""
+
+    def __init__(self, offsets, data, valid, null_count):
+        self.offsets, self.data, self.valid, self.null_count = offsets, data, valid, null_count
+
+
+class ValueTable:
+    """What ExtractionResult.asMap() gives for the lines of one extraction, as columns: `rows` (int64) are the indexes of
+    those lines in the batch, ascending; `columns` maps each extractor name to a ValueColumn."""
+
+    def __init__(self, name, rows, columns):
+        self.name, self.rows, self.columns = name, rows, columns
+
+    @property
+    def n_rows(self):
+        return len(self.rows)
+
+    def to_arrow(self):
+        """A pyarrow.Table of large_string columns over this table's buffers (no copy). An extraction without groups gives
+        a table without columns."""
+        import pyarrow as pa
+        n = len(self.rows)
+        arrays = [pa.LargeStringArray.from_buffers(n, pa.py_buffer(c.offsets), pa.py_buffer(c.data), pa.py_buffer(c.valid), c.null_count)
+                  for c in self.columns.values()]
+        return pa.Table.from_arrays(arrays, names=list(self.columns))
+
+
+def _value_tables(gorp, dt: _ffi.DeviceTables):
+    """numpy copies of the host tables of a gorp_extract_*_utf8_tables call."""
+    out = []
+    for e in range(dt.n_tables):
+        t = dt.tables[e]
+        n = int(t.n_rows)
+        x = gorp._extractions[e]
+        cols = {}
+        for k, name in enumerate(x.getExtractorNames()[:t.n_columns]):
+            off = _host_array(t.d_offsets[k], n + 1, np.int64)
+            cols[name] = ValueColumn(off, _host_array(t.d_data[k], int(off[-1]), np.uint8), _host_array(t.d_valid[k], (n + 7) // 8, np.uint8),
+                                     int(t.null_count[k]))
+        out.append(ValueTable(x.getName(), _host_array(t.d_row, n, np.int64), cols))
+    return out
+
+
 class ExtractionBatch:
     """Columnar result of one batch call: numpy copies of the gorp_result arrays + lazy ExtractionResult views.
     `units` is the text the offsets index, in `encoding`: UTF-16 units, or the caller's UTF-8 bytes (byte coordinates);
-    a line or a value is decoded from its own slice only."""
+    a line or a value is decoded from its own slice only. `tables` (the UTF-8 calls with tables=True, else None): one
+    ValueTable per extraction."""
 
-    def __init__(self, gorp, units, res: _ffi.Result, sep, encoding="utf-16-le"):
+    def __init__(self, gorp, units, res: _ffi.Result, sep, encoding="utf-16-le", tables=None):
         n = res.n_lines
         self.gorp, self.units, self.sep, self.n_lines, self.encoding = gorp, units, sep, n, encoding
+        self.tables = None if tables is None else _value_tables(gorp, tables)
         self.ext_id = np.ctypeslib.as_array(res.ext_id, (max(n, 1),))[:n].copy()
         self.line_off = np.ctypeslib.as_array(res.line_off, (n + 1,)).copy()
         self.span_stride = w = int(res.span_stride)
@@ -291,12 +345,13 @@ class Gorp:
         finally:
             lib.gorp_result_release(self._eng(), C.byref(res))
 
-    def extract_batch_lines_utf8(self, lines, offsets=None) -> ExtractionBatch:
+    def extract_batch_lines_utf8(self, lines, offsets=None, tables=False) -> ExtractionBatch:
         """extract_batch_lines for strings held as UTF-8 bytes (gorp_extract_lines_utf8, all of the engine's devices): a '\\n'
         inside a string is data. `lines` is a sequence of bytes / str (str is UTF-8-encoded), or with `offsets` a bytes-like
         buffer in which string i is bytes [offsets[i], offsets[i+1]) (int64; offsets[0] may be > 0, as in an Arrow slice).
         line_off and spans are byte offsets into that buffer; the batch decodes only what a line(), spans_of() or result()
-        asks for. A string that is not well-formed UTF-8 on its own raises ValueError."""
+        asks for. A string that is not well-formed UTF-8 on its own raises ValueError. tables=True: the batch also holds the
+        values as one ValueTable per extraction (`.tables`, gorp_extract_lines_utf8_tables)."""
         if offsets is None:
             parts = [s.encode("utf-8") if isinstance(s, str) else bytes(s) for s in lines]
             off = np.zeros(len(parts) + 1, dtype=np.int64)
@@ -311,10 +366,13 @@ class Gorp:
                 raise ValueError("offsets must hold n_lines + 1 entries")
             if int(off[-1]) > len(b):
                 raise ValueError("offsets reach past the end of the buffer")
-        res = _ffi.Result()
-        _check(lib.gorp_extract_lines_utf8(self._eng(), b.ctypes.data, off.ctypes.data, len(off) - 1, C.byref(res)))
+        res, dt = _ffi.Result(), _ffi.DeviceTables() if tables else None
+        if tables:
+            _check(lib.gorp_extract_lines_utf8_tables(self._eng(), b.ctypes.data, off.ctypes.data, len(off) - 1, C.byref(res), C.byref(dt)))
+        else:
+            _check(lib.gorp_extract_lines_utf8(self._eng(), b.ctypes.data, off.ctypes.data, len(off) - 1, C.byref(res)))
         try:
-            return ExtractionBatch(self, b, res, 0, encoding="utf-8")
+            return ExtractionBatch(self, b, res, 0, encoding="utf-8", tables=dt)
         finally:
             lib.gorp_result_release(self._eng(), C.byref(res))
 
@@ -339,17 +397,25 @@ class Gorp:
         finally:
             lib.gorp_result_release(self._eng(), C.byref(res))
 
-    def extract_batch_text_utf8(self, data, byte_offsets=False) -> ExtractionBatch:
+    def extract_batch_text_utf8(self, data, byte_offsets=False, tables=False) -> ExtractionBatch:
         """'\n'-separated text held as UTF-8 bytes (a log file as it is on disk): decoded to UTF-16 on the device, results are
         those of extract_batch_text on the decoded text (offsets in UTF-16 units). Malformed UTF-8 raises ValueError.
         byte_offsets=True: line_off and spans are byte offsets into `data` (gorp_extract_text_utf8_bytes, all of the engine's
-        devices); the batch slices `data` and decodes only what a line(), spans_of() or result() asks for."""
+        devices); the batch slices `data` and decodes only what a line(), spans_of() or result() asks for. tables=True (with
+        byte_offsets only): the batch also holds the values as one ValueTable per extraction (`.tables`,
+        gorp_extract_text_utf8_tables)."""
+        if tables and not byte_offsets:
+            raise ValueError("tables=True needs byte_offsets=True: the tables hold bytes of `data`")
         b = np.ascontiguousarray(np.frombuffer(data, dtype=np.uint8) if isinstance(data, (bytes, bytearray)) else data, dtype=np.uint8)
         res = _ffi.Result()
         if byte_offsets:
-            _check(lib.gorp_extract_text_utf8_bytes(self._eng(), b.ctypes.data, len(b), C.byref(res)))
+            dt = _ffi.DeviceTables() if tables else None
+            if tables:
+                _check(lib.gorp_extract_text_utf8_tables(self._eng(), b.ctypes.data, len(b), C.byref(res), C.byref(dt)))
+            else:
+                _check(lib.gorp_extract_text_utf8_bytes(self._eng(), b.ctypes.data, len(b), C.byref(res)))
             try:
-                return ExtractionBatch(self, b, res, 1, encoding="utf-8")
+                return ExtractionBatch(self, b, res, 1, encoding="utf-8", tables=dt)
             finally:
                 lib.gorp_result_release(self._eng(), C.byref(res))
         _check(lib.gorp_extract_text_utf8(self._eng(), b.ctypes.data, len(b), C.byref(res)))

@@ -120,6 +120,41 @@ T* upload(const std::vector<T>& v, std::vector<void*>& owned) {
     return static_cast<T*>(p);
 }
 
+// The host descriptors of a gorp_device_tables: one gorp_value_table per extraction, and per column (of all tables, in
+// table order) the pointers and null count the tables point into.
+struct TableDescs {
+    std::vector<gorp_value_table> tables;
+    std::vector<const int64_t*> offsets;
+    std::vector<const void*> data;
+    std::vector<const uint8_t*> valid;
+    std::vector<int64_t> nulls;
+    void reset(size_t n_tables, int64_t n_cols) {
+        tables.assign(n_tables, gorp_value_table{});
+        offsets.assign(static_cast<size_t>(n_cols), nullptr);
+        data.assign(static_cast<size_t>(n_cols), nullptr);
+        valid.assign(static_cast<size_t>(n_cols), nullptr);
+        nulls.assign(static_cast<size_t>(n_cols), 0);
+    }
+    // table t: columns [col_base, col_base + n_cols) of the column arrays
+    void set_table(size_t t, int64_t n_rows, const int64_t* rows, int64_t col_base, int64_t n_cols) {
+        gorp_value_table& v = tables[t];
+        v.n_rows = n_rows;
+        v.n_columns = static_cast<int32_t>(n_cols);
+        v.d_row = rows;
+        if (n_cols) {
+            v.d_offsets = offsets.data() + col_base;
+            v.d_data = data.data() + col_base;
+            v.d_valid = valid.data() + col_base;
+            v.null_count = nulls.data() + col_base;
+        }
+    }
+    void describe(gorp_device_tables* out, int unit_bytes) const {
+        out->n_tables = static_cast<int32_t>(tables.size());
+        out->unit_bytes = unit_bytes;
+        out->tables = tables.data();
+    }
+};
+
 constexpr int kMaxTimed = 16;
 struct DeviceCtx {
     int device = 0;
@@ -171,11 +206,10 @@ struct DeviceCtx {
     gorp_device_result last{};
     // value tables of gorp_extract_tables_device: device buffers, and the host descriptors the caller reads
     DevBuf tb_counts, tb_starts, tb_scan, tb_layout, tb_rows, tb_lens, tb_valid, tb_stats, tb_offs, tb_colinfo, tb_data;
-    std::vector<gorp_value_table> tb_tables;
-    std::vector<const int64_t*> tb_off_ptr;
-    std::vector<const void*> tb_data_ptr;
-    std::vector<const uint8_t*> tb_valid_ptr;
-    std::vector<int64_t> tb_nulls;
+    TableDescs tb_desc;
+    // tables of the UTF-8 host calls: the device's whole byte range [R0, R1) of the batch, the merge jobs and the shifted
+    // bitmaps of a call on several devices
+    DevBuf resident, tb_jobs, tb_stage;
     // per-kernel device time: CUDA events on the launching stream, accumulated over timed calls
     cudaEvent_t ev[kMaxTimed + 1]{};
     const char* ev_name[kMaxTimed]{};
@@ -248,10 +282,13 @@ struct NumaPrefer {
     }
 };
 
-struct HostResult {  // pinned host arrays behind a gorp_result
+// Pinned host arrays behind a gorp_result: 0-3 ext_id, line_off, spans, histogram; with value tables (the *_tables calls)
+// 4-7 row indexes, offsets, values and bitmaps of every table, described by `tables`.
+struct HostResult {
     int numa_node = -1;  // of the device that fills the arrays (first device of the engine)
-    void* p[4] = {nullptr, nullptr, nullptr, nullptr};
-    size_t cap[4] = {0, 0, 0, 0};
+    void* p[8] = {};
+    size_t cap[8] = {};
+    TableDescs tables;
     void reserve(int i, size_t bytes, size_t keep = 0) {  // keeps the first `keep` bytes when it has to grow
         if (bytes <= cap[i]) return;
         void* q = nullptr;
@@ -1126,8 +1163,10 @@ struct DeviceRun {  // what one device produced for its pieces
 // caller's strings are bytes [off[i], off[i+1]) of `text8`; the piece is decoded at textbuf + kTextPad, its strings' unit
 // offsets (relative to the piece) feed the lines form of the pipeline, and the rows go back to the caller's byte offsets.
 // The caller holds c.mu (a multi-device call keeps every participating device locked until its rows are copied out).
+// `keep_bytes` (UTF-8 in byte coordinates, for the value tables): the staged bytes of every piece are also copied to
+// c.resident, which then holds bytes [pieces[p0].u0, pieces[p1 - 1].u1) of `text8`.
 void run_pieces(gorp_engine* e, DeviceCtx& c, const uint16_t* text, const uint8_t* text8, bool utf8, bool byte_coords, const int64_t* off,
-                const std::vector<Piece>& pieces, size_t p0, size_t p1, HostResult* hr, DeviceRun& run) {
+                const std::vector<Piece>& pieces, size_t p0, size_t p1, HostResult* hr, DeviceRun& run, bool keep_bytes = false) {
     CK(cudaSetDevice(c.device));
     // a device-resident call on another stream may still use the scratch: the kernels wait for it, and so do the staging
     // copies (the UTF-8 device calls decode into textbuf[0] and stage into bytebuf[0], which the first piece's copy overwrites)
@@ -1151,6 +1190,7 @@ void run_pieces(gorp_engine* e, DeviceCtx& c, const uint16_t* text, const uint8_
         if (text8) c.bytebuf[b].reserve(max_units + 64);
         if (off) c.offbuf[b].reserve((max_lines + 1) * 8);
     }
+    if (keep_bytes) c.resident.reserve(static_cast<size_t>(units_total) + 64);
     if (off && utf8) {
         c.unit_off.reserve((max_lines + 1) * 8);
         c.slice_units.reserve((max_units / 16 + 1) * 2);
@@ -1197,6 +1237,9 @@ void run_pieces(gorp_engine* e, DeviceCtx& c, const uint16_t* text, const uint8_
         if (k + 1 < p1) stage(k + 1);  // the other buffer: its previous piece was computed (this thread waited for it)
         CK(cudaStreamWaitEvent(c.stream, c.ev_in[b], 0));
         const int64_t units = pc.u1 - pc.u0;
+        if (keep_bytes && units)
+            CK(cudaMemcpyAsync(c.resident.as<uint8_t>() + (pc.u0 - pieces[p0].u0), c.bytebuf[b].p, static_cast<size_t>(units), cudaMemcpyDeviceToDevice,
+                               c.stream));
         int64_t piece_bias = pc.u0;  // what turns the piece's line offsets into offsets of the whole batch
         gorp_device_result dr{};
         int64_t nl;
@@ -1275,8 +1318,223 @@ void run_pieces(gorp_engine* e, DeviceCtx& c, const uint16_t* text, const uint8_
     run.stride = static_cast<int32_t>(stride);
 }
 
+// Host copy of the layout that build_tables leaves in c.tb_*.
+struct TablesBuilt {
+    std::vector<TableLayout> lay;   // [E + 1]; entry E holds the totals
+    std::vector<int64_t> stats;     // [2 * columns]: value units, nulls
+    std::vector<int64_t> col_info;  // [2 * columns + 2]: first entry of the column in the offset scan, byte offset of its data
+    int64_t n_cols = 0;
+};
+
+// The value tables (kernels/tables.cu, DESIGN.md §5.5) of rows `r` of context c, values read from `text` (unit_bytes per
+// unit) at line_off + span: row indexes in c.tb_rows, offsets in c.tb_offs (from 0 in every column), values in c.tb_data,
+// bitmaps in c.tb_valid, positions in `b`. Four stages on `st`, one host round trip (the per-column totals size the values).
+void build_tables(gorp_engine* e, DeviceCtx& c, cudaStream_t st, Timer& tm, const gorp_device_result& r, const void* text, int ub,
+                  TablesBuilt& b) {
+    Launch L{st, c.sm_count};
+    const uint32_t E = c.n_ext;
+    const int64_t n = r.n_lines;
+    const uint32_t stride = static_cast<uint32_t>(r.span_stride);
+    int64_t n_cols = 0;  // columns of all tables
+    for (const auto& x : e->def.extractions) n_cols += stride ? x.n_groups : 0;
+    // 1. rank: stable partition of the matched lines by extraction
+    const int64_t tile = tables_tile_lines(E), n_tiles = std::max<int64_t>(1, (n + tile - 1) / tile), cells = n_tiles * E;
+    c.tb_counts.reserve(static_cast<size_t>(cells) * 4 + 64);
+    c.tb_starts.reserve(static_cast<size_t>(cells + 1) * 8 + 64);
+    c.tb_layout.reserve((E + 1) * sizeof(TableLayout));
+    c.tb_rows.reserve(static_cast<size_t>(n + 8 * E + 8) * 8);
+    c.tb_stats.reserve(static_cast<size_t>(n_cols) * 16 + 64);
+    TableLayout* lay = c.tb_layout.as<TableLayout>();
+    k_tables_count(L, r.d_ext_id, n, E, tile, n_tiles, c.tb_counts.as<uint32_t>());
+    c.tb_scan.reserve(static_cast<size_t>(cells / 4096 + 8) * 8);
+    scan_u32_to_i64(L, c.tb_counts.as<uint32_t>(), cells, c.tb_starts.as<int64_t>(), c.tb_scan.as<int64_t>());
+    k_tables_layout(L, c.tb_starts.as<int64_t>(), n_tiles, E, c.d_slots, stride != 0, lay);
+    k_tables_scatter(L, r.d_ext_id, n, E, tile, n_tiles, c.tb_starts.as<int64_t>(), lay, c.tb_rows.as<int64_t>());
+    CK(cudaGetLastError());
+    tm.mark("tables_rank", 6);
+    // 2. lengths, validity, per-column totals and null counts (sized for every line in the widest extraction)
+    const int64_t slots_ub = n * (stride / 2) + 8 * n_cols + 8, words_ub = n * (stride / 2) / 32 + 17 * n_cols + 16;
+    c.tb_lens.reserve(static_cast<size_t>(slots_ub) * 4);
+    c.tb_valid.reserve(static_cast<size_t>(words_ub) * 4);
+    CK(cudaMemsetAsync(c.tb_valid.p, 0, static_cast<size_t>(words_ub) * 4, st));
+    if (n_cols) CK(cudaMemsetAsync(c.tb_stats.p, 0, static_cast<size_t>(n_cols) * 16, st));
+    k_tables_len(L, lay, E, c.tb_rows.as<int64_t>(), r.d_spans, stride, c.tb_lens.as<uint32_t>(), c.tb_valid.as<uint32_t>(),
+                 c.tb_stats.as<unsigned long long>());
+    CK(cudaGetLastError());
+    tm.mark("tables_len", 1);
+    // the one round trip: the layout and the column totals
+    b.lay.assign(E + 1, TableLayout{});
+    b.stats.assign(static_cast<size_t>(n_cols) * 2, 0);
+    CK(cudaMemcpyAsync(b.lay.data(), lay, (E + 1) * sizeof(TableLayout), cudaMemcpyDeviceToHost, st));
+    if (n_cols) CK(cudaMemcpyAsync(b.stats.data(), c.tb_stats.p, b.stats.size() * 8, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    if (b.lay[E].col_base != n_cols) throw std::runtime_error("value tables: column count mismatch");
+    // 3. offsets: one scan over the lengths of every column; 4. gather into 64-byte aligned columns
+    const int64_t n_off = b.lay[E].off_base;
+    b.n_cols = n_cols;
+    b.col_info.assign(static_cast<size_t>(n_cols) * 2 + 2, 0);
+    int64_t flat = 0, data_bytes = 0;
+    for (int64_t k = 0; k < n_cols; ++k) {
+        b.col_info[2 * k] = flat;
+        b.col_info[2 * k + 1] = data_bytes;
+        flat += b.stats[2 * k];
+        data_bytes += (b.stats[2 * k] * ub + 63) / 64 * 64;
+    }
+    c.tb_offs.reserve(static_cast<size_t>(n_off + 1) * 8 + 64);
+    c.tb_scan.reserve(static_cast<size_t>(n_off / 4096 + 8) * 8);
+    scan_u32_to_i64(L, c.tb_lens.as<uint32_t>(), n_off, c.tb_offs.as<int64_t>(), c.tb_scan.as<int64_t>());
+    CK(cudaGetLastError());
+    tm.mark("tables_scan", 3);
+    c.tb_colinfo.reserve(b.col_info.size() * 8);
+    // (pageable: the copy has been staged by the time cudaMemcpyAsync returns)
+    CK(cudaMemcpyAsync(c.tb_colinfo.p, b.col_info.data(), b.col_info.size() * 8, cudaMemcpyHostToDevice, st));
+    c.tb_data.reserve(static_cast<size_t>(data_bytes) + 64);
+    k_tables_gather(L, lay, E, c.tb_rows.as<int64_t>(), r.d_line_off, r.d_spans, stride, text, ub, c.tb_lens.as<uint32_t>(),
+                    c.tb_offs.as<int64_t>(), c.tb_colinfo.as<int64_t>(), c.tb_data.as<uint8_t>());
+    CK(cudaGetLastError());
+    tm.mark("tables_gather", 1);
+}
+
+// The tables of a UTF-8 host call in pinned memory of hr: device d < G built the tables of its rows (bt[d], lines
+// [base[d], base[d + 1]) of the result); table e takes device d's rows after those of the devices before it. On one device
+// the buffers are copied as they are. On several, device d first adds its line base to its row indexes and the column's
+// value base to its offsets, and moves its bitmaps to the bit position of its first row (k_tables_rebase); where that
+// position is not a multiple of 8, the first byte is ORed into the byte the previous device wrote, here on the host. The
+// copies of all devices run at once; returns when they are done.
+void merge_tables(gorp_engine* e, size_t G, const std::vector<TablesBuilt>& bt, const std::vector<int64_t>& base, HostResult& hr) {
+    const size_t E = e->def.extractions.size();
+    const int64_t n_cols = bt[0].n_cols;
+    auto up64 = [](int64_t x) { return (x + 63) / 64 * 64; };
+    // positions in the host buffers (bytes) and every device's row and value bases
+    std::vector<int64_t> n_rows(E, 0), row_at(E), col_rows(static_cast<size_t>(n_cols)), off_at(static_cast<size_t>(n_cols)),
+        data_at(static_cast<size_t>(n_cols)), valid_at(static_cast<size_t>(n_cols)), values(static_cast<size_t>(n_cols), 0),
+        nulls(static_cast<size_t>(n_cols), 0);
+    std::vector<int64_t> row_base(G * E), value_base(G * static_cast<size_t>(n_cols));
+    for (size_t d = 0; d < G; ++d)
+        for (size_t t = 0; t < E; ++t) {
+            row_base[d * E + t] = n_rows[t];
+            n_rows[t] += bt[d].lay[t].n_rows;
+        }
+    for (size_t d = 0; d < G; ++d)
+        for (int64_t k = 0; k < n_cols; ++k) {
+            value_base[d * n_cols + k] = values[k];
+            values[k] += bt[d].stats[2 * k];
+            nulls[k] += bt[d].stats[2 * k + 1];
+        }
+    int64_t rows_bytes = 0, off_bytes = 0, data_bytes = 0, valid_bytes = 0;
+    for (size_t t = 0; t < E; ++t) {
+        row_at[t] = rows_bytes;
+        rows_bytes += up64(n_rows[t] * 8);
+        const TableLayout& x = bt[0].lay[t];
+        for (int64_t k = x.col_base; k < x.col_base + x.n_cols; ++k) {
+            col_rows[k] = n_rows[t];
+            off_at[k] = off_bytes;
+            off_bytes += up64((n_rows[t] + 1) * 8);
+            data_at[k] = data_bytes;
+            data_bytes += up64(values[k]);
+            valid_at[k] = valid_bytes;
+            valid_bytes += up64((n_rows[t] + 7) / 8);
+        }
+    }
+    // (behind the bitmaps: the first byte of every device's shifted bitmaps, ORed in below)
+    const int64_t side_at = valid_bytes;
+    hr.reserve(4, static_cast<size_t>(rows_bytes) + 64);
+    hr.reserve(5, static_cast<size_t>(off_bytes) + 64);
+    hr.reserve(6, static_cast<size_t>(data_bytes) + 64);
+    hr.reserve(7, static_cast<size_t>(valid_bytes + static_cast<int64_t>(G) * n_cols) + 64);
+    uint8_t* h_rows = static_cast<uint8_t*>(hr.p[4]);
+    uint8_t* h_off = static_cast<uint8_t*>(hr.p[5]);
+    uint8_t* h_data = static_cast<uint8_t*>(hr.p[6]);
+    uint8_t* h_valid = static_cast<uint8_t*>(hr.p[7]);
+    for (size_t d = 0; d < G; ++d) {
+        DeviceCtx& c = *e->devs[d];
+        CK(cudaSetDevice(c.device));
+        const TablesBuilt& b = bt[d];
+        auto dev_rows = [&](size_t t) { return c.tb_rows.as<int64_t>() + b.lay[t].row_base; };
+        auto dev_off = [&](size_t t, int64_t k) { return c.tb_offs.as<int64_t>() + b.lay[t].off_base + (k - b.lay[t].col_base) * b.lay[t].seg; };
+        auto dev_valid = [&](size_t t, int64_t k) {
+            return reinterpret_cast<uint8_t*>(c.tb_valid.as<uint32_t>() + b.lay[t].valid_base + (k - b.lay[t].col_base) * b.lay[t].vwords);
+        };
+        // the rebase: row indexes and offsets in place, bitmaps into tb_stage
+        std::vector<RebaseJob> jobs;
+        std::vector<int64_t> stage_at(static_cast<size_t>(n_cols), -1);
+        int64_t blocks = 0, stage_bytes = 0;
+        auto add_job = [&](RebaseJob j) {
+            j.first_block = blocks;
+            blocks += tables_rebase_blocks(j);
+            jobs.push_back(j);
+        };
+        for (size_t t = 0; t < E; ++t) {
+            const TableLayout& x = b.lay[t];
+            const int64_t rb = row_base[d * E + t];
+            if (x.n_rows && base[d]) add_job({dev_rows(t), dev_rows(t), x.n_rows, base[d], 0, 0});
+            for (int64_t k = x.col_base; k < x.col_base + x.n_cols; ++k) {
+                if (value_base[d * n_cols + k]) add_job({dev_off(t, k), dev_off(t, k), x.n_rows + 1, value_base[d * n_cols + k], 0, 0});
+                if (x.n_rows && rb % 8) {
+                    stage_at[k] = stage_bytes;
+                    stage_bytes += up64((x.n_rows + rb % 8 + 7) / 8);
+                }
+            }
+        }
+        c.tb_stage.reserve(static_cast<size_t>(stage_bytes) + 64);
+        for (size_t t = 0; t < E; ++t)
+            for (int64_t k = b.lay[t].col_base; k < b.lay[t].col_base + b.lay[t].n_cols; ++k)
+                if (stage_at[k] >= 0)
+                    add_job({dev_valid(t, k), c.tb_stage.as<uint8_t>() + stage_at[k], b.lay[t].n_rows, 0, row_base[d * E + t] % 8, 0});
+        if (!jobs.empty()) {
+            c.tb_jobs.reserve(jobs.size() * sizeof(RebaseJob));
+            CK(cudaMemcpyAsync(c.tb_jobs.p, jobs.data(), jobs.size() * sizeof(RebaseJob), cudaMemcpyHostToDevice, c.stream));  // (pageable)
+            k_tables_rebase(Launch{c.stream, c.sm_count}, c.tb_jobs.as<RebaseJob>(), static_cast<uint32_t>(jobs.size()), blocks);
+            CK(cudaGetLastError());
+            c.launches += 1;
+        }
+        // the copies to the host buffers
+        auto d2h = [&](void* dst, const void* src, int64_t bytes) {
+            if (bytes > 0) CK(cudaMemcpyAsync(dst, src, static_cast<size_t>(bytes), cudaMemcpyDeviceToHost, c.stream));
+        };
+        for (size_t t = 0; t < E; ++t) {
+            const TableLayout& x = b.lay[t];
+            const int64_t rb = row_base[d * E + t];
+            d2h(h_rows + row_at[t] + rb * 8, dev_rows(t), x.n_rows * 8);
+            for (int64_t k = x.col_base; k < x.col_base + x.n_cols; ++k) {
+                // offsets: entries [rb, rb + n) (the last device also the closing entry); values; bitmaps
+                d2h(h_off + off_at[k] + rb * 8, dev_off(t, k), (x.n_rows + (d + 1 == G ? 1 : 0)) * 8);
+                d2h(h_data + data_at[k] + value_base[d * n_cols + k], c.tb_data.as<uint8_t>() + b.col_info[2 * k + 1], b.stats[2 * k]);
+                if (stage_at[k] < 0) {
+                    d2h(h_valid + valid_at[k] + rb / 8, dev_valid(t, k), (x.n_rows + 7) / 8);
+                } else {
+                    const uint8_t* s = c.tb_stage.as<uint8_t>() + stage_at[k];
+                    d2h(h_valid + side_at + d * n_cols + k, s, 1);
+                    d2h(h_valid + valid_at[k] + rb / 8 + 1, s + 1, (x.n_rows + rb % 8 + 7) / 8 - 1);
+                }
+            }
+        }
+    }
+    for (size_t d = 0; d < G; ++d) {
+        CK(cudaSetDevice(e->devs[d]->device));
+        CK(cudaStreamSynchronize(e->devs[d]->stream));
+        CK(cudaEventRecord(e->devs[d]->ev_done, e->devs[d]->stream));
+    }
+    hr.tables.reset(E, n_cols);
+    for (size_t t = 0; t < E; ++t) {
+        const TableLayout& x = bt[0].lay[t];
+        for (int64_t k = x.col_base; k < x.col_base + x.n_cols; ++k) {
+            uint8_t* v = h_valid + valid_at[k];
+            for (size_t d = 1; d < G; ++d)
+                if (bt[d].lay[t].n_rows && row_base[d * E + t] % 8) v[row_base[d * E + t] / 8] |= h_valid[side_at + d * n_cols + k];
+            const int64_t used = (n_rows[t] + 7) / 8;
+            std::memset(v + used, 0, static_cast<size_t>(up64(used) - used));
+            hr.tables.offsets[k] = reinterpret_cast<const int64_t*>(h_off + off_at[k]);
+            hr.tables.data[k] = h_data + data_at[k];
+            hr.tables.valid[k] = v;
+            hr.tables.nulls[k] = nulls[k];
+        }
+        hr.tables.set_table(t, n_rows[t], reinterpret_cast<const int64_t*>(h_rows + row_at[t]), x.col_base, x.n_cols);
+    }
+}
+
 int extract_host(gorp_engine* e, const uint16_t* text, const uint8_t* text8, int64_t n_units, const int64_t* off, int64_t n_lines,
-                 gorp_result* out, bool utf8 = false, bool byte_coords = false) {
+                 gorp_result* out, bool utf8 = false, bool byte_coords = false, gorp_device_tables* tables = nullptr) {
     if (!e || !out || (!text && !text8 && n_units > 0) || n_units < 0 || n_lines < 0) return fail(GORP_E_ARG, "bad argument");
     if (e->devs.empty()) return fail(GORP_E_CUDA, "engine has no CUDA device");
     return guarded([&]() -> int {
@@ -1307,12 +1565,28 @@ int extract_host(gorp_engine* e, const uint16_t* text, const uint8_t* text8, int
         int64_t nl = 0;
         int32_t stride = 0;
         DeviceGuard restore_device;
+        // value tables (UTF-8 in byte coordinates): every device builds the tables of its rows over its resident bytes
+        auto device_tables = [&](DeviceCtx& c, const DeviceRun& run, size_t p0, TablesBuilt& b) {
+            gorp_device_result r{};
+            r.n_lines = run.n_rows;
+            r.span_stride = run.stride;
+            r.d_ext_id = c.acc_ext.as<int32_t>();
+            r.d_line_off = c.acc_off.as<int64_t>();
+            r.d_spans = c.acc_spans.as<int32_t>();
+            Timer tm(c, c.stream, false);  // (untimed: counts the launches)
+            build_tables(e, c, c.stream, tm, r, c.resident.as<uint8_t>() - pieces[p0].u0, 1, b);
+        };
         if (G <= 1) {
             DeviceRun run;
             CtxLock lock(*e->devs[0]);
-            run_pieces(e, *e->devs[0], text, text8, utf8, byte_coords, off, pieces, 0, pieces.size(), hr.get(), run);
+            run_pieces(e, *e->devs[0], text, text8, utf8, byte_coords, off, pieces, 0, pieces.size(), hr.get(), run, tables != nullptr);
             nl = run.n_rows;
             stride = run.stride;
+            if (tables) {
+                std::vector<TablesBuilt> bt(1);
+                device_tables(*e->devs[0], run, 0, bt[0]);
+                merge_tables(e, 1, bt, {0}, *hr);
+            }
         } else {
             // contiguous ranges of pieces per device (lines shard as contiguous ranges: no data crosses devices); one
             // host thread per device; the rows are copied out once every device's row base is known
@@ -1321,13 +1595,16 @@ int extract_host(gorp_engine* e, const uint16_t* text, const uint8_t* text8, int
             std::vector<CtxLock> locks;
             for (size_t d = 0; d < G; ++d) locks.emplace_back(*e->devs[d]);
             std::vector<DeviceRun> runs(G);
+            std::vector<TablesBuilt> bt(tables ? G : 0);
             std::vector<size_t> first(G + 1);
             for (size_t d = 0; d <= G; ++d) first[d] = pieces.size() * d / G;
             std::vector<std::thread> th;
             for (size_t d = 0; d < G; ++d)
                 th.emplace_back([&, d]() {
                     runs[d].status = guarded([&]() -> int {
-                        run_pieces(e, *e->devs[d], text, text8, utf8, byte_coords, off, pieces, first[d], first[d + 1], nullptr, runs[d]);
+                        run_pieces(e, *e->devs[d], text, text8, utf8, byte_coords, off, pieces, first[d], first[d + 1], nullptr, runs[d],
+                                   tables != nullptr);
+                        if (tables) device_tables(*e->devs[d], runs[d], first[d], bt[d]);
                         return GORP_OK;
                     });
                     if (runs[d].status != GORP_OK) runs[d].error = g_error;
@@ -1356,6 +1633,7 @@ int extract_host(gorp_engine* e, const uint16_t* text, const uint8_t* text8, int
                                        cudaMemcpyDeviceToHost, c.stream));
                 CK(cudaMemcpyAsync(hist.data() + d * E2, c.acc_hist.p, E2 * 8, cudaMemcpyDeviceToHost, c.stream));
             }
+            if (tables) merge_tables(e, G, bt, base, *hr);  // (its copies run alongside those of the rows)
             for (size_t d = 0; d < G; ++d) {
                 CK(cudaSetDevice(e->devs[d]->device));
                 CK(cudaStreamSynchronize(e->devs[d]->stream));
@@ -1373,6 +1651,7 @@ int extract_host(gorp_engine* e, const uint16_t* text, const uint8_t* text8, int
         out->line_off = static_cast<const int64_t*>(hr->p[1]);
         out->spans = static_cast<const int32_t*>(hr->p[2]);
         out->histogram = static_cast<const int64_t*>(hr->p[3]);
+        if (tables) hr->tables.describe(tables, 1);
         out->owner = hr.release();
         return GORP_OK;
     });
@@ -1666,12 +1945,28 @@ int gorp_extract_text_utf8_bytes(gorp_engine* e, const uint8_t* text, int64_t n_
     return extract_host(e, nullptr, text, n_bytes, nullptr, 0, out, true, true);
 }
 
-int gorp_extract_lines_utf8(gorp_engine* e, const uint8_t* text, const int64_t* off, int64_t n_lines, gorp_result* out) {
+static int extract_lines_utf8(gorp_engine* e, const uint8_t* text, const int64_t* off, int64_t n_lines, gorp_result* out,
+                              gorp_device_tables* tables) {
     if (!e || !out || !off || n_lines < 0) return fail(GORP_E_ARG, "bad argument");
     if (off[0] < 0) return fail(GORP_E_ARG, "offsets must start at >= 0");
     if (const int64_t i = first_decreasing_offset(off, n_lines); i >= 0)
         return fail(GORP_E_ARG, strfmt("offsets must be non-decreasing (line %lld)", static_cast<long long>(i)));
-    return extract_host(e, nullptr, text, n_lines > 0 ? off[n_lines] : 0, off, n_lines, out, true, true);
+    return extract_host(e, nullptr, text, n_lines > 0 ? off[n_lines] : 0, off, n_lines, out, true, true, tables);
+}
+
+int gorp_extract_lines_utf8(gorp_engine* e, const uint8_t* text, const int64_t* off, int64_t n_lines, gorp_result* out) {
+    return extract_lines_utf8(e, text, off, n_lines, out, nullptr);
+}
+
+int gorp_extract_text_utf8_tables(gorp_engine* e, const uint8_t* text, int64_t n_bytes, gorp_result* out, gorp_device_tables* tables) {
+    if (!tables) return fail(GORP_E_ARG, "bad argument");
+    return extract_host(e, nullptr, text, n_bytes, nullptr, 0, out, true, true, tables);
+}
+
+int gorp_extract_lines_utf8_tables(gorp_engine* e, const uint8_t* text, const int64_t* off, int64_t n_lines, gorp_result* out,
+                                   gorp_device_tables* tables) {
+    if (!tables) return fail(GORP_E_ARG, "bad argument");
+    return extract_lines_utf8(e, text, off, n_lines, out, tables);
 }
 
 int gorp_match_all_lines(gorp_engine* e, const uint16_t* text, const int64_t* off, int64_t n_lines, gorp_match_result* out) {
@@ -1895,98 +2190,22 @@ int gorp_extract_tables_device(gorp_engine* e, int dev_index, void* stream, int 
         CK(cudaSetDevice(c.device));
         cudaStream_t st = static_cast<cudaStream_t>(stream);
         CK(cudaStreamWaitEvent(st, c.ev_done, 0));  // the previous call on this context (any stream) used the same scratch
-        Launch L{st, c.sm_count};
         Timer tm(c, st, (flags & GORP_FLAG_TIME_KERNELS) != 0);
-        const gorp_device_result& r = c.last;
-        const uint32_t E = c.n_ext;
-        const int64_t n = r.n_lines;
-        const uint32_t stride = static_cast<uint32_t>(r.span_stride);
-        int64_t n_cols = 0;  // columns of all tables
-        for (const auto& x : e->def.extractions) n_cols += stride ? x.n_groups : 0;
-        // 1. rank: stable partition of the matched lines by extraction
-        const int64_t tile = tables_tile_lines(E), n_tiles = std::max<int64_t>(1, (n + tile - 1) / tile), cells = n_tiles * E;
-        c.tb_counts.reserve(static_cast<size_t>(cells) * 4 + 64);
-        c.tb_starts.reserve(static_cast<size_t>(cells + 1) * 8 + 64);
-        c.tb_layout.reserve((E + 1) * sizeof(TableLayout));
-        c.tb_rows.reserve(static_cast<size_t>(n + 8 * E + 8) * 8);
-        c.tb_stats.reserve(static_cast<size_t>(n_cols) * 16 + 64);
-        TableLayout* lay = c.tb_layout.as<TableLayout>();
-        k_tables_count(L, r.d_ext_id, n, E, tile, n_tiles, c.tb_counts.as<uint32_t>());
-        c.tb_scan.reserve(static_cast<size_t>(cells / 4096 + 8) * 8);
-        scan_u32_to_i64(L, c.tb_counts.as<uint32_t>(), cells, c.tb_starts.as<int64_t>(), c.tb_scan.as<int64_t>());
-        k_tables_layout(L, c.tb_starts.as<int64_t>(), n_tiles, E, c.d_slots, stride != 0, lay);
-        k_tables_scatter(L, r.d_ext_id, n, E, tile, n_tiles, c.tb_starts.as<int64_t>(), lay, c.tb_rows.as<int64_t>());
-        CK(cudaGetLastError());
-        tm.mark("tables_rank", 6);
-        // 2. lengths, validity, per-column totals and null counts (sized for every line in the widest extraction)
-        const int64_t slots_ub = n * (stride / 2) + 8 * n_cols + 8, words_ub = n * (stride / 2) / 32 + 17 * n_cols + 16;
-        c.tb_lens.reserve(static_cast<size_t>(slots_ub) * 4);
-        c.tb_valid.reserve(static_cast<size_t>(words_ub) * 4);
-        CK(cudaMemsetAsync(c.tb_valid.p, 0, static_cast<size_t>(words_ub) * 4, st));
-        if (n_cols) CK(cudaMemsetAsync(c.tb_stats.p, 0, static_cast<size_t>(n_cols) * 16, st));
-        k_tables_len(L, lay, E, c.tb_rows.as<int64_t>(), r.d_spans, stride, c.tb_lens.as<uint32_t>(), c.tb_valid.as<uint32_t>(),
-                     c.tb_stats.as<unsigned long long>());
-        CK(cudaGetLastError());
-        tm.mark("tables_len", 1);
-        // the one round trip: the layout and the column totals
-        std::vector<TableLayout> h_lay(E + 1);
-        std::vector<int64_t> h_stats(static_cast<size_t>(n_cols) * 2);
-        CK(cudaMemcpyAsync(h_lay.data(), lay, (E + 1) * sizeof(TableLayout), cudaMemcpyDeviceToHost, st));
-        if (n_cols) CK(cudaMemcpyAsync(h_stats.data(), c.tb_stats.p, h_stats.size() * 8, cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-        if (h_lay[E].col_base != n_cols) throw std::runtime_error("value tables: column count mismatch");
-        // 3. offsets: one scan over the lengths of every column; 4. gather into 64-byte aligned columns
-        const int64_t n_off = h_lay[E].off_base;
-        const int ub = c.last_unit_bytes;
-        std::vector<int64_t> col_info(static_cast<size_t>(n_cols) * 2 + 2);
-        int64_t flat = 0, data_bytes = 0;
-        for (int64_t k = 0; k < n_cols; ++k) {
-            col_info[2 * k] = flat;
-            col_info[2 * k + 1] = data_bytes;
-            flat += h_stats[2 * k];
-            data_bytes += (h_stats[2 * k] * ub + 63) / 64 * 64;
-        }
-        c.tb_offs.reserve(static_cast<size_t>(n_off + 1) * 8 + 64);
-        c.tb_scan.reserve(static_cast<size_t>(n_off / 4096 + 8) * 8);
-        scan_u32_to_i64(L, c.tb_lens.as<uint32_t>(), n_off, c.tb_offs.as<int64_t>(), c.tb_scan.as<int64_t>());
-        CK(cudaGetLastError());
-        tm.mark("tables_scan", 3);
-        c.tb_colinfo.reserve(col_info.size() * 8);
-        CK(cudaMemcpyAsync(c.tb_colinfo.p, col_info.data(), col_info.size() * 8, cudaMemcpyHostToDevice, st));
-        c.tb_data.reserve(static_cast<size_t>(data_bytes) + 64);
-        k_tables_gather(L, lay, E, c.tb_rows.as<int64_t>(), r.d_line_off, r.d_spans, stride, c.last_text, ub, c.tb_lens.as<uint32_t>(),
-                        c.tb_offs.as<int64_t>(), c.tb_colinfo.as<int64_t>(), c.tb_data.as<uint8_t>());
-        CK(cudaGetLastError());
-        tm.mark("tables_gather", 1);
-        // (the host copy of col_info above is pageable: it has been staged by the time cudaMemcpyAsync returns)
-        c.tb_tables.assign(E, gorp_value_table{});
-        c.tb_off_ptr.assign(static_cast<size_t>(n_cols), nullptr);
-        c.tb_data_ptr.assign(static_cast<size_t>(n_cols), nullptr);
-        c.tb_valid_ptr.assign(static_cast<size_t>(n_cols), nullptr);
-        c.tb_nulls.assign(static_cast<size_t>(n_cols), 0);
-        for (uint32_t t = 0; t < E; ++t) {
-            const TableLayout& x = h_lay[t];
-            gorp_value_table& v = c.tb_tables[t];
-            v.n_rows = x.n_rows;
-            v.n_columns = static_cast<int32_t>(x.n_cols);
-            v.d_row = c.tb_rows.as<int64_t>() + x.row_base;
+        TablesBuilt b;
+        build_tables(e, c, st, tm, c.last, c.last_text, c.last_unit_bytes, b);
+        c.tb_desc.reset(c.n_ext, b.n_cols);
+        for (uint32_t t = 0; t < c.n_ext; ++t) {
+            const TableLayout& x = b.lay[t];
             for (int64_t k = 0; k < x.n_cols; ++k) {
                 const int64_t col = x.col_base + k;
-                c.tb_off_ptr[col] = c.tb_offs.as<int64_t>() + x.off_base + k * x.seg;
-                c.tb_data_ptr[col] = c.tb_data.as<uint8_t>() + col_info[2 * col + 1];
-                c.tb_valid_ptr[col] = reinterpret_cast<const uint8_t*>(c.tb_valid.as<uint32_t>() + x.valid_base + k * x.vwords);
-                c.tb_nulls[col] = h_stats[2 * col + 1];
+                c.tb_desc.offsets[col] = c.tb_offs.as<int64_t>() + x.off_base + k * x.seg;
+                c.tb_desc.data[col] = c.tb_data.as<uint8_t>() + b.col_info[2 * col + 1];
+                c.tb_desc.valid[col] = reinterpret_cast<const uint8_t*>(c.tb_valid.as<uint32_t>() + x.valid_base + k * x.vwords);
+                c.tb_desc.nulls[col] = b.stats[2 * col + 1];
             }
-            if (x.n_cols) {
-                v.d_offsets = c.tb_off_ptr.data() + x.col_base;
-                v.d_data = c.tb_data_ptr.data() + x.col_base;
-                v.d_valid = c.tb_valid_ptr.data() + x.col_base;
-                v.null_count = c.tb_nulls.data() + x.col_base;
-            }
+            c.tb_desc.set_table(t, x.n_rows, c.tb_rows.as<int64_t>() + x.row_base, x.col_base, x.n_cols);
         }
-        out->n_tables = static_cast<int32_t>(E);
-        out->unit_bytes = ub;
-        out->tables = c.tb_tables.data();
+        c.tb_desc.describe(out, c.last_unit_bytes);
         CK(cudaEventRecord(c.ev_done, st));
         if (flags & GORP_FLAG_SYNC) CK(cudaStreamSynchronize(st));
         return GORP_OK;

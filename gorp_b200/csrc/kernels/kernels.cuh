@@ -390,6 +390,19 @@ void k_tables_len(const Launch&, const TableLayout* lay, uint32_t n_ext, const i
 // offs = scan of lens; col_info[2 * col] = offs at the column's entry 0, col_info[2 * col + 1] = byte offset of its data
 void k_tables_gather(const Launch&, const TableLayout* lay, uint32_t n_ext, const int64_t* rows, const int64_t* line_off, const int32_t* spans,
                      uint32_t stride, const void* text, int unit_bytes, const uint32_t* lens, int64_t* offs, const int64_t* col_info, uint8_t* data);
+// The merge of one device's tables into the tables of a host call on several devices: n int64 entries of src plus `add`
+// (row indexes, offsets; src may be dst), or with shift 1..7 a validity bitmap of n bits moved up by `shift` bits into
+// (n + shift + 7) / 8 bytes of dst (the bits below `shift` of byte 0 are 0: the host ORs that byte into the bitmap).
+struct RebaseJob {
+    const void* src;
+    void* dst;
+    int64_t n;
+    int64_t add;
+    int64_t shift;
+    int64_t first_block;  // blocks of the jobs before this one (tables_rebase_blocks)
+};
+int64_t tables_rebase_blocks(const RebaseJob&);
+void k_tables_rebase(const Launch&, const RebaseJob* jobs, uint32_t n_jobs, int64_t n_blocks);
 
 // K3: per-extraction histogram (E entries, then MISS, then capture failures).
 void k3_histogram(const Launch&, const int32_t* ext_id, int64_t n_lines, uint32_t n_ext, unsigned long long* hist);

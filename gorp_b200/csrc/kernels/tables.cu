@@ -8,6 +8,8 @@
 //   len     : 256 rows of a table per task: u32 lengths, validity words, per-column totals and null counts
 //   (host: the per-column totals size the data) scan over every column's lengths at once -> offsets
 //   gather  : 32 rows of a column per task: offsets rebased in place, values copied with 16-byte stores
+//   rebase  : (host calls on several devices) a device's row indexes and offsets plus its bases, its bitmaps shifted to
+//             the bit position of its first row -> one table per extraction across the devices
 #include "kernels.cuh"
 
 namespace gorp {
@@ -240,6 +242,30 @@ __global__ void __launch_bounds__(kThreads) tables_gather_kernel(const TableLayo
     }
 }
 
+// One block of kRebaseBlock entries (or output bytes) of one job per iteration; the job is found by binary search over the
+// jobs' first blocks, as the table of a task above.
+constexpr int64_t kRebaseBlock = 8 * kThreads;
+__global__ void __launch_bounds__(kThreads) tables_rebase_kernel(const RebaseJob* __restrict__ jobs, uint32_t n_jobs, int64_t n_blocks) {
+    for (int64_t blk = blockIdx.x; blk < n_blocks; blk += gridDim.x) {
+        const RebaseJob J = jobs[table_of(blk, n_jobs, [&](uint32_t j) { return jobs[j].first_block; })];
+        const int64_t i0 = (blk - J.first_block) * kRebaseBlock;
+        if (!J.shift) {
+            const int64_t* src = static_cast<const int64_t*>(J.src);
+            int64_t* dst = static_cast<int64_t*>(J.dst);
+            for (int64_t i = i0 + threadIdx.x; i < min(i0 + kRebaseBlock, J.n); i += kThreads) dst[i] = src[i] + J.add;
+        } else {
+            // output byte j holds input bits [8j - shift, 8j + 8 - shift): the top of byte j - 1 and the bottom of byte j
+            const uint8_t* src = static_cast<const uint8_t*>(J.src);
+            uint8_t* dst = static_cast<uint8_t*>(J.dst);
+            const int64_t nb_in = (J.n + 7) / 8, nb_out = (J.n + J.shift + 7) / 8;
+            for (int64_t j = i0 + threadIdx.x; j < min(i0 + kRebaseBlock, nb_out); j += kThreads) {
+                const uint32_t lo = j >= 1 ? src[j - 1] : 0u, hi = j < nb_in ? src[j] : 0u;
+                dst[j] = static_cast<uint8_t>((hi << J.shift) | (lo >> (8 - J.shift)));
+            }
+        }
+    }
+}
+
 int grid_of(const Launch& L, const void* fn) {
     int per_sm = 1;
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, kThreads, 0);
@@ -247,6 +273,16 @@ int grid_of(const Launch& L, const void* fn) {
 }
 
 }  // namespace
+
+int64_t tables_rebase_blocks(const RebaseJob& j) {
+    const int64_t n = j.shift ? (j.n + j.shift + 7) / 8 : j.n;
+    return (n + kRebaseBlock - 1) / kRebaseBlock;
+}
+
+void k_tables_rebase(const Launch& L, const RebaseJob* jobs, uint32_t n_jobs, int64_t n_blocks) {
+    const int grid = static_cast<int>(std::min<int64_t>(n_blocks, static_cast<int64_t>(L.sm_count) * 8));
+    tables_rebase_kernel<<<grid, kThreads, 0, L.stream>>>(jobs, n_jobs, n_blocks);
+}
 
 int64_t tables_tile_lines(uint32_t n_ext) {
     // keeps the count matrix (E x tiles) at <= 1 entry per 32 lines

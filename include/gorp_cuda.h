@@ -231,6 +231,8 @@ typedef struct gorp_value_table {       /* the lines of extraction e, in line or
     const int64_t* null_count;          /* host [n_columns] */
 } gorp_value_table;
 
+/* (after gorp_extract_text_utf8_tables / gorp_extract_lines_utf8_tables every pointer here, d_row, d_offsets[k], d_data[k]
+ * and d_valid[k] included, is a pinned HOST pointer) */
 typedef struct gorp_device_tables {
     int32_t n_tables;                   /* == n_extractions; table e = extraction e */
     int32_t unit_bytes;                 /* 2 after the UTF-16 calls, 1 after the UTF-8 calls */
@@ -238,6 +240,34 @@ typedef struct gorp_device_tables {
 } gorp_device_tables;
 
 int gorp_extract_tables_device(gorp_engine* e, int dev_index, void* stream, int flags, gorp_device_tables* out);
+
+/* gorp_extract_text_utf8_bytes / gorp_extract_lines_utf8 that also return the values as tables in HOST memory — for callers
+ * whose text is on the host (a log file, a batch of records, an Arrow or Parquet string column read on the CPU) and that
+ * hand the values on as columns (Parquet, pandas, Arrow Java) rather than one string per group per line.
+ *
+ * *out is exactly what the plain call returns on the same arguments, and the call fails exactly where the plain call fails,
+ * with the same status and message; a null `tables` is GORP_E_ARG. *tables follows the contract of
+ * gorp_extract_tables_device with these differences: every pointer in it is pinned host memory; unit_bytes is 1; d_row
+ * indexes rows of *out; the values are bytes [line_off[row] + s, line_off[row] + t) of the caller's `text`. Every buffer is
+ * 64-byte aligned, bitmap padding bits are 0, an extraction without groups (and every extraction of a match-only engine,
+ * gorp_compile_patterns) has rows and no columns. On several devices every table is still one table: device d's rows
+ * follow those of the devices before it.
+ *
+ * The tables belong to the result: they stay valid until gorp_result_release(e, out), whatever other calls run on the
+ * engine in between, and their pinned buffers return to the engine with the result (allocated on the NUMA node of the
+ * engine's first device, as the rows are). Like every host call, these calls make the last device-resident result
+ * unreadable for gorp_extract_tables_device.
+ *
+ * Cost on top of the plain call, per device: the device keeps its whole byte range of the batch in engine scratch (1 byte
+ * per input byte; one device-to-device copy per staged piece), builds the tables of its rows after its last piece with the
+ * stages and the engine scratch of gorp_extract_tables_device, and copies them to the host. Host round trips: one per
+ * device (the per-column totals), then on several devices one synchronisation of all of them before the merge. Pinned
+ * host memory: 8 B per matched line (row indexes), 8 B per (matched line, group) (offsets), the values, and the bitmaps,
+ * each segment rounded up to 64 B. */
+int gorp_extract_text_utf8_tables(gorp_engine* e, const uint8_t* text, int64_t n_bytes, gorp_result* out,
+                                  gorp_device_tables* tables);
+int gorp_extract_lines_utf8_tables(gorp_engine* e, const uint8_t* text, const int64_t* off, int64_t n_lines, gorp_result* out,
+                                   gorp_device_tables* tables);
 
 /* Device time per pipeline stage, summed over the calls made with GORP_FLAG_TIME_KERNELS on (e, dev_index) since the
  * last reset: names[i] / total_ms[i] for i < *n (at most `cap`), `calls` = timed calls, `launches` = kernels launched
